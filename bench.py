@@ -2,8 +2,11 @@
 """Benchmark of the post-processing hot path (BASELINE.json metric: post-proc tiles/s & boxes/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload slide|tiles640|tiles1024|hnet] [--masks proto|none]
-                    [--dtype f32|f16]
+                    [--dtype f32|f16] [--dump-outputs DIR]
     python bench.py --impl reference ...      # the reference's CPU path (oracle port) on host cores
+
+--dump-outputs DIR writes what the last timed step returned (detections in the caller's order, mask pixels) as .npy
+files; the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 slide (default; BASELINE.json configs[3], the configuration the north-star target is quoted on): one "step" = a whole
 synthetic 100k x 100k px slide (11 025 tiles of 1024 px, 64 px overlap, ~3 000 nuclei per tile) cut from one global
@@ -102,7 +105,15 @@ def parse():
     ap.add_argument("--slide-streams", type=int, default=3,
                     help="slide workload: tile batches alternate over this many streams (SlidePostprocessor(streams=))")
     ap.add_argument("--inflight", type=int, default=3, help="steps in flight (CUDA graphs on separate streams)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32 or "
+                         "float64; a fixed, seeded sample of the detections and masks of a large step; with --gpus > 1 the part of "
+                         "rank 0)")
     a = ap.parse_args()
+    if a.steps is not None and a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl == "reference" or a.workload == "hnet"):
+        ap.error("--dump-outputs covers --impl ours on the slide, tiles640 and tiles1024 workloads")
     if a.masks is None:
         a.masks = "paste" if a.impl == "reference" else "proto"
     if a.steps is None:
@@ -338,14 +349,14 @@ def common_config(args, wl, masks):
 
 def run_reference(args, wl):
     """--impl reference: the reference's own CPU implementation (oracle port: same torch/torchvision calls) on all
-    host threads of ONE process; each step is a bounded sample of the workload, timed whole -- ms_per_step is the
-    measured time of one sample pass, `steps` the passes actually run."""
+    host threads of ONE process; each step is one pass over a bounded sample of the workload, --steps passes timed
+    whole -- ms_per_step is the measured time of one sample pass."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
     masks = args.masks
     wk = args.workload if args.workload != "hnet" else "tiles1024"
-    r = time_cpu(wk, wl, masks, budget_s=60.0, max_passes=max(1, min(args.steps, 50)), dtype=args.dtype,
+    r = time_cpu(wk, wl, masks, budget_s=float("inf"), max_passes=args.steps, dtype=args.dtype,
                  slide_size=args.slide_size)
     other = None
     if masks in ("paste", "proto"):      # the other mask variant beside it (one pass)
@@ -459,8 +470,51 @@ def load_peak():
         return 6650.0, "fallback 6650 GB/s (of fallback)"
 
 
+DUMP_ROWS = 1 << 19     # detections written by --dump-outputs (a seeded sample above that)
+DUMP_MASKS = 2048       # of which the first DUMP_MASKS also have their mask pixels written
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, boxes, scores, labels, mask_rows, masks, extra):
+    """--dump-outputs: the detections of the last timed step in the order the caller receives them (boxes [K,4],
+    scores [K], labels [K]) and their masks (row mask_rows[k] of the PackedMasks `masks`, or None).  Above DUMP_ROWS
+    detections a fixed, seeded sample is written (sample.npy: the positions in [0, K)); the masks of the first
+    DUMP_MASKS detections of the sample are unpacked to 0/1 pixels (mask_windows.npy: x0, y0, w, h; mask_pixels.npy:
+    every window row-major, one after the other).  `extra`: further small arrays, written as they are."""
+    import numpy as np
+    import torch
+    K = int(boxes.shape[0])
+    pos = np.arange(K) if K <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(K, DUMP_ROWS, replace=False))
+    sel = torch.from_numpy(pos).to(boxes.device)
+    arrays = dict(extra)
+    arrays.update(sample=pos.astype(np.float64), boxes=boxes[sel].float().cpu().numpy(),
+                  scores=scores[sel].float().cpu().numpy(), labels=labels[sel].cpu().numpy().astype(np.float32))
+    if masks is not None:
+        rows = mask_rows[sel[:DUMP_MASKS]].to(torch.int64)
+        g = masks.geom[rows].to(torch.int64)
+        wpr = (g[:, 2] + 31) >> 5                          # 32-bit words per mask row
+        words = wpr * g[:, 3]
+        owner = torch.repeat_interleave(torch.arange(rows.numel(), device=rows.device), words)
+        j = torch.arange(int(words.sum()), device=rows.device) - (torch.cumsum(words, 0) - words)[owner]
+        bits = np.unpackbits(masks.bits[masks.offsets[rows][owner] + j].cpu().numpy().view(np.uint8), bitorder="little")
+        g, wpr = g.cpu().numpy(), wpr.cpu().numpy()
+        pix, o = [], 0
+        for (_, _, w, h), n in zip(g, wpr):                # pixel (x, y) of a window is bit x of its row y
+            pix.append(bits[o:o + h * n * 32].reshape(h, n * 32)[:, :w].reshape(-1))
+            o += h * n * 32
+        arrays["mask_windows"] = g.astype(np.float32)
+        arrays["mask_pixels"] = (np.concatenate(pix) if pix else np.zeros((0,), np.uint8)).astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES} byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------ tiles workloads
-def run_tiles(args, wl, c):
+def run_tiles(args, wl, c, dump=None):
     import torch
     import hd_yolo_b200 as hdy
     from hd_yolo_b200 import masks as hmasks
@@ -554,6 +608,12 @@ def run_tiles(args, wl, c):
     ops.profile.reset()
     ms = c.timed(gstep2, K, side_streams=side)
     launches = ops.profile.launches
+    if dump and c.rank == 0:        # the last timed step replayed graph (K-1) mod R, whose outputs stay in place
+        o, p = graphs[(K - 1) % R].out
+        live = torch.arange(o.max_det, device=c.dev)[None, :] < o.counts[:, None]
+        rows = torch.nonzero(live.reshape(-1)).flatten()     # tile-major; mask index = tile * max_det + slot
+        dump_outputs(dump, o.boxes.reshape(-1, 4)[rows], o.scores.reshape(-1)[rows], o.labels.reshape(-1)[rows], rows,
+                     p, {"counts": o.counts.cpu().numpy().astype("float64")})
     tiles_per_s = c.world * bs * K / (ms * 1e-3)
     torch.cuda.synchronize()
     out, pm = gstep(0)
@@ -725,7 +785,8 @@ def _timed_phase(c, fn, reps):
     return c.timed(lambda i: fn(), reps) / reps
 
 
-def run_slide(args, wl, c, steps, warmup, want_e2e, want_cpu_merge=False, masks="proto", want_stages=True):
+def run_slide(args, wl, c, steps, warmup, want_e2e, want_cpu_merge=False, masks="proto", want_stages=True, dump=None):
+    import numpy as np
     import torch
     import hd_yolo_b200 as hdy
     from hd_yolo_b200 import ops, synth
@@ -788,6 +849,10 @@ def run_slide(args, wl, c, steps, warmup, want_e2e, want_cpu_merge=False, masks=
     launches = ops.profile.launches
     r = res["r"]
     n_local = int(r["n"])
+    if dump and c.rank == 0:        # this rank's survivors in score order, their masks by slide row
+        dump_outputs(dump, r["boxes"], r["scores"], r["labels"], r["index"] - int(r["base"]),
+                     r["masks"] if with_masks else None,
+                     {"counts": np.array([n_local, int(r["boxes"].shape[0])], dtype=np.float64)})
     seam_rows, exchanges = r.get("seam_rows"), r.get("exchanges")
     dg = kept_digest(r["state"], r["base"])
     words_local = int(r["masks"].offsets[n_local]) if with_masks else 0
@@ -977,7 +1042,7 @@ def main():
         sampler = ClockSampler(c.local)
         sampler.start()
         s = run_slide(args, wl, c, args.steps, args.warmup, want_e2e=not args.no_e2e,
-                      want_cpu_merge=not args.no_cpu_baseline, masks=masks)
+                      want_cpu_merge=not args.no_cpu_baseline, masks=masks, dump=args.dump_outputs)
         clocks = sampler.stop()
         cfg = common_config(args, wl, masks)
         cfg.update({"tiles": s["tiles"], "tiles_per_step_per_gpu": s["tiles"] / c.world, "detections": s["detections"],
@@ -1027,7 +1092,7 @@ def main():
         from tools.hnet_bench import run_hnet     # configs[4]: kept in its own file
         line = run_hnet(args, wl, c, common_config, load_peak, ClockSampler)
     else:
-        line = run_tiles(args, wl, c)
+        line = run_tiles(args, wl, c, dump=args.dump_outputs)
         if not args.no_sub:
             sargs = argparse.Namespace(**vars(args))
             line["slide"] = run_slide(sargs, WORKLOADS["slide"], c, steps=3, warmup=2, want_e2e=False,

@@ -1,79 +1,45 @@
-"""The oracle port against the REAL reference, live (skipped where /root/reference is absent, i.e. on the GPU box: the
-committed goldens of oracle/make_golden.py carry the same comparison there).  Random seeded inputs beyond the goldens:
-every function of the path the reference itself contains must agree bit for bit with its restatement in oracle/port.py."""
+"""The oracle port against the reference on seeded inputs beyond the goldens of oracle/make_golden.py: every function of
+the path the reference itself contains must agree bit for bit with its restatement in oracle/port.py.  Each case is
+checked against its stored record (tests/golden/live_cases.npz, see oracle/live_cases.py) everywhere, and also against
+the reference itself where its source tree is present (HD_YOLO_REFERENCE)."""
+import numpy as np
 import pytest
 import torch
 
-from oracle import port, ref_shim
-from hd_yolo_b200 import synth
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
+from conftest import load_golden
+from oracle import live_cases, port, ref_shim
 
 
 @pytest.fixture(scope="module")
 def ref():
-    return ref_shim.load()
+    return live_cases.reference_impl(ref_shim.load()) if ref_shim.available() else None
 
 
-@pytest.mark.parametrize("seed,n,nc,conf", [(0, 3000, 4, 0.2), (1, 800, 7, 0.05), (2, 50, 1, 0.5)])
+def _check(case, ref, *args):
+    got = case(port, *args)
+    gold = load_golden("live_cases")
+    assert sorted(got) == sorted(k for k in gold.files if k.startswith(next(iter(got)).split("_")[0] + "_"))
+    for k, v in got.items():
+        assert np.array_equal(live_cases.digest(v), gold[k]), f"{k} differs from the record ({gold['source']})"
+    if ref is not None:
+        want = case(ref, *args)
+        assert sorted(want) == sorted(got)
+        for k, v in got.items():
+            assert torch.equal(v, want[k]), k
+
+
+@pytest.mark.parametrize("seed,n,nc,conf", live_cases.NMS_CASES)
 def test_nms_per_image_and_nms_equal_reference(ref, seed, n, nc, conf):
-    g = torch.Generator().manual_seed(seed)
-    c = torch.rand((2, n, 2), generator=g) * 600
-    wh = torch.rand((2, n, 2), generator=g) * 40 + 1
-    sc = torch.rand((2, n, 1 + nc), generator=g)
-    extra = torch.rand((2, n, 2), generator=g)
-    preds = torch.cat([c, wh, sc, extra], -1)
-    a = ref.nms_per_image(preds.clone(), nc, conf_thres=conf, iou_thres=0.45, max_det=300)
-    b = port.nms_per_image(preds.clone(), nc, conf, 0.45, 300)
-    for x, y in zip(a, b):
-        assert all(torch.equal(x[k], y[k]) for k in ("boxes", "scores", "extra"))
-    y5 = torch.cat([c, wh, sc], -1)
-    for kw in (dict(), dict(agnostic=True), dict(multi_label=True), dict(classes=[0])):
-        ra = ref.non_max_suppression(y5.clone(), conf, 0.45, max_det=300, **kw)
-        rb = port.non_max_suppression(y5.clone(), conf, 0.45, max_det=300, **kw)
-        assert all(torch.equal(p, q) for p, q in zip(ra, rb)), kw
+    _check(live_cases.nms_case, ref, seed, n, nc, conf)
 
 
 def test_box_helpers_equal_reference(ref):
-    g = torch.Generator().manual_seed(5)
-    a = torch.rand((300, 4), generator=g) * 500
-    b = torch.rand((200, 4), generator=g) * 500
-    a[:, 2:] += a[:, :2]
-    b[:, 2:] += b[:, :2]
-    assert torch.equal(ref.box_iou(a, b), port.box_iou(a, b))
-    assert torch.equal(ref.xywh2xyxy(a), port.xywh2xyxy(a))
-    for img1, img0, rp in [((640, 640), (480, 720), None), ((320, 512), (777, 333), ((0.5, 0.5), (10.0, 20.0)))]:
-        assert torch.equal(ref.scale_coords(img1, a.clone(), img0, rp), port.scale_coords(img1, a.clone(), img0, rp))
+    _check(live_cases.box_case, ref)
 
 
 def test_scanner_and_tile_merge_equal_reference(ref):
-    for size, roi, ov in [((3000, 2500), (1024, 1024), 64), ((700, 900), (512, 512), 0), ((100000, 100000), (1024, 1024), 64)]:
-        assert torch.equal(ref.sliding_window_scanner(size, roi, ov), port.sliding_window_scanner(size, roi, ov))
-    g = torch.Generator().manual_seed(9)
-    tiles = []
-    for t in range(6):
-        k = 150
-        c = torch.rand((k, 2), generator=g) * 512
-        wh = torch.rand((k, 2), generator=g) * 30 + 8
-        tiles.append({'boxes': torch.cat([c - wh / 2, c + wh / 2], 1), 'scores': torch.rand((k,), generator=g),
-                      'labels': torch.randint(1, 5, (k,), generator=g),
-                      'roi': torch.tensor([(t % 3) * 448.0, (t // 3) * 448.0, 0.0, 0.0])})
-    m_ref = ref.Detect.merge_outputs(None, [{k: (v.clone() if torch.is_tensor(v) else v) for k, v in t.items()} for t in tiles])
-    m_port = port.merge_outputs(tiles)
-    assert all(torch.equal(m_ref[k], m_port[k]) for k in ("boxes", "scores", "labels"))
-    params = {'conf_thres': 0.3, 'iou_thres': 0.45, 'max_det': 500}
-    e_ref = ref.Ensemble([], nms_params=params).merge([{'det': m_ref}])['det']
-    e_port = port.ensemble_merge([{'det': m_port}], params)['det']
-    assert all(torch.equal(e_ref[k], e_port[k]) for k in ("boxes", "scores", "labels"))
+    _check(live_cases.merge_case, ref)
 
 
 def test_compute_proposals_equals_reference_head(ref):
-    torch.manual_seed(3)
-    strides, anchors, nc = synth.STRIDES_3, synth.ANCHORS_3, 4
-    det = ref.Detect(ch=[8, 8, 8], anchors=anchors, strides=strides, nc=nc, masks={}, is_scripting=True)
-    det.eval()
-    dets = [torch.randn(2, 3, 160 // s, 160 // s, 5 + nc) for s in strides]
-    with torch.no_grad():
-        want = det.compute_proposals([d.clone() for d in dets])
-    got = port.compute_proposals(dets, anchors, strides)
-    assert all(torch.equal(a, b) for a, b in zip(want, got))
+    _check(live_cases.proposals_case, ref)
