@@ -15,7 +15,6 @@
 // atomicAdd per CTA (warp ballot + block prefix); the list is unordered, the 64-bit key carries the
 // row index so that the NMS kernel's sort restores the reference's order exactly.
 #include <math.h>
-#include <stdlib.h>
 #include "hdy_common.cuh"
 
 namespace hdy {
@@ -167,82 +166,14 @@ __global__ void __launch_bounds__(kThreads) filter_compact_logits_kernel(
 }
 
 // ------------------------------------------------------------------------------------------------
-// Wide rows (mask coefficients behind the scores: no = 41 is 164 bytes per row).  The filter needs ONE float of every
-// row -- the objectness logit -- and the box of the few per cent that pass; everything else in a rejected row is
-// dead weight.  Instead of streaming whole rows through shared memory (filter_tma.cu), every thread reads the logits
-// of kSparseRows rows directly: one sector per row, a fifth of the bytes -- an experiment kept selectable
-// (HDY_FILTER=sparse) because it did NOT pay: 62.9 us against 58.3 us on B200, HBM delivers the rows either way.
-// Rows are rejected on the logit (x < logit(conf) - margin), survivors
-// fetch their box from the sector(s) just touched.  Same candidates, same arithmetic, arbitrary list order (the NMS
-// sorts) -- as with the other filter kernels.
-// ------------------------------------------------------------------------------------------------
-constexpr int kSparseRows = 4;
-constexpr int kSparseChunk = kThreads * kSparseRows;
-
-__global__ void __launch_bounds__(kThreads) filter_compact_sparse_kernel(
-    const __grid_constant__ LevelTable T, float t_lo, float conf_thres, float min_size, int cap,
-    uint64_t* __restrict__ cand_keys, float4* __restrict__ cand_boxes, int32_t* __restrict__ counts,
-    int32_t* __restrict__ status) {
-  const int tile = blockIdx.x / T.chunks_per_tile;
-  const int chunk = blockIdx.x - tile * T.chunks_per_tile;
-  int l;
-  const LevelDev& L = find_level(T, chunk, l);
-  const int row0 = (chunk - L.chunk_begin) * kSparseChunk;
-  const int rows = min(kSparseChunk, L.rows - row0);
-  const int no = T.no;
-  const int t = threadIdx.x, lane = t & 31;
-  const int plane = L.ny * L.nx;
-  const float* g = L.ptr + ((size_t)tile * L.rows + row0) * no;
-  float x[kSparseRows];
-#pragma unroll
-  for (int k = 0; k < kSparseRows; ++k) {
-    const int r = t + k * kThreads;
-    x[k] = r < rows ? ldg_stream_f(g + (size_t)r * no + 4) : -3.0e38f;
-  }
-#pragma unroll
-  for (int k = 0; k < kSparseRows; ++k) {
-    const int r = t + k * kThreads;
-    bool cand = false;
-    float p_obj = 0.f;
-    float4 box = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (x[k] >= t_lo) {
-      p_obj = sigmoidf_ref(x[k]);
-      if (p_obj > conf_thres) {
-        const float* rp = g + (size_t)r * no;
-        const int row = row0 + r;
-        const int a = row / plane, p = row - a * plane;
-        const int gy = p / L.nx, gx = p - gy * L.nx;
-        Decoded d = decode_box(__ldg(rp), __ldg(rp + 1), __ldg(rp + 2), __ldg(rp + 3), (float)gx, (float)gy, L.stride,
-                               L.aw[a], L.ah[a]);
-        box = xywh_to_xyxy(d.cx, d.cy, d.w, d.h);
-        cand = (__fsub_rn(box.z, box.x) >= min_size) && (__fsub_rn(box.w, box.y) >= min_size);
-      }
-    }
-    const unsigned m = __ballot_sync(0xffffffffu, cand);
-    if (m) {
-      int base = 0;
-      if (lane == 0) base = atomicAdd(counts + tile, __popc(m));
-      base = __shfl_sync(0xffffffffu, base, 0);
-      if (cand) {
-        const int pos = base + __popc(m & ((1u << lane) - 1u));
-        if (pos < cap) {
-          const size_t o = (size_t)tile * cap + pos;
-          cand_keys[o] = make_key(p_obj, (uint32_t)(L.row_offset + row0 + r));
-          cand_boxes[o] = box;
-        } else {
-          atomicOr(status, HDY_STATUS_OVERFLOW);
-        }
-      }
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
 // Conv-native layout [bs, na*no, ny, nx] (layout 1, the yolo_head.py:141-145 permute skipped): the objectness logits of
 // an (image, anchor) pair are ONE contiguous plane, so the filter streams 4 bytes per row instead of 4*no -- 6.5 MB
 // instead of 266 MB per tiles640 batch with mask coefficients.  Every thread takes four consecutive rows with one
 // 128-bit load, rejects on the logit, and survivors gather their four box logits from the neighbouring planes.
 // ------------------------------------------------------------------------------------------------
+constexpr int kPlanarRows = 4;
+constexpr int kPlanarChunk = kThreads * kPlanarRows;
+
 __global__ void __launch_bounds__(kThreads) filter_compact_planar_kernel(
     const __grid_constant__ LevelTable T, float t_lo, float conf_thres, float min_size, int cap,
     uint64_t* __restrict__ cand_keys, float4* __restrict__ cand_boxes, int32_t* __restrict__ counts,
@@ -251,19 +182,19 @@ __global__ void __launch_bounds__(kThreads) filter_compact_planar_kernel(
   // phase B (the first q_n threads): sigmoid, box gather, decode, min-size, one global atomic per block.  Handling
   // survivors inline made 3 warps in 4 run the whole decode for one lane each and chained four global atomics per
   // warp behind two dependent loads (ncu: 32 us, 12 M warp instructions for 1.6 M rows).
-  __shared__ int q_row[kSparseChunk];
-  __shared__ float q_x[kSparseChunk];
+  __shared__ int q_row[kPlanarChunk];
+  __shared__ float q_x[kPlanarChunk];
   __shared__ int q_n;
   const int tile = blockIdx.x / T.chunks_per_tile;
   const int chunk = blockIdx.x - tile * T.chunks_per_tile;
   int l;
   const LevelDev& L = find_level(T, chunk, l);
-  const int row0 = (chunk - L.chunk_begin) * kSparseChunk + threadIdx.x * kSparseRows;  // first of this thread's rows
+  const int row0 = (chunk - L.chunk_begin) * kPlanarChunk + threadIdx.x * kPlanarRows;  // first of this thread's rows
   const int no = T.no, lane = threadIdx.x & 31;
   const int plane = L.ny * L.nx;
   if (threadIdx.x == 0) q_n = 0;
-  float x[kSparseRows];
-  const bool vec = (plane & 3) == 0 && row0 + kSparseRows <= L.rows;  // four rows of one plane, 16-byte aligned
+  float x[kPlanarRows];
+  const bool vec = (plane & 3) == 0 && row0 + kPlanarRows <= L.rows;  // four rows of one plane, 16-byte aligned
   if (vec) {
     const int a = row0 / plane, p = row0 - a * plane;
     const float4 v = ldg_stream_f4(reinterpret_cast<const float4*>(
@@ -271,7 +202,7 @@ __global__ void __launch_bounds__(kThreads) filter_compact_planar_kernel(
     x[0] = v.x, x[1] = v.y, x[2] = v.z, x[3] = v.w;
   } else {
 #pragma unroll
-    for (int k = 0; k < kSparseRows; ++k) {
+    for (int k = 0; k < kPlanarRows; ++k) {
       const int r = row0 + k;
       x[k] = -3.0e38f;
       if (r < L.rows) {
@@ -282,7 +213,7 @@ __global__ void __launch_bounds__(kThreads) filter_compact_planar_kernel(
   }
   __syncthreads();  // q_n = 0 is visible
 #pragma unroll
-  for (int k = 0; k < kSparseRows; ++k) {
+  for (int k = 0; k < kPlanarRows; ++k) {
     const bool pass = x[k] >= t_lo;  // (false for the -3e38 padding)
     const unsigned m = __ballot_sync(0xffffffffu, pass);
     if (m) {
@@ -616,35 +547,17 @@ int hdy_filter_compact_logits(const hdy_level_t* levels_host, int nl, int bs, in
   if (rc) return rc;
   T.nc = nc;
   if (bs == 0) return HDY_OK;
-  // HDY_FILTER=sparse selects the sector-sparse kernel (read per call: tests and A/B runs switch it).  Measured on B200
-  // at no = 41: 62.9 us against 58.3 us for the TMA streamer -- touching one 32-byte sector of every 164-byte row does
-  // not make HBM deliver less than the whole rows, so it is not the default.
-  const char* fsel = getenv("HDY_FILTER");
-  if (T.dtype == HDY_F16) fsel = nullptr;  // the experimental kernels read fp32 only
   const bool conf_ok = conf_thres > 1e-6f && conf_thres < 1.0f - 1e-6f;
-  if (layout == 0 && conf_ok && fsel && fsel[0] == 's') {
-    LevelTable S;
-    rc = build_level_table(levels_host, nl, na, no, 0, kSparseChunk, &S);
-    if (rc) return rc;
-    S.nc = nc;
-    const double lg = log((double)conf_thres / (1.0 - (double)conf_thres));
-    const float t_lo = (float)(lg - 1e-4 * (1.0 + fabs(lg)));  // sigmoid(x) <= conf for certain below this logit
-    const size_t nblk = (size_t)bs * S.chunks_per_tile;
-    HDY_REQUIRE(nblk < (1ull << 31), "grid too large");
-    filter_compact_sparse_kernel<<<(unsigned)nblk, kThreads, 0, (cudaStream_t)stream>>>(
-        S, t_lo, conf_thres, min_size, cap, cand_keys, reinterpret_cast<float4*>(cand_boxes), counts, status);
-    return check_launch("hdy_filter_compact_logits(sparse)");
-  }
-  if (layout == 1 && conf_ok && !(fsel && fsel[0] == 'g')) {  // (HDY_FILTER=generic: the one-row-per-thread kernel)
+  if (layout == 1 && conf_ok) {
     bool aligned = true;
     for (int i = 0; i < nl; ++i) aligned = aligned && (((uintptr_t)levels_host[i].logits & 15) == 0);
     if (aligned) {
       LevelTable S;
-      rc = build_level_table(levels_host, nl, na, no, 1, kSparseChunk, &S);
+      rc = build_level_table(levels_host, nl, na, no, 1, kPlanarChunk, &S);
       if (rc) return rc;
       S.nc = nc;
       const double lg = log((double)conf_thres / (1.0 - (double)conf_thres));
-      const float t_lo = (float)(lg - 1e-4 * (1.0 + fabs(lg)));
+      const float t_lo = (float)(lg - 1e-4 * (1.0 + fabs(lg)));  // sigmoid(x) <= conf for certain below this logit
       const size_t nblk = (size_t)bs * S.chunks_per_tile;
       HDY_REQUIRE(nblk < (1ull << 31), "grid too large");
       filter_compact_planar_kernel<<<(unsigned)nblk, kThreads, 0, (cudaStream_t)stream>>>(

@@ -20,7 +20,6 @@
 // phase B:    (32 survivors at a time) every lane takes one queue entry: sigmoid, the reference's own `> conf` test
 //             (so the verdict is identical to comparing the fp32 sigmoid), box decode, min-size test; one atomicAdd
 //             per (warp, tile) reserves the run in the tile's candidate list and the lanes write key + box.
-#include <stdlib.h>
 #include "hdy_common.cuh"
 
 namespace hdy {
@@ -265,12 +264,17 @@ __global__ void __launch_bounds__(WARPS * 32) filter_compact_tma_kernel(
   flush_pending();
 }
 
-template <int WARPS, int NBUF, int RPL, bool HALF>
-static int launch_variant_t(const LevelTable& T, const ItemTable& I, int bs, int buf_bytes, int ctas_per_sm,
-                          int sm_count, float t_lo, float conf_thres, float min_size, int cap, uint64_t* cand_keys,
-                          float* cand_boxes, int32_t* counts, int32_t* status, cudaStream_t stream) {
-  const size_t smem = per_warp_bytes(NBUF, buf_bytes) * WARPS;
-  cudaError_t e = cudaFuncSetAttribute(filter_compact_tma_kernel<WARPS, NBUF, RPL, HALF>,
+// The launched shape, measured best on B200 (DESIGN.md 3.5): four streamer warps per CTA with two buffers each, and
+// chunks of at most kTmaChunkBytes
+constexpr int kTmaWarps = 4, kTmaNbuf = 2;
+constexpr int kTmaChunkBytes = 14336;
+
+template <int RPL, bool HALF>
+static int launch_tma(const LevelTable& T, const ItemTable& I, int bs, int buf_bytes, int ctas_per_sm, int sm_count,
+                      float t_lo, float conf_thres, float min_size, int cap, uint64_t* cand_keys, float* cand_boxes,
+                      int32_t* counts, int32_t* status, cudaStream_t stream) {
+  const size_t smem = per_warp_bytes(kTmaNbuf, buf_bytes) * kTmaWarps;
+  cudaError_t e = cudaFuncSetAttribute(filter_compact_tma_kernel<kTmaWarps, kTmaNbuf, RPL, HALF>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) {
     set_error("cudaFuncSetAttribute(filter_compact_tma_kernel): %s", cudaGetErrorString(e));
@@ -278,23 +282,23 @@ static int launch_variant_t(const LevelTable& T, const ItemTable& I, int bs, int
   }
   const int total = I.begin[T.nl];
   long long grid = (long long)sm_count * ctas_per_sm;
-  const long long need = ((long long)total + WARPS - 1) / WARPS;
+  const long long need = ((long long)total + kTmaWarps - 1) / kTmaWarps;
   if (grid > need) grid = need;
-  filter_compact_tma_kernel<WARPS, NBUF, RPL, HALF><<<(unsigned)grid, WARPS * 32, smem, stream>>>(
+  filter_compact_tma_kernel<kTmaWarps, kTmaNbuf, RPL, HALF><<<(unsigned)grid, kTmaWarps * 32, smem, stream>>>(
       T, I, bs, buf_bytes, t_lo, conf_thres, min_size, cap, cand_keys, reinterpret_cast<float4*>(cand_boxes),
       counts, status);
   return check_launch("hdy_filter_compact_logits(tma)");
 }
 
-template <int WARPS, int NBUF, int RPL>
-static int launch_variant(const LevelTable& T, const ItemTable& I, int bs, int buf_bytes, int ctas_per_sm,
+template <int RPL>
+static int launch_tma_rpl(const LevelTable& T, const ItemTable& I, int bs, int buf_bytes, int ctas_per_sm,
                           int sm_count, float t_lo, float conf_thres, float min_size, int cap, uint64_t* cand_keys,
                           float* cand_boxes, int32_t* counts, int32_t* status, cudaStream_t stream) {
   if (T.dtype == HDY_F16)
-    return launch_variant_t<WARPS, NBUF, RPL, true>(T, I, bs, buf_bytes, ctas_per_sm, sm_count, t_lo, conf_thres,
-                                                    min_size, cap, cand_keys, cand_boxes, counts, status, stream);
-  return launch_variant_t<WARPS, NBUF, RPL, false>(T, I, bs, buf_bytes, ctas_per_sm, sm_count, t_lo, conf_thres,
-                                                   min_size, cap, cand_keys, cand_boxes, counts, status, stream);
+    return launch_tma<RPL, true>(T, I, bs, buf_bytes, ctas_per_sm, sm_count, t_lo, conf_thres, min_size, cap,
+                                 cand_keys, cand_boxes, counts, status, stream);
+  return launch_tma<RPL, false>(T, I, bs, buf_bytes, ctas_per_sm, sm_count, t_lo, conf_thres, min_size, cap,
+                                cand_keys, cand_boxes, counts, status, stream);
 }
 
 // Host side: returns HDY_OK, an error, or 1 when the layout does not meet the bulk-copy alignment rules
@@ -302,22 +306,15 @@ static int launch_variant(const LevelTable& T, const ItemTable& I, int bs, int b
 int launch_filter_compact_tma(const hdy_level_t* levels_host, int nl, int bs, int na, int nc, int no, float conf_thres,
                               float min_size, int cap, uint64_t* cand_keys, float* cand_boxes, int32_t* counts,
                               int32_t* status, cudaStream_t stream) {
-  // tuning knobs (defaults measured on B200, see DESIGN.md); HDY_TMA_VARIANT="warps,nbuf,chunk_bytes" overrides
-  static int kWarps = 4, kNbuf = 2, kChunk = 14336;
-  static bool env_read = false;
-  if (!env_read) {
-    env_read = true;
-    if (const char* v = getenv("HDY_TMA_VARIANT")) sscanf(v, "%d,%d,%d", &kWarps, &kNbuf, &kChunk);
-  }
-  // rows per lane and chunk: 1, 2, 4 or 8, the largest whose chunk stays within kChunk bytes (9 KB chunks at no = 9,
+  // rows per lane and chunk: 1, 2, 4 or 8, the largest whose chunk stays within kTmaChunkBytes (9 KB chunks at no = 9,
   // 10.5 KB at no = 41: measured best on B200, smaller chunks pay the per-chunk handshake, larger ones leave too few
   // warps per SM)
   const int esz = levels_host[0].dtype == HDY_F16 ? 2 : 4;
-  int rpl = kChunk / (32 * no * esz);
+  int rpl = kTmaChunkBytes / (32 * no * esz);
   rpl = rpl >= 8 ? 8 : (rpl >= 4 ? 4 : (rpl >= 2 ? 2 : 1));
   const int chunk_rows = 32 * rpl;
   const int buf_bytes = (chunk_rows * no * esz + 127) & ~127;
-  const size_t smem = per_warp_bytes(kNbuf, buf_bytes) * kWarps;
+  const size_t smem = per_warp_bytes(kTmaNbuf, buf_bytes) * kTmaWarps;
   if (smem > 227 * 1024) return 1;
   if (!(conf_thres > 1e-6f && conf_thres < 1.0f - 1e-6f)) return 1;  // logit(conf) is not finite enough
   for (int l = 0; l < nl; ++l)
@@ -348,29 +345,17 @@ int launch_filter_compact_tma(const hdy_level_t* levels_host, int nl, int bs, in
   }
   int per_sm = (int)((228 * 1024) / (smem + 1024));
   per_sm = per_sm < 1 ? 1 : (per_sm > 8 ? 8 : per_sm);
-#define HDY_TMA_CASE(W, B)                                                                                        \
-  if (kWarps == W && kNbuf == B) {                                                                                \
-    if (rpl == 8)                                                                                                 \
-      return launch_variant<W, B, 8>(T, I, bs, buf_bytes, per_sm, sm_count, t_lo, conf_thres, min_size, cap,      \
-                                     cand_keys, cand_boxes, counts, status, stream);                              \
-    if (rpl == 4)                                                                                                 \
-      return launch_variant<W, B, 4>(T, I, bs, buf_bytes, per_sm, sm_count, t_lo, conf_thres, min_size, cap,      \
-                                     cand_keys, cand_boxes, counts, status, stream);                              \
-    if (rpl == 2)                                                                                                 \
-      return launch_variant<W, B, 2>(T, I, bs, buf_bytes, per_sm, sm_count, t_lo, conf_thres, min_size, cap,      \
-                                     cand_keys, cand_boxes, counts, status, stream);                              \
-    return launch_variant<W, B, 1>(T, I, bs, buf_bytes, per_sm, sm_count, t_lo, conf_thres, min_size, cap,        \
-                                   cand_keys, cand_boxes, counts, status, stream);                                \
-  }
-  HDY_TMA_CASE(4, 2)
-  HDY_TMA_CASE(5, 2)
-  HDY_TMA_CASE(11, 2)
-  HDY_TMA_CASE(8, 2)
-  HDY_TMA_CASE(7, 3)
-  HDY_TMA_CASE(16, 2)
-#undef HDY_TMA_CASE
-  set_error("HDY_TMA_VARIANT: unsupported (warps, nbuf) = (%d, %d)", kWarps, kNbuf);
-  return HDY_ERR_INVALID;
+  if (rpl == 8)
+    return launch_tma_rpl<8>(T, I, bs, buf_bytes, per_sm, sm_count, t_lo, conf_thres, min_size, cap, cand_keys,
+                             cand_boxes, counts, status, stream);
+  if (rpl == 4)
+    return launch_tma_rpl<4>(T, I, bs, buf_bytes, per_sm, sm_count, t_lo, conf_thres, min_size, cap, cand_keys,
+                             cand_boxes, counts, status, stream);
+  if (rpl == 2)
+    return launch_tma_rpl<2>(T, I, bs, buf_bytes, per_sm, sm_count, t_lo, conf_thres, min_size, cap, cand_keys,
+                             cand_boxes, counts, status, stream);
+  return launch_tma_rpl<1>(T, I, bs, buf_bytes, per_sm, sm_count, t_lo, conf_thres, min_size, cap, cand_keys,
+                           cand_boxes, counts, status, stream);
 }
 
 }  // namespace hdy

@@ -15,28 +15,23 @@
 //            FFMA each) and writes them into the detection's PATCH (<= 16x16 floats) in the workspace.  Three CTAs
 //            per SM, no halo, no atomics.  The tile origin of a TMA load must be 16-byte aligned in the innermost
 //            dimension (measured: tools/micro/tma4d_test.cu faults otherwise), hence 24-pixel regions.
-//   phase 2  mask_upsample_pack_kernel, one WARP per detection, 48 warps per SM.  The patch (with a ring of zeros: the
-//            crop) goes to shared memory; per 32-pixel output word the lanes first interpolate their column along x
-//            for every source row, then every output row is one 2-tap blend of two of those values, a compare and a
-//            ballot -- ATen's bilinear (align_corners=False) operation by operation.  Every word of every mask is
-//            stored exactly once, so the bit planes need no clearing.
-//   Detections whose kept range exceeds 16x16 proto pixels (64 px boxes at the usual 4x) are listed by phase 2 and
-//   handled by the per-detection kernel of mask.cu.
-#include <stdlib.h>
+//   phase 2  one WARP per detection: the patch (with a ring of zeros: the crop) goes to shared memory and is
+//            upsampled with ATen's bilinear (align_corners=False) operation by operation, thresholded and stored.
+//            Every word of every mask is stored exactly once, so the bit planes need no clearing.
+//              * bit-packed + upsampled (the throughput form): mask_upsample_pack2_kernel (upsample_pack_v2 below).
+//              * the other forms (dense output, or packed at proto resolution): mask_upsample_pack_kernel.
+//   Detections whose kept range exceeds 16x16 proto pixels (64 px boxes at the usual 4x), or that fall into an overfull
+//   region, are listed and handled by the per-detection body of mask.cu.  In the packed + upsampled form they ride in
+//   the first CTAs of the phase-1 launch; in the other forms they get a launch of their own behind phase 2.
+//   The packed + upsampled form needs the windows of hdy_process_mask_geometry; without them the caller falls back to
+//   the per-detection kernel.
 #include "tma_common.cuh"
 #include "mask_common.cuh"
 
-#ifndef HDY_MASK_DEFAULT_PATH
-#define HDY_MASK_DEFAULT_PATH 1  // 1: two kernels (regions -> patches, upsample_pack_v2); 2: fused persistent kernel
-#endif
-#ifndef HDY_REG_BOX_X
-#define HDY_REG_BOX_X 24
-#define HDY_REG_BOX_Y 24
-#endif
-
 namespace hdy {
 
-constexpr int kRegBoxX = HDY_REG_BOX_X, kRegBoxY = HDY_REG_BOX_Y;  // region == TMA box (x origin 16-byte aligned)
+// region == TMA box: a tile origin must be 16-byte aligned in x (24 fp32 = 96 bytes, 24 fp16 = 48 bytes)
+constexpr int kRegBoxX = 24, kRegBoxY = 24;
 constexpr int kRegNm = 32;
 constexpr int kRegThreads = 256;
 constexpr int kRegWarps = kRegThreads / 32;
@@ -64,29 +59,24 @@ struct RegionList {
 };
 static_assert(sizeof(RegionList) == 512, "one region list is 512 bytes");
 struct PmWorkspace {
-  int32_t* large_count;   // [0]: detections left to the per-detection kernel
-  int32_t* work_counter;  // [1]: next (tile, region) item of the fused kernel
+  int32_t* large_count;   // detections left to the per-detection kernel
   int32_t* large_list;
   float* patches;
   RegionList* regions;
-  int32_t* done;          // per slot: pieces of the patch written so far (fused kernel)
   int4* kr;               // per slot: kept proto range (px0, py0, px1, py1), written by the binning kernel
 };
 static inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 size_t process_mask_workspace_bytes(long long bs, long long max_det) {
   const long long slots = bs * max_det;
-  return 256 + 2 * align256((size_t)slots * 4) + align256((size_t)slots * 16) +
+  return 256 + align256((size_t)slots * 4) + align256((size_t)slots * 16) +
          (size_t)slots * kPatchPitch * kPatchPitch * 4 + (size_t)bs * kMaxRegionsPerTile * sizeof(RegionList);
 }
 static PmWorkspace pm_workspace(void* base, long long slots) {
   PmWorkspace w;
   unsigned char* p = static_cast<unsigned char*>(base);
   w.large_count = reinterpret_cast<int32_t*>(p);
-  w.work_counter = reinterpret_cast<int32_t*>(p) + 1;
   p += 256;
   w.large_list = reinterpret_cast<int32_t*>(p);
-  p += align256((size_t)slots * 4);
-  w.done = reinterpret_cast<int32_t*>(p);
   p += align256((size_t)slots * 4);
   w.kr = reinterpret_cast<int4*>(p);
   p += align256((size_t)slots * 16);
@@ -320,6 +310,7 @@ __global__ void __launch_bounds__(kUpWarps * 32) mask_upsample_pack_kernel(
     const int32_t* __restrict__ geom4, const int64_t* __restrict__ offsets, uint32_t* __restrict__ bits,
     long long capacity_words,
     int32_t* __restrict__ status, int32_t* __restrict__ large_count, int32_t* __restrict__ large_list) {
+  static_assert(!(PACKED && UPSAMPLE), "the packed + upsampled form runs mask_upsample_pack2_kernel");
   __shared__ UpSmem S;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const long long slot = (long long)blockIdx.x * kUpWarps + warp;
@@ -425,20 +416,13 @@ __global__ void __launch_bounds__(kUpWarps * 32) mask_upsample_pack_kernel(
           for (int s = lr; s < src_rows; s += rows_per)
             col[s][lc] = __fadd_rn(__fmul_rn(X.l0, P[s * kPatchRing + xi0]), __fmul_rn(X.l1, P[s * kPatchRing + xi1]));
         __syncwarp();
-        const unsigned row_mask = vw == 32 ? 0xffffffffu : ((1u << vw) - 1u);
         for (int rb = 0; rb < nr; rb += rows_per) {
           const int r = rb + lr;
-          bool bit = false;
           if (active && r < nr) {
             const float4 rt = *reinterpret_cast<const float4*>(&rowtab[r]);
             const float v = __fadd_rn(__fmul_rn(rt.z, col[__float_as_int(rt.x)][lc]),
                                       __fmul_rn(rt.w, col[__float_as_int(rt.y)][lc]));
-            bit = v > 0.5f;
-            if (!PACKED) out_dense[slot * oh * ow + (size_t)(g.y0 + r0 + r) * ow + g.x0 + (w << 5) + lc] = bit ? 1.f : 0.f;
-          }
-          if (PACKED) {
-            const unsigned m = __ballot_sync(0xffffffffu, bit);
-            if (active && lc == 0 && r < nr) bits[off + (long long)(r0 + r) * wpr + w] = (m >> (lr * vw)) & row_mask;
+            out_dense[slot * oh * ow + (size_t)(g.y0 + r0 + r) * ow + g.x0 + (w << 5) + lc] = v > 0.5f ? 1.f : 0.f;
           }
         }
         continue;
@@ -452,45 +436,32 @@ __global__ void __launch_bounds__(kUpWarps * 32) mask_upsample_pack_kernel(
       for (int s = 0; s < src_rows; ++s)
         col[s][lane] = __fadd_rn(__fmul_rn(X.l0, P[s * kPatchRing + xi0]), __fmul_rn(X.l1, P[s * kPatchRing + xi1]));
       __syncwarp();
-      uint32_t* dst = bits + off + (long long)r0 * wpr + w;
       float* dd = out_dense + slot * oh * ow + (size_t)(g.y0 + r0) * ow + g.x0 + c;
-      unsigned myword = 0;
 #pragma unroll 4
       for (int r = 0; r < nr; ++r) {
         const float4 rt = *reinterpret_cast<const float4*>(&rowtab[r]);
         const float v = __fadd_rn(__fmul_rn(rt.z, col[__float_as_int(rt.x)][lane]),
                                   __fmul_rn(rt.w, col[__float_as_int(rt.y)][lane]));
-        const bool bit = valid && v > 0.5f;
-        if (PACKED) {
-          const unsigned word = __ballot_sync(0xffffffffu, bit);
-          if ((r & 31) == lane) myword = word;
-          if ((r & 31) == 31 || r == nr - 1) {  // lanes store the words of up to 32 rows at once
-            const int rr = (r & ~31) + lane;
-            if (rr <= r) dst[(long long)rr * wpr] = myword;
-          }
-        } else if (valid) {
-          dd[(size_t)r * ow] = bit ? 1.f : 0.f;
-        }
+        if (valid) dd[(size_t)r * ow] = v > 0.5f ? 1.f : 0.f;
       }
     }
   }
 }
 
 // ------------------------------------------------------------------------------------------------ packed + upsampled
-// The throughput form (bit planes of the upsampled masks) has kernels of its own.  What they share:
-//   * the binning kernel records every slot's kept proto range (so nobody recomputes it from the box), zeroes the
-//     per-slot piece counters and lists the detections that do not fit the patch path (kept range over 16 x 16 proto
-//     pixels, or an overfull region list): those go to the per-detection kernel of mask.cu afterwards;
+// The throughput form (bit planes of the upsampled masks) has kernels of its own:
+//   * the binning kernel records every slot's kept proto range (so nobody recomputes it from the box) and lists the
+//     detections that do not fit the patch path (kept range over 16 x 16 proto pixels, or an overfull region list):
+//     those ride in the region launch (ListedRide), their words cleared beforehand by pm_clear_listed_kernel;
 //   * upsample_pack_v2: one warp per detection.  The sigmoid patch sits in shared memory with a ring of zeros (the
 //     crop).  x pass with lane = output column (two taps per source row), results stored TRANSPOSED; y pass with lane =
 //     output ROW: every lane walks the columns of its row, blends two of the stored values per pixel and sets the bit
 //     in a register -- 7 instructions per column for 32 rows at once, no ballots, no row tables, one coalesced store
-//     of the row words.  (The first version ran lane = column with a ballot per row: ~13 instructions per row and a
-//     special case for narrow tail words; 1 000 warp instructions per detection, 70 % of the issue slots.)
-constexpr int kFuWarps = 8;
-constexpr int kFuThreads = kFuWarps * 32;
-constexpr int kFuRows = kPatchPitch + 2;   // ringed source rows
-constexpr int kXRows = 20;                 // source rows the x pass may compute (src_rows rounded up to a multiple of 4)
+//     of the row words.  (mask_upsample_pack_kernel runs lane = column with a ballot per row: ~13 instructions per row
+//     and a special case for narrow tail words; 1 000 warp instructions per detection, 70 % of the issue slots.)
+constexpr int kV2Warps = 8;
+constexpr int kV2Threads = kV2Warps * 32;
+constexpr int kXRows = 20;                // source rows the x pass may compute (src_rows rounded up to a multiple of 4)
 // x-pass results of the current 32 output columns, stored for the y pass as PAIRS of adjacent columns:
 // [column >> 1][source row][column & 1], kPairPitch floats per column pair.  The y pass (lane = output row) reads
 // the two columns of a pair with one 64-bit load and multiplies them with one packed FMUL2 (sm_100 f32x2: two IEEE
@@ -523,7 +494,7 @@ __device__ __forceinline__ void f32x2_mul(unsigned long long a, unsigned long lo
 // Only what the taps can reach has to be zero: ring rows 0 and ph + 1 (columns 0 .. pw + 1) and the two ring columns
 // of the rows in between.  Entries past the kept range that a float4 copy of a workspace row drags in are never read.
 __device__ __forceinline__ void up_zero_ring(float* P, int pw, int ph, int lane) {
-  if (lane < kFuRows) {
+  if (lane < kPatchRing) {
     P[kUpX0 - 1 + lane] = 0.f;                              // ring row 0
     P[(ph + 1) * kUpPitch + kUpX0 - 1 + lane] = 0.f;        // ring row ph + 1
     if (lane < ph) {
@@ -534,14 +505,13 @@ __device__ __forceinline__ void up_zero_ring(float* P, int pw, int ph, int lane)
 }
 
 // workspace patch (pitch 16, [ph][pw] valid) -> ringed shared-memory patch: one float4 per lane and 8 rows
-template <bool CG>
 __device__ __forceinline__ void up_load_patch(float* P, const float* __restrict__ src, int pw, int ph, int lane) {
   const int row = lane >> 2, quad = lane & 3;
   const float4* s4 = reinterpret_cast<const float4*>(src);
   float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a;
   const bool ra = row < ph, rb = row + 8 < ph;
-  if (ra) a = CG ? __ldcg(s4 + row * 4 + quad) : s4[row * 4 + quad];
-  if (rb) b = CG ? __ldcg(s4 + (row + 8) * 4 + quad) : s4[(row + 8) * 4 + quad];
+  if (ra) a = s4[row * 4 + quad];
+  if (rb) b = s4[(row + 8) * 4 + quad];
   if (ra) *reinterpret_cast<float4*>(P + (row + 1) * kUpPitch + kUpX0 + quad * 4) = a;
   if (rb) *reinterpret_cast<float4*>(P + (row + 9) * kUpPitch + kUpX0 + quad * 4) = b;
   __syncwarp();
@@ -636,12 +606,10 @@ __global__ void __launch_bounds__(256) proto_bin_fused_kernel(const float4* __re
                                                               int max_det, int mh, int mw, int rxn, int ryn, float rx,
                                                               float ry, const int32_t* __restrict__ geom4,
                                                               RegionList* __restrict__ regions, int4* __restrict__ kr,
-                                                              int32_t* __restrict__ done,
                                                               int32_t* __restrict__ large_count,
                                                               int32_t* __restrict__ large_list) {
   const long long slot = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (slot >= n_slots) return;
-  done[slot] = 0;
   const int tile = (int)(slot / max_det), d = (int)(slot - (long long)tile * max_det);
   // empty window, not KEPT (slide form) or beyond counts: no patch, an empty kept range
   const bool live = d < counts[tile] && geom4[4 * slot + 2] > 0 && geom4[4 * slot + 3] > 0;
@@ -683,14 +651,14 @@ __global__ void pm_clear_listed_kernel(const int32_t* __restrict__ geom4, const 
   }
 }
 
-// phase 2 of the two-kernel form: one warp per detection, patch from the workspace
-__global__ void __launch_bounds__(kFuThreads) mask_upsample_pack2_kernel(
+// phase 2 of the packed + upsampled form: one warp per detection, patch from the workspace
+__global__ void __launch_bounds__(kV2Threads) mask_upsample_pack2_kernel(
     const float* __restrict__ patches, const int4* __restrict__ krs, const int32_t* __restrict__ geom4,
     const int64_t* __restrict__ offsets, long long n_slots, int mh, int mw, float sxs, float sys,
     uint32_t* __restrict__ bits, long long capacity_words, int32_t* __restrict__ status) {
-  __shared__ __align__(16) UpWarpSmem S[kFuWarps];
+  __shared__ __align__(16) UpWarpSmem S[kV2Warps];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const long long slot = (long long)blockIdx.x * kFuWarps + warp;
+  const long long slot = (long long)blockIdx.x * kV2Warps + warp;
   if (slot >= n_slots) return;
   const int4 kr = krs[slot];
   const int pw = kr.z - kr.x, ph = kr.w - kr.y;
@@ -702,140 +670,9 @@ __global__ void __launch_bounds__(kFuThreads) mask_upsample_pack2_kernel(
     return;
   }
   float* P = S[warp].patch;
-  up_load_patch<false>(P, patches + slot * (kPatchPitch * kPatchPitch), pw, ph, lane);
+  up_load_patch(P, patches + slot * (kPatchPitch * kPatchPitch), pw, ph, lane);
   __syncwarp();
   upsample_pack_v2(P, S[warp].colT, kr, wdw, off, bits, mh, mw, sxs, sys, lane);
-}
-
-// ------------------------------------------------------------------------------------------------ fused path
-// Phases 1 and 2 in ONE persistent kernel.  The two phases want different resources -- phase 1 waits on HBM (TMA
-// regions), phase 2 on issue slots -- and as two kernels they run back to back.  Here
-//   * two CTAs per SM (8 warps, one 72 KB region buffer each) walk the (tile, region) items handed out by a global
-//     counter: while one CTA waits for its region (TMA) and for the dependent loads of its first pieces, the other
-//     computes; the ticket of the next item is drawn at the start of an item and looked at only at its end;
-//   * a warp takes the next piece of the item (dynamic, shared-memory counter) and contracts it.  A detection that
-//     lies inside ONE region (about half of them) goes straight from the contraction into the warp's shared-memory
-//     patch and is upsampled and packed on the spot: no workspace, no fence, no atomic.  A piece of a detection that
-//     straddles regions is written to the detection's patch in the L2-resident workspace and counted; the warp that
-//     writes the LAST piece fetches the patch back and upsamples it.  The issue-bound half of the work thus fills
-//     the cycles the other warps of the SM spend waiting for their region.
-template <typename E>
-struct FuSmem {
-  E proto[kRegNm][kRegBoxY][kRegBoxX];  // TMA destination
-  float coef[kFuWarps][kRegNm];
-  UpWarpSmem up[kFuWarps];
-  uint64_t full;
-  int item;
-  int next_piece;
-};
-
-template <typename E>
-__global__ void __launch_bounds__(kFuThreads, 2) mask_fused_kernel(
-    const __grid_constant__ CUtensorMap tmap, const float* __restrict__ coef, const int4* __restrict__ krs, int max_det,
-    int mh, int mw, float sxs, float sys, int rxn, int ryn, long long n_items, float* __restrict__ patches,
-    const RegionList* __restrict__ regions, int32_t* __restrict__ done, int32_t* __restrict__ work_counter,
-    const int32_t* __restrict__ geom4, const int64_t* __restrict__ offsets, uint32_t* __restrict__ bits,
-    long long capacity_words, int32_t* __restrict__ status) {
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  FuSmem<E>& S = *reinterpret_cast<FuSmem<E>*>(smem_raw);
-  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-  const int per_tile = rxn * ryn;
-  long long ticket = 0;  // thread 0: the next item's ticket, drawn one item ahead
-  if (t == 0) {
-    mbar_init(&S.full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    ticket = (long long)atomicAdd(work_counter, 1);
-  }
-  uint32_t parity = 0u;
-  float* P = S.up[warp].patch;
-  for (;;) {
-    if (t == 0) {
-      // resolve the ticket drawn an item ago (regions nobody reaches into are skipped: they load nothing)
-      while (ticket < n_items && regions[ticket].count <= 0) ticket = (long long)atomicAdd(work_counter, 1);
-      const int item = ticket < n_items ? (int)ticket : -1;
-      if (item >= 0) {
-        const int tile = item / per_tile, reg = item - tile * per_tile;
-        const int RY = reg / rxn, RX = reg - RY * rxn;
-        mbar_arrive_expect_tx(&S.full, (uint32_t)sizeof(S.proto));
-        tma_load_4d(&S.proto[0][0][0], &tmap, RX * kRegBoxX, RY * kRegBoxY, 0, tile, &S.full);
-        ticket = (long long)atomicAdd(work_counter, 1);  // used at the top of the next iteration only
-      }
-      S.item = item;
-      S.next_piece = 0;
-    }
-    __syncthreads();
-    const int cur = S.item;
-    if (cur < 0) break;
-    const int tile = cur / per_tile, reg = cur - tile * per_tile;
-    const int RY = reg / rxn, RX = reg - RY * rxn;
-    const int X0 = RX * kRegBoxX, Y0 = RY * kRegBoxY;
-    const RegionList& RL = regions[cur];
-    const int nl = min(RL.count, kRegCap);
-    // first piece of this warp: its kept range and coefficient are requested before the wait for the region
-    int e = 0;
-    if (lane == 0) e = atomicAdd(&S.next_piece, 1);
-    e = __shfl_sync(0xffffffffu, e, 0);
-    size_t nslot = 0;
-    int4 nkr = make_int4(0, 0, 0, 0);
-    float ncoef = 0.f;
-    auto fetch = [&](int ee) {
-      nslot = (size_t)tile * max_det + RL.det[ee];
-      nkr = krs[nslot];
-      ncoef = coef[nslot * kRegNm + lane];
-    };
-    if (e < nl) fetch(e);
-    while (!mbar_try_wait(&S.full, parity)) {
-    }
-    parity ^= 1u;
-    while (e < nl) {
-      const size_t slot = nslot;
-      const int4 k = nkr;
-      __syncwarp();
-      S.coef[warp][lane] = ncoef;
-      __syncwarp();
-      int en = 0;
-      if (lane == 0) en = atomicAdd(&S.next_piece, 1);
-      en = __shfl_sync(0xffffffffu, en, 0);
-      if (en < nl) fetch(en);  // the next piece's loads fly while this one is computed
-      e = en;
-      if (k.z <= k.x) continue;  // handed to the per-detection kernel by the binning pass (overfull region)
-      const bool single = k.x >= X0 && k.z <= X0 + kRegBoxX && k.y >= Y0 && k.w <= Y0 + kRegBoxY;
-      bool upsample = single;
-      float* pbase = patches + slot * (kPatchPitch * kPatchPitch);
-      if (single) {
-        // the whole kept range lies in this region: contraction -> shared-memory patch, nothing leaves the SM
-        up_zero_ring(P, k.z - k.x, k.w - k.y, lane);
-        contract_piece<E>(S.proto, S.coef[warp], k, X0, Y0, lane,
-                          [&](int px, int py, float v) { P[(py + 1) * kUpPitch + kUpX0 + px] = v; });
-      } else {
-        contract_piece<E>(S.proto, S.coef[warp], k, X0, Y0, lane,
-                          [&](int px, int py, float v) { __stcg(pbase + py * kPatchPitch + px, v); });
-        // this piece is on its way to L2; the warp that completes the detection's patch upsamples it
-        const int npieces = ((k.z - 1) / kRegBoxX - k.x / kRegBoxX + 1) * ((k.w - 1) / kRegBoxY - k.y / kRegBoxY + 1);
-        asm volatile("fence.acq_rel.gpu;" ::: "memory");
-        __syncwarp();
-        int last = 0;
-        if (lane == 0) last = (atomicAdd(&done[slot], 1) == npieces - 1) ? 1 : 0;
-        last = __shfl_sync(0xffffffffu, last, 0);
-        if (last) {
-          asm volatile("fence.acq_rel.gpu;" ::: "memory");
-          up_load_patch<true>(P, pbase, k.z - k.x, k.w - k.y, lane);
-          upsample = true;
-        }
-      }
-      if (upsample) {
-        __syncwarp();
-        const int4 wdw = reinterpret_cast<const int4*>(geom4)[slot];
-        const long long off = offsets[slot];
-        if (off + (long long)((wdw.z + 31) >> 5) * wdw.w > capacity_words) {
-          if (lane == 0) atomicOr(status, HDY_STATUS_OVERFLOW);
-        } else {
-          upsample_pack_v2(P, S.up[warp].colT, k, wdw, off, bits, mh, mw, sxs, sys, lane);
-        }
-      }
-    }
-    __syncthreads();  // every warp is done with the region buffer (and with S.item / S.next_piece)
-  }
 }
 
 int launch_process_mask_regions(const void* protos, int proto_dtype, const float* coef, const float* boxes,
@@ -850,7 +687,10 @@ int launch_process_mask_regions(const void* protos, int proto_dtype, const float
   const int esz = half ? 2 : 4;
   // TMA: the global address and every stride are multiples of 16 bytes; a tile origin too (24 pixels: 96 / 48 bytes)
   if (nm != kRegNm || (mw * esz & 15) != 0 || ((uintptr_t)protos & 15) != 0 || max_det > 65535) return 1;
-  if (getenv("HDY_MASK_GENERIC")) return 1;  // debugging aid: force the per-detection kernel
+  // the packed + upsampled kernels read the windows hdy_process_mask_geometry wrote; without them the per-detection
+  // kernel recomputes the windows
+  const bool packed = out_dense == nullptr;
+  if (packed && upsample && !geom) return 1;
   const int rxn = (mw + kRegBoxX - 1) / kRegBoxX, ryn = (mh + kRegBoxY - 1) / kRegBoxY;
   if ((long long)bs * rxn * ryn >= (1ll << 31) || slots >= (1ll << 31) || rxn * ryn > kMaxRegionsPerTile) return 1;
   EncodeTiledFn enc = tensor_map_encoder();
@@ -878,87 +718,28 @@ int launch_process_mask_regions(const void* protos, int proto_dtype, const float
     return HDY_ERR_CUDA;
   }
   const float4* b4 = reinterpret_cast<const float4*>(boxes);
-  // bit-packed + upsampled (the throughput form) has kernels of its own: HDY_MASK_PATH = "fused" (one persistent
-  // kernel for both phases), "2" (two kernels: regions -> patches, then upsample_pack_v2), "1" (the first version's
-  // kernels, kept for A/B runs); read per call
-  int path = 0;
-  if (out_dense == nullptr && upsample && geom) {
-    const char* v = getenv("HDY_MASK_PATH");
-    path = !v ? HDY_MASK_DEFAULT_PATH : (v[0] == 'f' ? 2 : (v[0] == '1' ? 0 : 1));
-  }
-  if (path != 0) {
+  if (packed && upsample) {
+    // bit-packed + upsampled (the throughput form): binning, the listed detections' words cleared (their tiles OR into
+    // them), regions -> patches with the listed detections riding in the same launch, then upsample_pack_v2
     const float sxs = (float)mw / (float)iw, sys = (float)mh / (float)ih;  // ATen: scale = in / out (fp32)
-    static int sm_count = 0;
-    if (!sm_count) {
-      int dev = 0;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
-      if (sm_count <= 0) sm_count = 148;
-    }
-    e = cudaMemsetAsync(W.work_counter, 0, 4, stream);
-    const size_t smem = half ? sizeof(FuSmem<__half>) : sizeof(FuSmem<float>);
-    if (e == cudaSuccess && path == 2)
-      e = half ? cudaFuncSetAttribute(mask_fused_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-               : cudaFuncSetAttribute(mask_fused_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) {
-      set_error("process_mask(packed) setup: %s", cudaGetErrorString(e));
-      return HDY_ERR_CUDA;
-    }
     proto_bin_fused_kernel<<<(unsigned)((slots + 255) / 256), 256, 0, stream>>>(
-        b4, counts, slots, max_det, mh, mw, rxn, ryn, rx, ry, geom, W.regions, W.kr, W.done, W.large_count,
-        W.large_list);
-    const long long n_items = (long long)bs * rxn * ryn;
-    if (path == 2) {
-      const unsigned grid = (unsigned)(n_items < 2ll * sm_count ? n_items : 2ll * sm_count);   // two CTAs per SM
-      if (half)
-        mask_fused_kernel<__half><<<grid, kFuThreads, smem, stream>>>(
-            map, coef, W.kr, max_det, mh, mw, sxs, sys, rxn, ryn, n_items, W.patches, W.regions, W.done,
-            W.work_counter, geom, offsets, bits, capacity_words, status);
-      else
-        mask_fused_kernel<float><<<grid, kFuThreads, smem, stream>>>(
-            map, coef, W.kr, max_det, mh, mw, sxs, sys, rxn, ryn, n_items, W.patches, W.regions, W.done,
-            W.work_counter, geom, offsets, bits, capacity_words, status);
-    } else {
-      // HDY_PATCH_SMEM=<bytes>: pad the region kernel's shared memory (e.g. 92160: two CTAs per SM instead of three,
-      // which leaves room for an upsample CTA of the previous batch on the same SM -- an A/B knob)
-      size_t psmem = half ? sizeof(RegSmemT<__half>) : sizeof(RegSmemT<float>);
-      if (const char* v = getenv("HDY_PATCH_SMEM")) {
-        const size_t want = (size_t)atol(v);
-        if (want > psmem && want <= 227 * 1024) {
-          psmem = want;
-          e = half ? cudaFuncSetAttribute(proto_patch_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)psmem)
-                   : cudaFuncSetAttribute(proto_patch_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)psmem);
-          if (e != cudaSuccess) {
-            set_error("process_mask(packed) setup: %s", cudaGetErrorString(e));
-            return HDY_ERR_CUDA;
-          }
-        }
-      }
-      // the listed detections' words are cleared first (their tiles OR into them), then they ride in the region launch
-      pm_clear_listed_kernel<<<148, 256, 0, stream>>>(geom, offsets, bits, capacity_words, W.large_list, W.large_count);
-      ListedRide LR;
-      LR.protos = protos, LR.boxes = b4, LR.offsets = offsets, LR.bits = bits, LR.status = status;
-      LR.list = W.large_list, LR.list_count = W.large_count, LR.capacity_words = capacity_words;
-      LR.rx = rx, LR.ry = ry, LR.nm = nm, LR.mh = mh, LR.mw = mw, LR.ih = ih, LR.iw = iw;
-      LR.ctas = kListedTiles * 9;
-      if (half)
-        proto_patch_kernel<__half><<<(unsigned)(n_items + LR.ctas), kRegThreads, psmem, stream>>>(
-            map, coef, W.kr, counts, max_det, rxn, ryn, W.patches, W.regions, LR);
-      else
-        proto_patch_kernel<float><<<(unsigned)(n_items + LR.ctas), kRegThreads, psmem, stream>>>(
-            map, coef, W.kr, counts, max_det, rxn, ryn, W.patches, W.regions, LR);
-      mask_upsample_pack2_kernel<<<(unsigned)((slots + kFuWarps - 1) / kFuWarps), kFuThreads, 0, stream>>>(
-          W.patches, W.kr, geom, offsets, slots, mh, mw, sxs, sys, bits, capacity_words, status);
-      return check_launch("hdy_process_mask(packed)");
-    }
+        b4, counts, slots, max_det, mh, mw, rxn, ryn, rx, ry, geom, W.regions, W.kr, W.large_count, W.large_list);
     pm_clear_listed_kernel<<<148, 256, 0, stream>>>(geom, offsets, bits, capacity_words, W.large_list, W.large_count);
-    int rcf = check_launch("hdy_process_mask(packed)");
-    if (rcf) return rcf;
-    return launch_process_mask_listed(protos, proto_dtype, coef, boxes, counts, max_det, nm, mh, mw, ih, iw, upsample,
-                                      rx, ry, nullptr, offsets, bits, capacity_words, status, W.large_list,
-                                      W.large_count, stream);
+    ListedRide LR;
+    LR.protos = protos, LR.boxes = b4, LR.offsets = offsets, LR.bits = bits, LR.status = status;
+    LR.list = W.large_list, LR.list_count = W.large_count, LR.capacity_words = capacity_words;
+    LR.rx = rx, LR.ry = ry, LR.nm = nm, LR.mh = mh, LR.mw = mw, LR.ih = ih, LR.iw = iw;
+    LR.ctas = kListedTiles * 9;
+    const unsigned g1 = (unsigned)((long long)bs * rxn * ryn + LR.ctas);
+    if (half)
+      proto_patch_kernel<__half><<<g1, kRegThreads, sizeof(RegSmemT<__half>), stream>>>(
+          map, coef, W.kr, counts, max_det, rxn, ryn, W.patches, W.regions, LR);
+    else
+      proto_patch_kernel<float><<<g1, kRegThreads, sizeof(RegSmemT<float>), stream>>>(
+          map, coef, W.kr, counts, max_det, rxn, ryn, W.patches, W.regions, LR);
+    mask_upsample_pack2_kernel<<<(unsigned)((slots + kV2Warps - 1) / kV2Warps), kV2Threads, 0, stream>>>(
+        W.patches, W.kr, geom, offsets, slots, mh, mw, sxs, sys, bits, capacity_words, status);
+    return check_launch("hdy_process_mask(packed)");
   }
   ListedRide no_ride;
   memset(&no_ride, 0, sizeof(no_ride));
@@ -971,15 +752,12 @@ int launch_process_mask_regions(const void* protos, int proto_dtype, const float
     proto_patch_kernel<float><<<(unsigned)((long long)bs * rxn * ryn), kRegThreads, sizeof(RegSmemT<float>), stream>>>(
         map, coef, W.kr, counts, max_det, rxn, ryn, W.patches, W.regions, no_ride);
   const unsigned g2 = (unsigned)((slots + kUpWarps - 1) / kUpWarps);
-  const bool packed = out_dense == nullptr;
 #define HDY_UP(P, U)                                                                                              \
   mask_upsample_pack_kernel<P, U><<<g2, kUpWarps * 32, 0, stream>>>(W.patches, b4, counts, slots, max_det, mh, mw, \
                                                                     ih, iw, rx, ry, out_dense, geom, offsets, bits, \
                                                                     capacity_words, status, W.large_count,         \
                                                                     W.large_list)
-  if (packed && upsample)
-    HDY_UP(true, true);
-  else if (packed)
+  if (packed)
     HDY_UP(true, false);
   else if (upsample)
     HDY_UP(false, true);

@@ -1,11 +1,11 @@
 // Per-tile greedy IoU NMS for tiles with at most 4096 candidates: one CTA per tile, everything in shared memory.
 // Exact torchvision.ops.nms semantics (called at metayolo/models/utils_general.py:342 and :507).
 //
-//   1. sort      bitonic sort of the 64-bit order keys (score desc, row asc), P/THREADS keys per thread in
-//                registers: strides inside a thread are plain compare-exchanges, strides inside a warp are
-//                shuffles, only the strides that cross warps go through shared memory (15 of the 78 steps at
-//                P = 4096).  Only keys move; the slot of every rank is recovered afterwards by a binary search of
-//                each candidate's (unique) key in the sorted array.
+//   1. sort      the 64-bit order keys (score desc, row asc).  Up to THREADS keys: a bitonic sort, one key per
+//                thread in a register; strides inside a warp are shuffles, only the strides that cross warps go
+//                through shared memory.  Only keys move; the slot of every rank is recovered afterwards by a binary
+//                search of each candidate's (unique) key in the sorted array.  More keys: an LSD radix sort in shared
+//                memory that moves keys and slots together.
 //   2. bin       boxes are fetched once (by slot, from L2), classified against a torus grid whose cell is the
 //                largest box side (2 x mean side if the sizes are very uneven; larger boxes go to one "large"
 //                bucket everybody scans), counted per cell, and copied into CELL ORDER (box + rank), each cell
@@ -21,7 +21,6 @@
 // Binning only prunes pairs that cannot intersect; every pair that can is tested with hdy_common.cuh's iou_gt
 // (fp32, torchvision's operation order), so cell size and bucket choice never change a verdict.
 #include <stddef.h>
-#include <stdlib.h>
 #include "hdy_common.cuh"
 
 namespace hdy {
@@ -104,120 +103,54 @@ __device__ __forceinline__ int block_excl_scan_cells(int* a, int len, int* warp_
   return total;
 }
 
-// Bitonic sort of P = THREADS * ITEMS keys; thread t owns elements t*ITEMS .. t*ITEMS+ITEMS-1.
-__device__ __forceinline__ void cmp_swap(uint64_t& a, uint64_t& b, bool up) {
-  const uint64_t lo = a < b ? a : b, hi = a < b ? b : a;
-  a = up ? lo : hi;
-  b = up ? hi : lo;
-}
-
-template <int THREADS, int ITEMS>
-__device__ __forceinline__ void bitonic_sort_regs(uint64_t (&k)[ITEMS], uint64_t* smem) {
-  static_assert(ITEMS == 1 || ITEMS == 2 || ITEMS == 4, "ITEMS must be 1, 2 or 4");
-  constexpr int P = THREADS * ITEMS;
+// Bitonic sort of THREADS keys, one per thread (thread t owns element t).
+template <int THREADS>
+__device__ __forceinline__ void bitonic_sort_regs(uint64_t& k, uint64_t* smem) {
   const int t = threadIdx.x;
-  const int i0 = t * ITEMS;
 #pragma unroll 1
-  for (int kk = 2; kk <= P; kk <<= 1) {
+  for (int kk = 2; kk <= THREADS; kk <<= 1) {
 #pragma unroll 1
-    for (int j = kk >> 1; j >= 32 * ITEMS; j >>= 1) {  // partner lives in another warp: through shared memory
+    for (int j = kk >> 1; j >= 32; j >>= 1) {  // partner lives in another warp: through shared memory
       __syncthreads();
-      uint64_t o[ITEMS];
-      // 128-bit shared-memory accesses: a warp moves 1 KB per instruction pair without bank conflicts
-      if (ITEMS == 4) {
-        ulonglong2* w = reinterpret_cast<ulonglong2*>(smem + i0);
-        w[0] = make_ulonglong2(k[0], k[1 % ITEMS]);
-        w[1] = make_ulonglong2(k[2 % ITEMS], k[3 % ITEMS]);
-        __syncthreads();
-        const ulonglong2* r = reinterpret_cast<const ulonglong2*>(smem + (i0 ^ j));
-        const ulonglong2 r0 = r[0], r1 = r[1];
-        o[0] = r0.x;
-        o[1 % ITEMS] = r0.y;
-        o[2 % ITEMS] = r1.x;
-        o[3 % ITEMS] = r1.y;
-      } else if (ITEMS == 2) {
-        *reinterpret_cast<ulonglong2*>(smem + i0) = make_ulonglong2(k[0], k[1 % ITEMS]);
-        __syncthreads();
-        const ulonglong2 r0 = *reinterpret_cast<const ulonglong2*>(smem + (i0 ^ j));
-        o[0] = r0.x;
-        o[1 % ITEMS] = r0.y;
-      } else {
-        smem[i0] = k[0];
-        __syncthreads();
-        o[0] = smem[i0 ^ j];
-      }
-      const bool keep_min = ((i0 & j) == 0) == ((i0 & kk) == 0);  // same for all ITEMS elements (j, kk >= ITEMS)
-#pragma unroll
-      for (int e = 0; e < ITEMS; ++e) {
-        const uint64_t a = k[e], b = o[e];
-        k[e] = keep_min ? (a < b ? a : b) : (a > b ? a : b);
-      }
+      smem[t] = k;
+      __syncthreads();
+      const uint64_t o = smem[t ^ j];
+      const bool keep_min = ((t & j) == 0) == ((t & kk) == 0);
+      k = keep_min ? (k < o ? k : o) : (k > o ? k : o);
     }
-    {
-      const int jmax = min(kk >> 1, 16 * ITEMS);
+    const int jmax = min(kk >> 1, 16);
 #pragma unroll 1
-      for (int j = jmax; j >= ITEMS; j >>= 1) {          // partner lives in another lane: shuffles
-        const int lj = j / ITEMS;
-        const bool keep_min = ((i0 & j) == 0) == ((i0 & kk) == 0);
-#pragma unroll
-        for (int e = 0; e < ITEMS; ++e) {
-          const uint64_t a = k[e];
-          const uint64_t b = __shfl_xor_sync(0xffffffffu, a, lj);
-          k[e] = keep_min ? (a < b ? a : b) : (a > b ? a : b);
-        }
-      }
-    }
-    // partners inside the thread (constant register indices)
-    if (ITEMS == 4) {
-      if (kk >= 4) {
-        const bool up = (i0 & kk) == 0;  // kk >= 4: one direction for the whole thread
-        cmp_swap(k[0], k[2 % ITEMS], up);
-        cmp_swap(k[1 % ITEMS], k[3 % ITEMS], up);
-        cmp_swap(k[0], k[1 % ITEMS], up);
-        cmp_swap(k[2 % ITEMS], k[3 % ITEMS], up);
-      } else {  // kk == 2: pairs (0,1) ascending, (2,3) descending
-        cmp_swap(k[0], k[1 % ITEMS], true);
-        cmp_swap(k[2 % ITEMS], k[3 % ITEMS], false);
-      }
-    } else if (ITEMS == 2) {
-      cmp_swap(k[0], k[1 % ITEMS], (i0 & kk) == 0);
+    for (int j = jmax; j >= 1; j >>= 1) {  // partner lives in another lane: shuffles
+      const bool keep_min = ((t & j) == 0) == ((t & kk) == 0);
+      const uint64_t o = __shfl_xor_sync(0xffffffffu, k, j);
+      k = keep_min ? (k < o ? k : o) : (k > o ? k : o);
     }
   }
 }
 
-template <int THREADS, int ITEMS>
+template <int THREADS>
 __device__ __forceinline__ void load_sort_store(const uint64_t* __restrict__ gkeys, int n_in, uint64_t* skey,
                                                 uint16_t* slot) {
   const int t = threadIdx.x;
-  uint64_t k[ITEMS], mine[ITEMS];
-#pragma unroll
-  for (int e = 0; e < ITEMS; ++e) {
-    const int i = t * ITEMS + e;
-    mine[e] = k[e] = (i < n_in) ? gkeys[i] : ~0ull;  // (~orderable(score) << 32) | row, unique inside a tile
-  }
-  bitonic_sort_regs<THREADS, ITEMS>(k, skey);
+  const uint64_t mine = (t < n_in) ? gkeys[t] : ~0ull;  // (~orderable(score) << 32) | row, unique inside a tile
+  uint64_t k = mine;
+  bitonic_sort_regs<THREADS>(k, skey);
   __syncthreads();
-#pragma unroll
-  for (int e = 0; e < ITEMS; ++e) skey[t * ITEMS + e] = k[e];
+  skey[t] = k;
   __syncthreads();
-  // rank of candidate i = position of its key in the sorted array (keys are unique)
-  constexpr int P = THREADS * ITEMS;
+  // rank of candidate t = position of its key in the sorted array (keys are unique)
+  if (t < n_in) {
+    int lo = 0;
 #pragma unroll
-  for (int e = 0; e < ITEMS; ++e) {
-    const int i = t * ITEMS + e;
-    if (i < n_in) {
-      int lo = 0;
-#pragma unroll
-      for (int step = P >> 1; step > 0; step >>= 1)
-        if (skey[lo + step] <= mine[e]) lo += step;
-      slot[lo] = (uint16_t)i;
-    }
+    for (int step = THREADS >> 1; step > 0; step >>= 1)
+      if (skey[lo + step] <= mine) lo += step;
+    slot[lo] = (uint16_t)t;
   }
   __syncthreads();
 }
 
-// ---- LSD radix sort of the tile's keys in shared memory (the default; the bitonic network above remains selectable
-// for A/B runs).  Eight 8-bit digits, least significant first, bytes that are equal in every key skipped (row indices
+// ---- LSD radix sort of the tile's keys in shared memory (tiles with more than THREADS keys; the bitonic network above
+// sorts the smaller ones).  Eight 8-bit digits, least significant first, bytes that are equal in every key skipped (row indices
 // below 65 536 leave two of them constant).  Per pass: every warp ranks its own contiguous run of keys with
 // ballots (stable: item e of lane l is element w*EPW + e*32 + l), leaving per-warp digit counts in `whist`; a column
 // scan over the 32 warps and a 256-entry scan give every (warp, digit) its base; keys and slots are scattered to the
@@ -420,7 +353,7 @@ __global__ void __maxnreg__(CAP <= 3072 ? 56 : 64) nms_tiles_smem_kernel(
     int max_nms, int max_det, int32_t* __restrict__ keep_idx, int32_t* __restrict__ keep_slot,
     float4* __restrict__ keep_box, float* __restrict__ keep_score, float* __restrict__ keep_cls,
     int32_t* __restrict__ keep_counts, float gray_eps, uint8_t* __restrict__ keep_fragile,
-    unsigned long long* __restrict__ phase_cycles, int sort_mode) {
+    unsigned long long* __restrict__ phase_cycles) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   FastSmemT<CAP>& S = *reinterpret_cast<FastSmemT<CAP>*>(smem_raw);
   // gray zone: pairs that this NMS leaves alone (IoU <= thr in tile coordinates) but whose IoU may exceed thr once both
@@ -458,16 +391,11 @@ __global__ void __maxnreg__(CAP <= 3072 ? 56 : 64) nms_tiles_smem_kernel(
   mark(-1);
 
   // ---- 1. sort ----------------------------------------------------------------------------------------------
-  static_assert(MAXR == 4 || MAXR == 3, "the sort dispatch below assumes 3 or 4 ranks per thread at full capacity");
-  // the sorting network wins up to 1024 keys (20.7 k vs 22.7 k cycles); its 4-keys-per-thread form needs 4096 slots
-  if ((sort_mode == 0 && n_in > THREADS) || (MAXR < 4 && n_in > 2 * THREADS))
+  // the sorting network wins up to THREADS = 1024 keys (20.7 k vs 22.7 k cycles), the radix sort above
+  if (n_in > THREADS)
     radix_sort_store<THREADS, CAP>(gkeys, n_in, S);
-  else if (n_in <= THREADS)
-    load_sort_store<THREADS, 1>(gkeys, n_in, S.skey, S.slot);
-  else if (n_in <= 2 * THREADS)
-    load_sort_store<THREADS, 2>(gkeys, n_in, S.skey, S.slot);
   else
-    load_sort_store<THREADS, 4>(gkeys, n_in, S.skey, S.slot);
+    load_sort_store<THREADS>(gkeys, n_in, S.skey, S.slot);
   mark(1);
 
   // ---- 2. boxes (one L2 gather, kept in registers), statistics, binning -------------------------------------
@@ -800,7 +728,7 @@ static int launch_nms_instance(const uint64_t* cand_keys, const float4* cand_box
                                const int32_t* counts, int bs, int cap, float thr, float class_offset, int max_nms,
                                int max_det, int32_t* keep_idx, int32_t* keep_slot, float4* keep_box, float* keep_score,
                                float* keep_cls, int32_t* keep_counts, float gray_eps, uint8_t* keep_fragile,
-                               unsigned long long* phase_cycles, int sort_mode, cudaStream_t stream) {
+                               unsigned long long* phase_cycles, cudaStream_t stream) {
   // the attribute is per DEVICE: a process-wide flag would leave every GPU but the first without the opt-in
   static bool attr_set[64] = {};
   int dev_i = 0;
@@ -816,7 +744,7 @@ static int launch_nms_instance(const uint64_t* cand_keys, const float4* cand_box
   }
   nms_tiles_smem_kernel<kFastThreads, CAP><<<(unsigned)bs, kFastThreads, sizeof(FastSmemT<CAP>), stream>>>(
       cand_keys, cand_boxes, cand_cls, counts, cap, thr, class_offset, max_nms, max_det, keep_idx, keep_slot,
-      keep_box, keep_score, keep_cls, keep_counts, gray_eps, keep_fragile, phase_cycles, sort_mode);
+      keep_box, keep_score, keep_cls, keep_counts, gray_eps, keep_fragile, phase_cycles);
   return check_launch("hdy_nms_tiles(smem)");
 }
 
@@ -825,18 +753,14 @@ int launch_nms_tiles_smem(const uint64_t* cand_keys, const float4* cand_boxes, c
                           int max_det, int32_t* keep_idx, int32_t* keep_slot, float4* keep_box, float* keep_score,
                           float* keep_cls, int32_t* keep_counts, float gray_eps, uint8_t* keep_fragile,
                           unsigned long long* phase_cycles, cudaStream_t stream) {
-  static const int sort_mode = [] {  // HDY_NMS_SORT=bitonic selects the sorting network (A/B runs); default: radix
-    const char* v = getenv("HDY_NMS_SORT");
-    return (v && v[0] == 'b') ? 1 : 0;
-  }();
   // candidate lists of at most 3072 entries take the instance that leaves room for a filter CTA on the same SM
-  if (cap <= kFastCapSmall && !getenv("HDY_NMS_FULL"))
+  if (cap <= kFastCapSmall)
     return launch_nms_instance<kFastCapSmall>(cand_keys, cand_boxes, cand_cls, counts, bs, cap, thr, class_offset,
                                               max_nms, max_det, keep_idx, keep_slot, keep_box, keep_score, keep_cls,
-                                              keep_counts, gray_eps, keep_fragile, phase_cycles, sort_mode, stream);
+                                              keep_counts, gray_eps, keep_fragile, phase_cycles, stream);
   return launch_nms_instance<kFastCap>(cand_keys, cand_boxes, cand_cls, counts, bs, cap, thr, class_offset, max_nms,
                                        max_det, keep_idx, keep_slot, keep_box, keep_score, keep_cls, keep_counts,
-                                       gray_eps, keep_fragile, phase_cycles, sort_mode, stream);
+                                       gray_eps, keep_fragile, phase_cycles, stream);
 }
 
 }  // namespace hdy

@@ -268,15 +268,15 @@ def test_extra_channels_are_carried(cuda_device):
         assert torch.equal(out.extra[i, :k].cpu(), cat[i, rows, 9:])
 
 
-@pytest.mark.parametrize("kernel", ["tma", "sparse", "planar", "generic"])
+@pytest.mark.parametrize("kernel", ["tma", "planar", "generic"])
 @pytest.mark.parametrize("tile,bs,n_cand,conf", [(320, 3, 500, 0.25), (640, 2, 1000, 0.15), (160, 5, 60, 0.5)])
-def test_wide_rows_filters_equal_two_step_path(cuda_device, monkeypatch, tile, bs, n_cand, conf, kernel):
-    """no = 41 (32 mask coefficients behind the scores), through the TMA streamer and through the sector-sparse filter
-    (decode.cu, HDY_FILTER=sparse): same survivors, boxes, scores, labels and rows as decode_concat -> nms_per_image on
-    the same logits, and as the oracle on the device-decoded rows; ragged last chunks (160-px tiles: 1200 + 300 + 75
-    rows) and a level that contributes nothing included."""
-    monkeypatch.setenv("HDY_FILTER", kernel)
-    layout = 1 if kernel in ("planar", "generic") else 0          # conv-native [bs, na*no, ny, nx]: same logits
+def test_wide_rows_filters_equal_two_step_path(cuda_device, tile, bs, n_cand, conf, kernel):
+    """no = 41 (32 mask coefficients behind the scores), through the TMA streamer (layout 0), the planar filter
+    (conv-native layout 1) and the one-row-per-thread filter (layout 1 with level tensors 4 bytes off a 16-byte
+    boundary): same survivors, boxes, scores, labels and rows as decode_concat -> nms_per_image on the same logits, and
+    as the oracle on the device-decoded rows; ragged last chunks (160-px tiles: 1200 + 300 + 75 rows) and a level that
+    contributes nothing included."""
+    layout = 0 if kernel == "tma" else 1                          # conv-native [bs, na*no, ny, nx]: same logits
     dets = synth.nuclei_logits(bs, tile, 4, n_cand, seed=tile + bs, conf=conf, extra=32)
     dets[0][bs - 1, ..., 4] = -20.0                                # last tile: level 0 contributes nothing
     spec = hdy.HeadSpec(synth.ANCHORS_3, synth.STRIDES_3, nc=4, no=41)
@@ -284,6 +284,9 @@ def test_wide_rows_filters_equal_two_step_path(cuda_device, monkeypatch, tile, b
     raw = torch.cat([d.view(d.shape[0], -1, 41) for d in dets], 1)
     src = d0 if layout == 0 else [d.permute(0, 1, 4, 2, 3).reshape(d.shape[0], -1, d.shape[2], d.shape[3]).contiguous()
                                   for d in d0]
+    if kernel == "generic":
+        src = [torch.empty(d.numel() + 1, device=cuda_device)[1:].view(d.shape).copy_(d) for d in src]
+        assert all(d.data_ptr() % 16 == 4 for d in src)
     one = hdy.detect_postprocess(src, spec, conf, 0.45, 2000, layout=layout)
     cat = hdy.decode_concat(d0, spec)
     two = hdy.nms_per_image(cat, 4, conf, 0.45, 2000)
@@ -527,19 +530,17 @@ def test_kept_indices_from_raw_logits_match_torch_cuda_reference(cuda_device):
         hdy.set_iou_compare("cpu")
 
 
-def test_nms_instances_agree(cuda_device, monkeypatch):
-    """hdy_nms_tiles has two shared-memory instances (3072 candidates: 126 KB, shares an SM with a filter CTA; 4096:
-    168 KB).  The same candidate lists through both give identical survivors, and what the oracle keeps."""
+def test_nms_instances_agree(cuda_device):
+    """hdy_nms_tiles has two shared-memory instances, chosen by cap (<= 3072 candidates: 126 KB, shares an SM with a
+    filter CTA; 4096: 168 KB).  The same candidate lists through both give identical survivors, and what the oracle
+    keeps."""
     spec = hdy.HeadSpec(synth.ANCHORS_3, synth.STRIDES_3, nc=4)
     dets = synth.nuclei_logits(6, 1024, 4, 2900, seed=31, conf=0.25, generator_device="cuda")
     ref = None
-    for full in (False, True):
-        if full:
-            monkeypatch.setenv("HDY_NMS_FULL", "1")
-        else:
-            monkeypatch.delenv("HDY_NMS_FULL", raising=False)
-        out = hdy.detect_postprocess(dets, spec, 0.25, 0.45, 3072, cap=3072)
+    for cap in (3072, 4096):                                       # every list has <= 3072 candidates: the same lists
+        out = hdy.detect_postprocess(dets, spec, 0.25, 0.45, 3072, cap=cap)
         assert int(out.cand_counts[-1]) == 0 and int(out.cand_counts[:-1].max()) > 2900
+        assert int(out.cand_counts.max()) <= 3072
         got = (out.counts.clone(), out.rows.clone(), out.boxes.clone(), out.scores.clone())
         kc = got[0].cpu().tolist()
         if ref is None:
@@ -551,4 +552,3 @@ def test_nms_instances_agree(cuda_device, monkeypatch):
             assert torch.equal(got[0], ref[0])
             for i, k in enumerate(kc):
                 assert torch.equal(got[1][i, :k], ref[1][i, :k]) and torch.equal(got[2][i, :k], ref[2][i, :k])
-    monkeypatch.delenv("HDY_NMS_FULL", raising=False)

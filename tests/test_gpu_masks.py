@@ -329,11 +329,13 @@ def test_process_mask_full_size_config2(cuda_device):
                                                        (256, 256, 1024, 1024, 2650, 12, 36, False),
                                                        (64, 80, 250, 333, 300, 4, 120, False),
                                                        (128, 128, 512, 512, 700, 10, 70, True)])
-def test_packed_mask_kernel_paths_agree_bit_for_bit(cuda_device, monkeypatch, mh, mw, ih, iw, md, lo, hi, half):
-    """The bit-packed, upsampled form has three kernel paths (HDY_MASK_PATH: "1" = the first version's two kernels,
-    "2" = regions -> patches + upsample_pack_v2, "fused" = one persistent kernel): same geometry, same offsets, the
-    same bits -- including boxes too large for the patch path, crowded regions whose lists overflow, empty tiles and
+def test_packed_mask_kernel_paths_agree_bit_for_bit(cuda_device, mh, mw, ih, iw, md, lo, hi, half):
+    """The bit-packed, upsampled form runs regions -> patches + upsample_pack_v2, with the detections the patch path
+    leaves out riding in the region launch.  The per-detection kernel, reached by hdy_process_mask_packed without a
+    workspace (a) or without the windows (b, it recomputes them), must give the same bits on the same geometry and
+    offsets -- including boxes too large for the patch path, crowded regions whose lists overflow, empty tiles and
     non-integer scales."""
+    from hd_yolo_b200 import _lib, ops
     g = torch.Generator().manual_seed(mh + md)
     bs = 3
     protos = torch.randn((bs, 32, mh, mw), generator=g)
@@ -345,18 +347,25 @@ def test_packed_mask_kernel_paths_agree_bit_for_bit(cuda_device, monkeypatch, mh
                          _rand_boxes(g, md, ih, iw, lo, hi)])
     boxes[0, 3] = torch.tensor([5.0, 7.0, iw - 20.0, ih * 0.6])                       # huge: per-detection kernel
     counts = torch.tensor([md, md - 7, 0], dtype=torch.int32)
-    args = (protos.to(cuda_device), coef.to(cuda_device), boxes.to(cuda_device), counts.to(cuda_device), (ih, iw))
-    out = {}
-    for path in ("1", "2", "fused"):
-        monkeypatch.setenv("HDY_MASK_PATH", path)
-        pk = hm.process_mask_packed(*args, upsample=True)
-        pk.check()
-        out[path] = (pk.geom.clone(), pk.offsets.clone(), pk.bits.clone())
-    monkeypatch.delenv("HDY_MASK_PATH")
-    for path in ("2", "fused"):
-        for a, b, what in zip(out["1"], out[path], ("geom", "offsets", "bits")):
-            assert torch.equal(a, b), f"path {path}: {what} differ ({int((a != b).sum())} entries)"
-    assert int(out["1"][1][-1]) > 20 * (md - 7)
+    protos, coef, boxes, counts = (t.to(cuda_device) for t in (protos, coef, boxes, counts))
+    pk = hm.process_mask_packed(protos, coef, boxes, counts, (ih, iw), upsample=True)
+    pk.check()
+    words = int(pk.offsets[-1])
+    lib = _lib.load()
+    ws_bytes = lib.hdy_process_mask_workspace_bytes(bs, md)
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=cuda_device)
+    dtype = _lib.HDY_F16 if half else _lib.HDY_F32
+    for what, geom, workspace, nbytes in (("no workspace", pk.geom, None, 0), ("no geom", None, ws, ws_bytes)):
+        bits = torch.full((max(words, 1),), -1, dtype=torch.int32, device=cuda_device)
+        status = torch.zeros((1,), dtype=torch.int32, device=cuda_device)
+        _lib.check(lib.hdy_process_mask_packed(_lib.ptr(protos), dtype, _lib.ptr(coef), _lib.ptr(boxes),
+                                               _lib.ptr(counts), _lib.ptr(geom), _lib.ptr(pk.offsets), bs, md, 32, mh,
+                                               mw, ih, iw, 1, _lib.ptr(bits), words, _lib.ptr(status),
+                                               _lib.ptr(workspace), nbytes, ops._stream()))
+        assert int(status.item()) == 0, f"{what}: status {int(status.item())}"
+        d = bits[:words]
+        assert torch.equal(pk.bits, d), f"{what}: bits differ ({int((pk.bits != d).sum())} of {words} words)"
+    assert words > 20 * (md - 7)
 
 
 def test_mask_agreement_is_tight_inside_the_windows(cuda_device):
