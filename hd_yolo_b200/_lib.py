@@ -93,11 +93,7 @@ SIGNATURES = {
     "hdy_merge_dirty_tiles": (_i, [_vp, _vp, _vp, _i, _vp, _i, _vp, _vp]),
     "hdy_merge_workspace_bytes": (_sz, [_i64]),
     "hdy_merge_nms": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _f, _f, _i, _vp, _vp, _vp, _sz, _vp]),
-    "hdy_merge_build": (_i, [_vp, _vp, _vp, C.c_uint32, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _f, _f, _vp, _vp, _sz,
-                             _vp]),
     "hdy_merge_rounds": (_i, [_vp, _i64, _f, _i, _i, _vp]),
-    "hdy_merge_export_states": (_i, [_vp, _i64, _vp, _vp, _i64, _vp, _vp]),
-    "hdy_merge_import_states": (_i, [_vp, _i64, _i64, _vp, _i64, _vp]),
     "hdy_merge_finish": (_i, [_vp, _vp, _i64, _vp, _vp, _vp]),
     "hdy_seam_summary": (_i, [_vp, _i64, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp]),
     "hdy_seam_select": (_i, [_vp, _vp, _i64, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
@@ -106,9 +102,7 @@ SIGNATURES = {
     "hdy_seam_build": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _i64, _i64, _f, _f, _vp, _vp, _sz, _vp]),
     "hdy_seam_export": (_i, [_vp, _i64, _vp, _vp, _vp, _i, _vp, _vp]),
     "hdy_seam_import": (_i, [_vp, _i64, _i64, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
-    "hdy_merge_select": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _vp]),
     "hdy_sort_workspace_bytes": (_sz, [_i64]),
-    "hdy_sort_keys": (_i, [_vp, _vp, _vp, _i64, _vp, _sz, _vp]),
     "hdy_sort_keys_bytes": (_i, [_vp, _vp, _vp, _i64, _i, _i, _vp, _sz, _vp]),
     "hdy_merge_select_ordered": (_i, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp]),
     "hdy_rcnn_decode": (_i, [_vp, _vp, _i64, _i, _i64, _f, _f, _f, _f, _f, _vp, _vp]),

@@ -17,7 +17,7 @@
 //     higher-ranked box is SUPPRESSED, SUPPRESSED as soon as one of them is KEPT.  Rank = (score desc, global index
 //     asc), the order torchvision's stable sort visits boxes in; no global sort is needed for the verdicts;
 //   * multi-GPU: entries [n_local, n) are replicas of seam detections owned by other ranks; they take part in every
-//     test but their verdicts are imported from the owner between rounds (hdy_merge_export/import_states).
+//     test but their verdicts are imported from the owner between rounds (hdy_seam_export / hdy_seam_import).
 // The IoU arithmetic is hdy_common.cuh's iou_gt (fp32, torchvision's operation order).  Binning only prunes pairs
 // that cannot intersect, so it never changes a verdict.
 //
@@ -450,9 +450,9 @@ __global__ void merge_pick_cell_kernel(MergeStats* __restrict__ stats) {
 struct MergeIn {
   const float4* boxes;
   const float* scores;
-  const uint32_t* gidx;       // optional global index per entry (tie order); NULL: gidx_base + i
   const uint32_t* rep_gidx;   // optional global index of the replicas (entry n_local + k -> rep_gidx[k])
-  const uint32_t* gidx_base_dev;  // optional device copy of gidx_base (overrides it)
+  const uint32_t* gidx_base_dev;  // optional device global index of entry 0: own entry i ranks as *gidx_base_dev + i
+                                  // in score ties (NULL: i)
   int tile_base;              // tile_id[i] + tile_base indexes tile_cores / tile_dirty (ranks hold local tile ids)
   const int32_t* tile_id;     // optional
   const float4* tile_cores;   // optional [n_tiles] core rectangles (slide coordinates)
@@ -460,7 +460,6 @@ struct MergeIn {
   const float* margin;        // device float: largest overhang of any (not far-reaching) box over its tile
   const long long* n_dev;     // optional device count
   long long n_max, n_local;   // entries >= n_local are remote replicas
-  uint32_t gidx_base;
   float conf, thr;
 };
 
@@ -516,13 +515,8 @@ __global__ void merge_fill_kernel(const MergeIn in, const MergeStats* __restrict
       p = (uint32_t)atomicAdd(&cell[bucket], 1);
       cbox[p] = b;
       const bool remote = i >= in.n_local;
-      uint32_t gi;
-      if (remote && in.rep_gidx)
-        gi = in.rep_gidx[i - in.n_local];
-      else if (in.gidx)
-        gi = in.gidx[i];
-      else
-        gi = (in.gidx_base_dev ? *in.gidx_base_dev : in.gidx_base) + (uint32_t)i;
+      const uint32_t gi = (remote && in.rep_gidx) ? in.rep_gidx[i - in.n_local]
+                                                  : (in.gidx_base_dev ? *in.gidx_base_dev : 0u) + (uint32_t)i;
       ckey[p] = make_key(in.scores[i], gi);
       cstate[p] = remote ? (uint8_t)MS_REMOTE_UNKNOWN : (cls == 0 ? (uint8_t)MS_KEPT : (uint8_t)MS_UNKNOWN);
       blocked[p] = 0u;
@@ -532,15 +526,18 @@ __global__ void merge_fill_kernel(const MergeIn in, const MergeStats* __restrict
   }
 }
 
-// one round of the fixed point over cell-ordered positions
-__device__ __forceinline__ void merge_round_body(int bid, int nblk, const float4* __restrict__ cbox,
-                                                                    const uint64_t* __restrict__ ckey,
-                                                                    uint8_t* cstate, const int* __restrict__ cell,
-                                                                    MergeStats* stats, int G, float thr, int round,
+// One round of the fixed point over cell-ordered positions.  The two read-only directions of a round are kernels of
+// their own.  (Round 2 tried them as ONE launch -- block ranges of a fused kernel -- to save a dependent launch per
+// round at small per-rank sizes: no gain at N = 8, rounds 1.06 ms either way, and 5.8 -> 7.7 ms on one GPU, the
+// small-box part inheriting the large part's register count.)
+__global__ void __launch_bounds__(kMergeThreads) merge_round_kernel(const float4* __restrict__ cbox,
+                                                                    const uint64_t* __restrict__ ckey, uint8_t* cstate,
+                                                                    const int* __restrict__ cell, MergeStats* stats,
+                                                                    int G, float thr, int round,
                                                                     const uint32_t* __restrict__ blocked,
                                                                     const int32_t* __restrict__ ctile) {
   if (round > 0 && stats->unknown[round - 1] == 0) {
-    if (bid == 0 && threadIdx.x == 0) stats->unknown[round] = 0;
+    if (blockIdx.x == 0 && threadIdx.x == 0) stats->unknown[round] = 0;
     return;
   }
   const int NB = G * G + 1;
@@ -548,7 +545,7 @@ __device__ __forceinline__ void merge_round_body(int bid, int nblk, const float4
   const CellGeom g = cell_geom(stats);
   volatile uint8_t* vstate = cstate;
   int unknown = 0;
-  for (int p = bid * blockDim.x + threadIdx.x; p < large_begin; p += nblk * blockDim.x) {
+  for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < large_begin; p += gridDim.x * blockDim.x) {
     if (vstate[p] != MS_UNKNOWN) continue;
     const float4 bi = cbox[p];
     const uint64_t ki = ckey[p];
@@ -603,7 +600,7 @@ __device__ __forceinline__ void merge_round_body(int bid, int nblk, const float4
 // per entry.  A large box can intersect small boxes whose centre lies within half a cell of it, i.e. the cells
 // [floor((x1 - c/2) / cell), floor((x2 + c/2) / cell)] x [same in y]; the lanes share those cells (the whole grid if
 // the range wraps around the torus, the whole array if the coordinates are not finite) and the large bucket.
-__device__ __forceinline__ void merge_round_large_body(int bid, int nblk, const float4* __restrict__ cbox,
+__global__ void __launch_bounds__(kMergeThreads) merge_round_large_kernel(const float4* __restrict__ cbox,
                                                                           const uint64_t* __restrict__ ckey,
                                                                           uint8_t* cstate, const int* __restrict__ cell,
                                                                           MergeStats* stats, int G, float thr,
@@ -615,7 +612,7 @@ __device__ __forceinline__ void merge_round_large_body(int bid, int nblk, const 
   const CellGeom g = cell_geom(stats);
   volatile uint8_t* vstate = cstate;
   const int lane = threadIdx.x & 31;
-  const int warp = (bid * blockDim.x + threadIdx.x) >> 5, n_warps = (nblk * blockDim.x) >> 5;
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
   for (int p = large_begin + warp; p < n_active; p += n_warps) {
     if (vstate[p] != MS_UNKNOWN) continue;  // warp-uniform
     const float4 bi = cbox[p];
@@ -658,25 +655,6 @@ __device__ __forceinline__ void merge_round_large_body(int bid, int nblk, const 
         atomicAdd(&stats->unknown[round], 1);
     }
   }
-}
-
-// The two read-only directions of a round as kernels of their own.  (Round 2 tried them as ONE launch -- block ranges
-// of a fused kernel -- to save a dependent launch per round at small per-rank sizes: no gain at N = 8, rounds 1.06 ms
-// either way, and 5.8 -> 7.7 ms on one GPU, the small-box part inheriting the large part's register count.)
-__global__ void __launch_bounds__(kMergeThreads) merge_round_kernel(const float4* __restrict__ cbox,
-                                                                    const uint64_t* __restrict__ ckey, uint8_t* cstate,
-                                                                    const int* __restrict__ cell, MergeStats* stats,
-                                                                    int G, float thr, int round,
-                                                                    const uint32_t* __restrict__ blocked,
-                                                                    const int32_t* __restrict__ ctile) {
-  merge_round_body((int)blockIdx.x, (int)gridDim.x, cbox, ckey, cstate, cell, stats, G, thr, round, blocked, ctile);
-}
-__global__ void __launch_bounds__(kMergeThreads) merge_round_large_kernel(const float4* __restrict__ cbox,
-                                                                          const uint64_t* __restrict__ ckey,
-                                                                          uint8_t* cstate, const int* __restrict__ cell,
-                                                                          MergeStats* stats, int G, float thr,
-                                                                          int round) {
-  merge_round_large_body((int)blockIdx.x, (int)gridDim.x, cbox, ckey, cstate, cell, stats, G, thr, round);
 }
 
 // Large -> small direction of a round: ONE WARP per entry of the large bucket that is not SUPPRESSED walks the small
@@ -750,49 +728,11 @@ __global__ void merge_finish_kernel(const uint32_t* __restrict__ pos, const uint
   if (bad && status) atomicOr(status, HDY_STATUS_ROUNDS);
 }
 
-__global__ void merge_export_kernel(const uint32_t* __restrict__ pos, const uint8_t* __restrict__ cstate,
-                                    const uint8_t* __restrict__ state, const int64_t* __restrict__ sel, long long m,
-                                    uint8_t* __restrict__ out) {
-  for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < m; k += (long long)gridDim.x * blockDim.x) {
-    const int64_t i = sel[k];
-    const uint32_t p = pos[i];
-    out[k] = (p == 0xffffffffu) ? state[i] : cstate[p];
-  }
-}
-
-__global__ void merge_import_kernel(const uint32_t* __restrict__ pos, uint8_t* __restrict__ cstate, long long first,
-                                    const uint8_t* __restrict__ states, long long m) {
-  for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < m; k += (long long)gridDim.x * blockDim.x) {
-    const uint32_t p = pos[first + k];
-    if (p == 0xffffffffu) continue;
-    const uint8_t s = states[k];
-    cstate[p] = (s == MS_KEPT || s == MS_SUPPRESSED || s == MS_DROPPED) ? s : (uint8_t)MS_REMOTE_UNKNOWN;
-  }
-}
-
 // ------------------------------------------------------------------------------------------------
-// survivors -> keys (unordered compaction), LSD radix sort, gather
+// survivors -> keys in row order, LSD radix sort, gather
 // ------------------------------------------------------------------------------------------------
-__global__ void keep_keys_kernel(const uint8_t* __restrict__ state, const float* __restrict__ scores,
-                                 const long long* __restrict__ n_dev, long long n_max, uint64_t* __restrict__ keys,
-                                 int* __restrict__ count) {
-  const long long n = n_dev ? min(*n_dev, n_max) : n_max;
-  const long long span = (long long)gridDim.x * blockDim.x;
-  const long long iters = (n + span - 1) / span;
-  const int lane = threadIdx.x & 31;
-  for (long long it = 0; it < iters; ++it) {
-    const long long i = it * span + (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const bool k = i < n && state[i] == MS_KEPT;
-    const unsigned m = __ballot_sync(0xffffffffu, k);
-    int base = 0;
-    if (lane == 0 && m) base = atomicAdd(count, __popc(m));
-    base = __shfl_sync(0xffffffffu, base, 0);
-    if (k) keys[base + __popc(m & ((1u << lane) - 1u))] = make_key(scores[i], (uint32_t)i);
-  }
-}
-
-// Ordered variant: keys leave in ROW order, so that a stable sort on the score half alone (4 radix passes instead of 8)
-// already breaks ties by the lower row.  Blocks own contiguous row ranges: count -> scan of the block counts -> write.
+// Keys leave in ROW order, so that a stable sort on the score half alone (4 radix passes instead of 8) already breaks
+// ties by the lower row.  Blocks own contiguous row ranges: count -> scan of the block counts -> write.
 constexpr int kSelThreads = 256;
 constexpr int kSelMaxBlocks = 4096;
 
@@ -1303,25 +1243,27 @@ size_t hdy_merge_workspace_bytes(int64_t n_max) {
   return merge_layout(nullptr, n_max).bytes;
 }
 
-static int merge_build_common(MergeIn in, const float* tile_cores, uint8_t* state, void* workspace,
+// The build step of hdy_merge_nms and hdy_seam_build (`what` names the call in error messages): initial verdicts,
+// then the active entries copied into cell order.
+static int merge_build_common(const char* what, MergeIn in, const float* tile_cores, uint8_t* state, void* workspace,
                               size_t workspace_bytes, cudaStream_t st) {
   const int64_t n_max = in.n_max, n_local = in.n_local;
-  HDY_REQUIRE(n_max >= 0 && n_local >= 0 && n_local <= n_max, "hdy_merge_build: bad sizes");
-  HDY_REQUIRE(n_max < (1ll << 31), "hdy_merge_build: at most 2^31-1 detections per call");
-  HDY_REQUIRE(in.thr >= 0.f, "hdy_merge_build: iou_thres must be >= 0");
-  HDY_REQUIRE(workspace && workspace_bytes >= hdy_merge_workspace_bytes(n_max), "hdy_merge_build: workspace too small");
-  HDY_REQUIRE(!tile_cores || (in.tile_id && in.margin), "hdy_merge_build: tile_cores needs tile_id and margin");
+  HDY_REQUIRE(n_max >= 0 && n_local >= 0 && n_local <= n_max, "%s: bad sizes", what);
+  HDY_REQUIRE(n_max < (1ll << 31), "%s: at most 2^31-1 detections per call", what);
+  HDY_REQUIRE(in.thr >= 0.f, "%s: iou_thres must be >= 0", what);
+  HDY_REQUIRE(workspace && workspace_bytes >= hdy_merge_workspace_bytes(n_max), "%s: workspace too small", what);
+  HDY_REQUIRE(!tile_cores || (in.tile_id && in.margin), "%s: tile_cores needs tile_id and margin", what);
   MergeWs w = merge_layout(workspace, n_max > 0 ? n_max : 1);
   const size_t nb = (size_t)w.G * w.G + 2;
   cudaError_t e = cudaMemsetAsync(w.stats, 0, sizeof(MergeStats), st);
   if (e == cudaSuccess) e = cudaMemsetAsync(w.cell, 0, nb * 4, st);
   if (e != cudaSuccess) {
-    set_error("hdy_merge_build: cudaMemsetAsync: %s", cudaGetErrorString(e));
+    set_error("%s: cudaMemsetAsync: %s", what, cudaGetErrorString(e));
     return HDY_ERR_CUDA;
   }
   if (n_max == 0) return HDY_OK;
   HDY_REQUIRE(in.boxes && in.scores && state && (((uintptr_t)in.boxes | (uintptr_t)tile_cores) & 15) == 0,
-              "hdy_merge_build: NULL or misaligned pointer");
+              "%s: NULL or misaligned pointer", what);
   const unsigned blocks = blocks_for(n_max, kMergeThreads);
   merge_stats_kernel<<<blocks, kMergeThreads, 0, st>>>(in.boxes, in.scores, in.n_dev, n_max, in.conf, w.stats);
   merge_pick_cell_kernel<<<1, 32, 0, st>>>(w.stats);
@@ -1330,32 +1272,7 @@ static int merge_build_common(MergeIn in, const float* tile_cores, uint8_t* stat
   if (rc) return rc;
   merge_fill_kernel<<<blocks, kMergeThreads, 0, st>>>(in, w.stats, w.G, w.cell, state, w.cbox, w.ckey, w.cstate,
                                                       w.pos, w.blocked, w.ctile);
-  return check_launch("hdy_merge_build");
-}
-
-int hdy_merge_build(const float* boxes, const float* scores, const uint32_t* gidx, uint32_t gidx_base,
-                    const int32_t* tile_id, const float* tile_cores, const uint8_t* tile_dirty, const float* margin,
-                    const int64_t* n_dev,
-                    int64_t n_max, int64_t n_local, float conf_thres, float iou_thres, uint8_t* state,
-                    void* workspace, size_t workspace_bytes, hdy_stream_t stream) {
-  MergeIn in;
-  in.boxes = reinterpret_cast<const float4*>(boxes);
-  in.scores = scores;
-  in.gidx = gidx;
-  in.rep_gidx = nullptr;
-  in.gidx_base_dev = nullptr;
-  in.tile_base = 0;
-  in.tile_id = tile_id;
-  in.tile_cores = reinterpret_cast<const float4*>(tile_cores);
-  in.tile_dirty = tile_dirty;
-  in.margin = margin;
-  in.n_dev = reinterpret_cast<const long long*>(n_dev);
-  in.n_max = n_max;
-  in.n_local = n_local;
-  in.gidx_base = gidx_base;
-  in.conf = conf_thres;
-  in.thr = iou_thres;
-  return merge_build_common(in, tile_cores, state, workspace, workspace_bytes, (cudaStream_t)stream);
+  return check_launch(what);
 }
 
 // ---- multi-GPU seam exchange -------------------------------------------------------------------
@@ -1446,7 +1363,6 @@ int hdy_seam_build(const float* boxes, const float* scores, const uint32_t* rep_
   MergeIn in;
   in.boxes = reinterpret_cast<const float4*>(boxes);
   in.scores = scores;
-  in.gidx = nullptr;
   in.rep_gidx = rep_gidx;
   in.gidx_base_dev = reinterpret_cast<const uint32_t*>(meta + SM_GBASE);
   in.tile_base = tile_base;
@@ -1457,10 +1373,9 @@ int hdy_seam_build(const float* boxes, const float* scores, const uint32_t* rep_
   in.n_dev = reinterpret_cast<const long long*>(meta + SM_NTOTAL);
   in.n_max = n_max;
   in.n_local = n_local;
-  in.gidx_base = 0;
   in.conf = conf_thres;
   in.thr = iou_thres;
-  return merge_build_common(in, tile_cores, state, workspace, workspace_bytes, (cudaStream_t)stream);
+  return merge_build_common("hdy_seam_build", in, tile_cores, state, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int hdy_seam_export(void* workspace, int64_t n_max, const uint8_t* state, const int32_t* sel, const int32_t* my_block,
@@ -1518,35 +1433,28 @@ int hdy_merge_finish(void* workspace, const int64_t* n_dev, int64_t n_max, uint8
   return check_launch("hdy_merge_finish");
 }
 
-int hdy_merge_export_states(void* workspace, int64_t n_max, const uint8_t* state, const int64_t* sel, int64_t m,
-                            uint8_t* out, hdy_stream_t stream) {
-  HDY_REQUIRE(workspace && n_max >= 0 && m >= 0, "hdy_merge_export_states: bad arguments");
-  if (m == 0) return HDY_OK;
-  HDY_REQUIRE(state && sel && out, "hdy_merge_export_states: NULL pointer");
-  MergeWs w = merge_layout(workspace, n_max);
-  merge_export_kernel<<<blocks_for(m, 256), 256, 0, (cudaStream_t)stream>>>(w.pos, w.cstate, state, sel, m, out);
-  return check_launch("hdy_merge_export_states");
-}
-
-int hdy_merge_import_states(void* workspace, int64_t n_max, int64_t first, const uint8_t* states, int64_t m,
-                            hdy_stream_t stream) {
-  HDY_REQUIRE(workspace && n_max >= 0 && m >= 0 && first >= 0 && first + m <= n_max,
-              "hdy_merge_import_states: bad arguments");
-  if (m == 0) return HDY_OK;
-  HDY_REQUIRE(states != nullptr, "hdy_merge_import_states: NULL pointer");
-  MergeWs w = merge_layout(workspace, n_max);
-  merge_import_kernel<<<blocks_for(m, 256), 256, 0, (cudaStream_t)stream>>>(w.pos, w.cstate, first, states, m);
-  return check_launch("hdy_merge_import_states");
-}
-
 int hdy_merge_nms(const float* boxes, const float* scores, const int32_t* tile_id, const float* tile_cores,
                   const uint8_t* tile_dirty, const float* margin, const int64_t* n_dev, int64_t n_max, float conf_thres,
                   float iou_thres,
                   int max_rounds, uint8_t* state, int32_t* status, void* workspace, size_t workspace_bytes,
                   hdy_stream_t stream) {
   HDY_REQUIRE(max_rounds >= 1 && max_rounds <= kMaxRounds, "hdy_merge_nms: max_rounds out of range [1,%d]", kMaxRounds);
-  int rc = hdy_merge_build(boxes, scores, nullptr, 0, tile_id, tile_cores, tile_dirty, margin, n_dev, n_max, n_max,
-                           conf_thres, iou_thres, state, workspace, workspace_bytes, stream);
+  MergeIn in;
+  in.boxes = reinterpret_cast<const float4*>(boxes);
+  in.scores = scores;
+  in.rep_gidx = nullptr;
+  in.gidx_base_dev = nullptr;
+  in.tile_base = 0;
+  in.tile_id = tile_id;
+  in.tile_cores = reinterpret_cast<const float4*>(tile_cores);
+  in.tile_dirty = tile_dirty;
+  in.margin = margin;
+  in.n_dev = reinterpret_cast<const long long*>(n_dev);
+  in.n_max = n_max;
+  in.n_local = n_max;
+  in.conf = conf_thres;
+  in.thr = iou_thres;
+  int rc = merge_build_common("hdy_merge_nms", in, tile_cores, state, workspace, workspace_bytes, (cudaStream_t)stream);
   if (rc) return rc;
   rc = hdy_merge_rounds(workspace, n_max, iou_thres, 0, max_rounds, stream);
   if (rc) return rc;
@@ -1560,21 +1468,33 @@ size_t hdy_sort_workspace_bytes(int64_t n_max) {
   return align256((size_t)hist * 4) + align256(scan_scratch_ints(hist) * 4);
 }
 
-/* ascending LSD radix sort of 64-bit keys; result in `keys` (tmp is scratch of the same size) */
-static int sort_key_bytes(uint64_t* keys, uint64_t* tmp, const int32_t* n_dev, int64_t n_max, int first_byte,
-                          int n_bytes, void* workspace, size_t workspace_bytes, hdy_stream_t stream);
-
-int hdy_sort_keys(uint64_t* keys, uint64_t* tmp, const int32_t* n_dev, int64_t n_max, void* workspace,
-                  size_t workspace_bytes, hdy_stream_t stream) {
-  return sort_key_bytes(keys, tmp, n_dev, n_max, 0, 8, workspace, workspace_bytes, stream);
-}
-
 int hdy_sort_keys_bytes(uint64_t* keys, uint64_t* tmp, const int32_t* n_dev, int64_t n_max, int first_byte,
                         int n_bytes, void* workspace, size_t workspace_bytes, hdy_stream_t stream) {
   HDY_REQUIRE(first_byte >= 0 && n_bytes >= 0 && first_byte + n_bytes <= 8 && (n_bytes & 1) == 0,
               "hdy_sort_keys_bytes: bytes [%d, %d) -- an even number of bytes inside the key", first_byte,
               first_byte + n_bytes);
-  return sort_key_bytes(keys, tmp, n_dev, n_max, first_byte, n_bytes, workspace, workspace_bytes, stream);
+  HDY_REQUIRE(n_max >= 0 && n_max < (1ll << 31), "hdy_sort_keys_bytes: bad size");
+  if (n_max == 0) return HDY_OK;
+  HDY_REQUIRE(keys && tmp && workspace && workspace_bytes >= hdy_sort_workspace_bytes(n_max),
+              "hdy_sort_keys_bytes: NULL pointer or workspace too small");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int n_sub = (int)((n_max + kSortPerWarp - 1) / kSortPerWarp);
+  const long long hist_n = 256ll * n_sub;
+  int* hist = static_cast<int*>(workspace);
+  int* scratch = reinterpret_cast<int*>(static_cast<unsigned char*>(workspace) + align256((size_t)hist_n * 4));
+  const unsigned blocks = (unsigned)((n_sub + kSortWarps - 1) / kSortWarps);
+  uint64_t* src = keys;
+  uint64_t* dst = tmp;
+  for (int pass = first_byte; pass < first_byte + n_bytes; ++pass) {
+    sort_hist_kernel<<<blocks, kSortThreads, 0, st>>>(src, n_dev, (int)n_max, pass * 8, n_sub, hist);
+    int rc = device_exclusive_scan(hist, hist_n, scratch, nullptr, st);
+    if (rc) return rc;
+    sort_scatter_kernel<<<blocks, kSortThreads, 0, st>>>(src, n_dev, (int)n_max, pass * 8, n_sub, hist, dst);
+    uint64_t* t = src;
+    src = dst;
+    dst = t;
+  }
+  return check_launch("hdy_sort_keys_bytes");  // an even number of passes: the result is back in `keys`
 }
 
 int hdy_merge_select_ordered(const uint8_t* state, const float* scores, const int64_t* n_dev, int64_t n_max,
@@ -1600,48 +1520,6 @@ int hdy_merge_select_ordered(const uint8_t* state, const float* scores, const in
   select_scan_kernel<<<1, 1024, 0, st>>>(block_scratch, nblocks, count);
   select_write_kernel<<<nblocks, kSelThreads, 0, st>>>(state, scores, nd, n_max, chunk, block_scratch, keys);
   return check_launch("hdy_merge_select_ordered");
-}
-
-static int sort_key_bytes(uint64_t* keys, uint64_t* tmp, const int32_t* n_dev, int64_t n_max, int first_byte,
-                          int n_bytes, void* workspace, size_t workspace_bytes, hdy_stream_t stream) {
-  HDY_REQUIRE(n_max >= 0 && n_max < (1ll << 31), "hdy_sort_keys: bad size");
-  if (n_max == 0) return HDY_OK;
-  HDY_REQUIRE(keys && tmp && workspace && workspace_bytes >= hdy_sort_workspace_bytes(n_max),
-              "hdy_sort_keys: NULL pointer or workspace too small");
-  cudaStream_t st = (cudaStream_t)stream;
-  const int n_sub = (int)((n_max + kSortPerWarp - 1) / kSortPerWarp);
-  const long long hist_n = 256ll * n_sub;
-  int* hist = static_cast<int*>(workspace);
-  int* scratch = reinterpret_cast<int*>(static_cast<unsigned char*>(workspace) + align256((size_t)hist_n * 4));
-  const unsigned blocks = (unsigned)((n_sub + kSortWarps - 1) / kSortWarps);
-  uint64_t* src = keys;
-  uint64_t* dst = tmp;
-  for (int pass = first_byte; pass < first_byte + n_bytes; ++pass) {
-    sort_hist_kernel<<<blocks, kSortThreads, 0, st>>>(src, n_dev, (int)n_max, pass * 8, n_sub, hist);
-    int rc = device_exclusive_scan(hist, hist_n, scratch, nullptr, st);
-    if (rc) return rc;
-    sort_scatter_kernel<<<blocks, kSortThreads, 0, st>>>(src, n_dev, (int)n_max, pass * 8, n_sub, hist, dst);
-    uint64_t* t = src;
-    src = dst;
-    dst = t;
-  }
-  return check_launch("hdy_sort_keys");  // an even number of passes: the result is back in `keys`
-}
-
-int hdy_merge_select(const uint8_t* state, const float* scores, const int64_t* n_dev, int64_t n_max, uint64_t* keys,
-                     int32_t* count, hdy_stream_t stream) {
-  HDY_REQUIRE(n_max >= 0 && n_max < (1ll << 31) && count, "hdy_merge_select: bad arguments");
-  cudaStream_t st = (cudaStream_t)stream;
-  cudaError_t e = cudaMemsetAsync(count, 0, 4, st);
-  if (e != cudaSuccess) {
-    set_error("hdy_merge_select: %s", cudaGetErrorString(e));
-    return HDY_ERR_CUDA;
-  }
-  if (n_max == 0) return HDY_OK;
-  HDY_REQUIRE(state && scores && keys, "hdy_merge_select: NULL pointer");
-  keep_keys_kernel<<<blocks_for(n_max, 256), 256, 0, st>>>(state, scores, reinterpret_cast<const long long*>(n_dev),
-                                                           n_max, keys, count);
-  return check_launch("hdy_merge_select");
 }
 
 int hdy_merge_gather(const uint64_t* keys, const int32_t* count, int64_t max_det, const float* boxes,

@@ -1,8 +1,9 @@
-// Per-tile greedy IoU NMS, exact torchvision.ops.nms semantics, one CTA per tile.
+// Per-tile greedy IoU NMS for tiles with more than kNmsSmemCap (4 096) candidates, exact torchvision.ops.nms
+// semantics, one CTA per tile; smaller tiles are done by nms_tiles_smem_kernel (nms_smem.cu).
 //
 // torchvision's kernel builds a dense n x n/64 suppression bitmask in HBM and walks it
 // sequentially.  Nuclei are small boxes on a large tile, so almost every pair is disjoint; this
-// kernel never forms the matrix.  Per tile, entirely in shared memory (n <= kSmemCap):
+// kernel never forms the matrix.  Per tile, on a global-memory workspace (hdy_nms_workspace_bytes):
 //   1. bitonic sort of (key, slot) pairs; ascending key == descending score, ties by lower index
 //      (== scores.sort(stable, descending), the order torchvision visits boxes in);
 //   2. boxes gathered into rank order; cell size c = 2 x mean box extent (block reduction);
@@ -14,7 +15,6 @@
 //      at 3x3 cells + the large bucket.  The fixed point equals sequential greedy NMS; the number
 //      of rounds is the longest suppression chain (a handful for nuclei);
 //   5. rank-ordered compaction of KEPT boxes, first max_det.
-// Tiles with more than kSmemCap candidates run the same code on a global-memory workspace.
 // The grid/cell choice only affects speed, never the result: the IoU test itself is exact
 // (hdy_common.cuh: iou_gt) and is evaluated for every pair that can possibly intersect.
 #include "hdy_common.cuh"
@@ -22,35 +22,14 @@
 namespace hdy {
 
 constexpr int kNmsThreads = 512;
-constexpr int kSmemCap = 4096;
-constexpr int kGridSmem = 32;    // torus grid side, shared-memory path
-constexpr int kGridGlobal = 64;  // torus grid side, workspace path
+constexpr int kGridGlobal = 64;  // torus grid side
 constexpr float kCellMargin = 1.01f;
 constexpr float kMaxScaled = 16384.0f;  // |centre|/cell above this -> "large" bucket (fp32 safety)
 
 enum : uint8_t { ST_UNKNOWN = 0, ST_KEPT = 1, ST_SUPPRESSED = 2 };
 
-// Optional phase profile (hdy_debug_nms_phases): cycles summed over CTAs for
-// 0 load, 1 sort, 2 gather boxes, 3 binning, 4 rounds, 5 output, 6 #rounds, 7 #CTAs
-__device__ unsigned long long* g_phase_cycles = nullptr;
-static unsigned long long* g_phase_host = nullptr;  // same pointer, for kernels that take it as a parameter
-struct PhaseClock {
-  unsigned long long* buf;
-  long long t0;
-  __device__ PhaseClock() : buf(g_phase_cycles), t0(0) {
-    if (buf && threadIdx.x == 0) t0 = clock64();
-  }
-  __device__ void mark(int phase) {
-    if (buf && threadIdx.x == 0) {
-      const long long t1 = clock64();
-      atomicAdd(buf + phase, (unsigned long long)(t1 - t0));
-      t0 = t1;
-    }
-  }
-  __device__ void add(int slot, unsigned long long v) {
-    if (buf && threadIdx.x == 0) atomicAdd(buf + slot, v);
-  }
-};
+// Optional phase profile of nms_tiles_smem_kernel (hdy_debug_nms_phases), passed to it as a kernel parameter
+static unsigned long long* g_phase_host = nullptr;
 
 __device__ __forceinline__ uint32_t next_pow2(uint32_t v) {
   if (v <= 1) return 1;
@@ -106,9 +85,8 @@ struct TileOut {
   uint8_t* keep_frag;  // optional: 1 for every survivor (this path does not analyse the gray zone; conservative)
 };
 
-template <typename IdxT, int G>
-__device__ void nms_tile_body(const int n_in, const int max_nms, uint64_t* keys, IdxT* slots, float4* boxes, uint8_t* state,
-                              IdxT* items, int* cell, int* warp_tmp, float* red_tmp,
+__device__ void nms_tile_body(const int n_in, const int max_nms, uint64_t* keys, uint32_t* slots, float4* boxes,
+                              uint8_t* state, uint32_t* items, int* cell, int* warp_tmp, float* red_tmp,
                               const uint64_t* __restrict__ gkeys, const float4* __restrict__ gboxes,
                               const float* __restrict__ gcls, const float class_offset, const float thr,
                               const int max_det, const TileOut out) {
@@ -118,15 +96,14 @@ __device__ void nms_tile_body(const int n_in, const int max_nms, uint64_t* keys,
   // (ties at the cut are resolved by lower index here; the reference's unstable argsort leaves
   //  them unspecified)
   const int n = (max_nms > 0 && n_in > max_nms) ? max_nms : n_in;
-  PhaseClock pc;
+  constexpr int G = kGridGlobal;
 
   // ---- 1. load + bitonic sort ------------------------------------------------------------------
   for (uint32_t i = t; i < P; i += T) {
     keys[i] = (i < (uint32_t)n_in) ? gkeys[i] : ~0ull;
-    slots[i] = (IdxT)i;
+    slots[i] = i;
   }
   __syncthreads();
-  pc.mark(0);
   for (uint32_t k = 2; k <= P; k <<= 1) {
     for (uint32_t j = k >> 1; j > 0; j >>= 1) {
       for (uint32_t p = t; p < (P >> 1); p += T) {
@@ -137,7 +114,7 @@ __device__ void nms_tile_body(const int n_in, const int max_nms, uint64_t* keys,
         if ((a > b) == up) {
           keys[i] = b;
           keys[x] = a;
-          const IdxT sa = slots[i];
+          const uint32_t sa = slots[i];
           slots[i] = slots[x];
           slots[x] = sa;
         }
@@ -146,12 +123,11 @@ __device__ void nms_tile_body(const int n_in, const int max_nms, uint64_t* keys,
     }
   }
 
-  pc.mark(1);
   // ---- 2. boxes into rank order (+ class offset), extent statistics ------------------------------
   float ext_sum = 0.f;
   int ext_cnt = 0;
   for (int r = t; r < n; r += T) {
-    const uint32_t s = (uint32_t)slots[r];
+    const uint32_t s = slots[r];
     float4 b = gboxes[s];
     if (gcls) {
       const float c = __fmul_rn(gcls[s], class_offset);  // c = x[:, 5:6] * max_wh   utils_general.py:505
@@ -173,7 +149,7 @@ __device__ void nms_tile_body(const int n_in, const int max_nms, uint64_t* keys,
     ext_sum += __shfl_xor_sync(0xffffffffu, ext_sum, o);
     ext_cnt += __shfl_xor_sync(0xffffffffu, ext_cnt, o);
   }
-  __syncthreads();  // keys region is dead from here on (state/items/cell alias it in the smem path)
+  __syncthreads();
   if ((t & 31) == 0) {
     red_tmp[t >> 5] = ext_sum;
     warp_tmp[t >> 5] = ext_cnt;
@@ -205,7 +181,6 @@ __device__ void nms_tile_body(const int n_in, const int max_nms, uint64_t* keys,
     return 2;  // also NaN / inf coordinates
   };
 
-  pc.mark(2);
   // ---- 3. counting sort into the torus grid ------------------------------------------------------
   constexpr int NB = G * G + 1;
   for (int i = t; i < NB; i += T) cell[i] = 0;
@@ -220,17 +195,15 @@ __device__ void nms_tile_body(const int n_in, const int max_nms, uint64_t* keys,
   block_excl_scan(cell, NB, warp_tmp);
   for (int r = t; r < n; r += T) {
     int bucket = 0;
-    if (classify(boxes[r], bucket)) items[atomicAdd(&cell[bucket], 1)] = (IdxT)r;
+    if (classify(boxes[r], bucket)) items[atomicAdd(&cell[bucket], 1)] = (uint32_t)r;
   }
   __syncthreads();
   // now: bucket b occupies items[ (b ? cell[b-1] : 0) .. cell[b] )
   const int large_begin = cell[NB - 2], large_end = cell[NB - 1];
 
-  pc.mark(3);
   // ---- 4. parallel greedy rounds -------------------------------------------------------------------
   volatile uint8_t* vstate = state;
   while (true) {
-    pc.add(6, 1);
     int unknown = 0;
     for (int r = t; r < n; r += T) {
       if (vstate[r] != ST_UNKNOWN) continue;
@@ -280,7 +253,6 @@ __device__ void nms_tile_body(const int n_in, const int max_nms, uint64_t* keys,
     if (!__syncthreads_or(unknown)) break;
   }
 
-  pc.mark(4);
   // ---- 5. rank-ordered compaction of survivors ----------------------------------------------------
   {
     const int items_per = (n + T - 1) / T;
@@ -304,7 +276,7 @@ __device__ void nms_tile_body(const int n_in, const int max_nms, uint64_t* keys,
     int pos = base + incl - cnt;
     for (int r = b; r < e && pos < max_det; ++r) {
       if (state[r] == ST_KEPT) {
-        const uint32_t s = (uint32_t)slots[r];
+        const uint32_t s = slots[r];
         const uint64_t k = gkeys[s];
         out.keep_idx[pos] = (int32_t)key_index(k);
         out.keep_slot[pos] = (int32_t)s;
@@ -317,8 +289,6 @@ __device__ void nms_tile_body(const int n_in, const int max_nms, uint64_t* keys,
     }
     if (t == 0) *out.keep_count = min(total, max_det);
   }
-  pc.mark(5);
-  pc.add(7, 1);
 }
 
 struct WorkspaceLayout {
@@ -348,27 +318,18 @@ __host__ __device__ inline WorkspaceLayout workspace_layout(int cap) {
   return L;
 }
 
-constexpr size_t kSmemBoxes = 0;
-constexpr size_t kSmemSlots = kSmemBoxes + (size_t)kSmemCap * 16;
-constexpr size_t kSmemA = kSmemSlots + (size_t)kSmemCap * 2;
-constexpr size_t kSmemBytes = kSmemA + (size_t)kSmemCap * 8;
-// region A after the sort: state (4 KB) | items (8 KB) | cell (G*G+4 ints)
-static_assert((size_t)kSmemCap + (size_t)kSmemCap * 2 + (kGridSmem * kGridSmem + 4) * 4 <= (size_t)kSmemCap * 8,
-              "aliased region does not fit");
-
 __global__ void __launch_bounds__(kNmsThreads, 2) nms_tiles_kernel(
     const uint64_t* __restrict__ cand_keys, const float4* __restrict__ cand_boxes,
     const float* __restrict__ cand_cls, const int32_t* __restrict__ counts, int cap, float thr,
     float class_offset, int max_nms, int max_det, int32_t* __restrict__ keep_idx,
     int32_t* __restrict__ keep_slot, float4* __restrict__ keep_box, float* __restrict__ keep_score,
     float* __restrict__ keep_cls, int32_t* __restrict__ keep_counts, unsigned char* __restrict__ workspace,
-    int min_n, uint8_t* __restrict__ keep_fragile) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
+    uint8_t* __restrict__ keep_fragile) {
   __shared__ int warp_tmp[kNmsThreads / 32 + 1];
   __shared__ float red_tmp[kNmsThreads / 32];
   const int tile = blockIdx.x;
   const int n = min(counts[tile], cap);
-  if (n <= min_n) return;  // done by nms_tiles_smem_kernel
+  if (n <= kNmsSmemCap) return;  // done by nms_tiles_smem_kernel
   TileOut out;
   out.keep_idx = keep_idx + (size_t)tile * max_det;
   out.keep_slot = keep_slot + (size_t)tile * max_det;
@@ -377,30 +338,14 @@ __global__ void __launch_bounds__(kNmsThreads, 2) nms_tiles_kernel(
   out.keep_cls = keep_cls ? keep_cls + (size_t)tile * max_det : nullptr;
   out.keep_count = keep_counts + tile;
   out.keep_frag = keep_fragile ? keep_fragile + (size_t)tile * max_det : nullptr;
-  if (n <= 0) {
-    if (threadIdx.x == 0) *out.keep_count = 0;
-    return;
-  }
   const uint64_t* gk = cand_keys + (size_t)tile * cap;
   const float4* gb = cand_boxes + (size_t)tile * cap;
   const float* gc = cand_cls ? cand_cls + (size_t)tile * cap : nullptr;
-  if (n <= kSmemCap) {
-    float4* boxes = reinterpret_cast<float4*>(smem_raw + kSmemBoxes);
-    uint16_t* slots = reinterpret_cast<uint16_t*>(smem_raw + kSmemSlots);
-    uint64_t* keys = reinterpret_cast<uint64_t*>(smem_raw + kSmemA);
-    uint8_t* state = smem_raw + kSmemA;
-    uint16_t* items = reinterpret_cast<uint16_t*>(smem_raw + kSmemA + kSmemCap);
-    int* cell = reinterpret_cast<int*>(smem_raw + kSmemA + (size_t)kSmemCap * 3);
-    nms_tile_body<uint16_t, kGridSmem>(n, max_nms, keys, slots, boxes, state, items, cell, warp_tmp, red_tmp, gk, gb,
-                                       gc, class_offset, thr, max_det, out);
-  } else {
-    const WorkspaceLayout L = workspace_layout(cap);
-    unsigned char* w = workspace + (size_t)tile * L.per_tile;
-    nms_tile_body<uint32_t, kGridGlobal>(
-        n, max_nms, reinterpret_cast<uint64_t*>(w + L.keys), reinterpret_cast<uint32_t*>(w + L.slots),
-        reinterpret_cast<float4*>(w + L.boxes), w + L.state, reinterpret_cast<uint32_t*>(w + L.items),
-        reinterpret_cast<int*>(w + L.cell), warp_tmp, red_tmp, gk, gb, gc, class_offset, thr, max_det, out);
-  }
+  const WorkspaceLayout L = workspace_layout(cap);
+  unsigned char* w = workspace + (size_t)tile * L.per_tile;
+  nms_tile_body(n, max_nms, reinterpret_cast<uint64_t*>(w + L.keys), reinterpret_cast<uint32_t*>(w + L.slots),
+                reinterpret_cast<float4*>(w + L.boxes), w + L.state, reinterpret_cast<uint32_t*>(w + L.items),
+                reinterpret_cast<int*>(w + L.cell), warp_tmp, red_tmp, gk, gb, gc, class_offset, thr, max_det, out);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -604,18 +549,12 @@ using namespace hdy;
 extern "C" {
 
 int hdy_debug_nms_phases(uint64_t* device_buf8) {
-  unsigned long long* p = reinterpret_cast<unsigned long long*>(device_buf8);
-  g_phase_host = p;
-  cudaError_t e = cudaMemcpyToSymbol(g_phase_cycles, &p, sizeof(p));
-  if (e != cudaSuccess) {
-    set_error("hdy_debug_nms_phases: %s", cudaGetErrorString(e));
-    return HDY_ERR_CUDA;
-  }
+  g_phase_host = reinterpret_cast<unsigned long long*>(device_buf8);
   return HDY_OK;
 }
 
 size_t hdy_nms_workspace_bytes(int bs, int cap) {
-  if (bs <= 0 || cap <= kSmemCap) return 0;
+  if (bs <= 0 || cap <= kNmsSmemCap) return 0;
   return (size_t)bs * workspace_layout(cap).per_tile;
 }
 
@@ -642,23 +581,10 @@ int hdy_nms_tiles(const uint64_t* cand_keys, const float* cand_boxes, const floa
                                  reinterpret_cast<float4*>(keep_box), keep_score, keep_cls, keep_counts, gray_eps,
                                  keep_fragile, g_phase_host, (cudaStream_t)stream);
   if (rc || cap <= kNmsSmemCap) return rc;
-  // the attribute is per DEVICE: a process-wide flag would leave every GPU but the first without the opt-in
-  static bool attr_set[64] = {};
-  int dev_i = 0;
-  cudaGetDevice(&dev_i);
-  if (dev_i < 0 || dev_i >= 64 || !attr_set[dev_i]) {
-    cudaError_t e = cudaFuncSetAttribute(nms_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)kSmemBytes);
-    if (e != cudaSuccess) {
-      set_error("cudaFuncSetAttribute(nms_tiles_kernel): %s", cudaGetErrorString(e));
-      return HDY_ERR_CUDA;
-    }
-    if (dev_i >= 0 && dev_i < 64) attr_set[dev_i] = true;
-  }
-  nms_tiles_kernel<<<(unsigned)bs, kNmsThreads, kSmemBytes, (cudaStream_t)stream>>>(
+  nms_tiles_kernel<<<(unsigned)bs, kNmsThreads, 0, (cudaStream_t)stream>>>(
       cand_keys, reinterpret_cast<const float4*>(cand_boxes), cand_cls, counts, cap, iou_thres, class_offset,
       max_nms, max_det, keep_idx, keep_slot, reinterpret_cast<float4*>(keep_box), keep_score, keep_cls,
-      keep_counts, static_cast<unsigned char*>(workspace), kNmsSmemCap, keep_fragile);
+      keep_counts, static_cast<unsigned char*>(workspace), keep_fragile);
   return check_launch("hdy_nms_tiles");
 }
 

@@ -53,7 +53,7 @@ def match_predictions(output: Dict[str, torch.Tensor], target: Dict[str, torch.T
     if k == 0:
         return {'order': torch.empty(0, **i64), 'scores': scores.reshape(0), 'labels': output['labels'].reshape(0), **empty}
     boxes = _aligned16(boxes.contiguous())
-    # 1. predictions by score: one ascending radix sort of the (~score, row) keys (hdy_sort_keys), row = low word
+    # 1. predictions by score: one ascending radix sort of the (~score, row) keys (hdy_sort_keys_bytes), row = low word
     from .slide import sort_keys
     scores = scores.contiguous()
     keys = torch.empty(k, dtype=torch.int64, device=dev)

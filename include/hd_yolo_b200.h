@@ -150,9 +150,10 @@ HDY_API int hdy_nms_tiles(const uint64_t* cand_keys, const float* cand_boxes, co
                   float* keep_cls, int32_t* keep_counts, float gray_eps, uint8_t* keep_fragile, void* workspace,
                   size_t workspace_bytes, hdy_stream_t stream);
 
-/* Debug: when device_buf8 (8 x u64, zeroed by the caller) is non-NULL, hdy_nms_tiles accumulates per-phase
- * SM cycles into it (0 load, 1 sort, 2 gather, 3 binning, 4 rounds, 5 output, 6 rounds run, 7 CTAs).
- * Pass NULL to switch it off (the default). Synchronises the device. */
+/* Debug: when device_buf8 (8 x u64, zeroed by the caller) is non-NULL, the following hdy_nms_tiles calls accumulate
+ * into it, over the tiles with at most 4096 candidates: 0 sweeps of the fixed point, SM cycles of 1 sort, 3 binning,
+ * 4 pairs, 5 resolve, 6 emit (2 stays 0), and 7 the number of such tiles.  Pass NULL to switch it off (the default).
+ * Only records the pointer: nothing is launched or synchronised. */
 HDY_API int hdy_debug_nms_phases(uint64_t* device_buf8);
 
 /* Keys for a plain torchvision.ops.nms(boxes, scores, thr) call: scores [bs, seg_len] ->
@@ -327,21 +328,11 @@ HDY_API int hdy_merge_nms(const float* boxes, const float* scores, const int32_t
                           float iou_thres, int max_rounds, uint8_t* state, int32_t* status, void* workspace,
                           size_t workspace_bytes, hdy_stream_t stream);
 
-/* The same in steps, for the multi-GPU seam exchange: rows [n_local, n_max) are replicas of detections owned by
- * other ranks (their verdicts are imported, never computed); gidx (or gidx_base + row) is the row's index in the
- * slide-wide concatenation, which breaks score ties exactly as the single-device call does.
- *   build -> { rounds(first_round, n_rounds) -> export_states(sel) -> [all-gather] -> import_states } ... -> finish */
-HDY_API int hdy_merge_build(const float* boxes, const float* scores, const uint32_t* gidx, uint32_t gidx_base,
-                            const int32_t* tile_id, const float* tile_cores, const uint8_t* tile_dirty,
-                            const float* margin,
-                            const int64_t* n_dev, int64_t n_max, int64_t n_local, float conf_thres, float iou_thres,
-                            uint8_t* state, void* workspace, size_t workspace_bytes, hdy_stream_t stream);
+/* hdy_merge_nms in steps, for the multi-GPU seam exchange below: after hdy_seam_build, hdy_merge_rounds runs rounds
+ * [first_round, first_round + n_rounds) of the fixed point (at most 64 in all) on the workspace, and hdy_merge_finish
+ * writes state [n_max] (rows not resolved by then: HDY_STATE_UNKNOWN and HDY_STATUS_ROUNDS in *status). */
 HDY_API int hdy_merge_rounds(void* workspace, int64_t n_max, float iou_thres, int first_round, int n_rounds,
                              hdy_stream_t stream);
-HDY_API int hdy_merge_export_states(void* workspace, int64_t n_max, const uint8_t* state, const int64_t* sel,
-                                    int64_t m, uint8_t* out, hdy_stream_t stream);
-HDY_API int hdy_merge_import_states(void* workspace, int64_t n_max, int64_t first, const uint8_t* states, int64_t m,
-                                    hdy_stream_t stream);
 HDY_API int hdy_merge_finish(void* workspace, const int64_t* n_dev, int64_t n_max, uint8_t* state, int32_t* status,
                              hdy_stream_t stream);
 
@@ -390,8 +381,12 @@ HDY_API int hdy_seam_scatter(const int32_t* payloads, const int32_t* summaries, 
 /* hdy_merge_dirty_tiles over every rank's far list (global tile ids, tile_rois of the whole slide). */
 HDY_API int hdy_seam_dirty_tiles(const int32_t* summaries, int world, int far_cap, const float* tile_rois, int n_tiles,
                                  uint8_t* dirty, hdy_stream_t stream);
-/* hdy_merge_build over own rows + replicas: row count, margin and global index base are read from meta; tile_id
- * [n_local] holds LOCAL tile ids (tile_id + tile_base indexes tile_cores / tile_dirty, which cover the whole slide). */
+/* First step of the merge (as hdy_merge_nms, with its conf_thres / iou_thres / interior shortcut) over the own rows
+ * [0, n_local) and the replicas behind them; the replicas take part in every pair test, but their verdicts are only
+ * ever imported.  Row count, margin and the global index of own row 0 are read from meta; a row's global index
+ * (replicas: rep_gidx) breaks score ties exactly as the single-device call does.  tile_id [n_local] holds LOCAL tile
+ * ids (tile_id + tile_base indexes tile_cores / tile_dirty, which cover the whole slide).  workspace:
+ * hdy_merge_workspace_bytes(n_max) bytes, kept for the later steps. */
 HDY_API int hdy_seam_build(const float* boxes, const float* scores, const uint32_t* rep_gidx, const int32_t* meta,
                            const int32_t* tile_id, int tile_base, const float* tile_cores, const uint8_t* tile_dirty,
                            int64_t n_max, int64_t n_local, float conf_thres, float iou_thres, uint8_t* state,
@@ -404,20 +399,15 @@ HDY_API int hdy_seam_import(void* workspace, int64_t n_max, int64_t n_local, con
                             const int32_t* payloads, int32_t* meta, int world, int rank, int seam_cap, int exchange,
                             hdy_stream_t stream);
 
-/* Survivors in the reference's order (`nms(...)[:max_det]`, yolo.py:195): select writes one 64-bit order key per
- * KEPT row (unordered) and their number, sort_keys sorts them ascending (== score-descending, ties by lower row),
- * gather emits the first max_det rows.  hdy_sort_keys is a plain LSD radix sort (8 passes of 8 bits), result in
- * `keys`, `tmp` is scratch of the same size. */
-HDY_API int hdy_merge_select(const uint8_t* state, const float* scores, const int64_t* n_dev, int64_t n_max,
-                             uint64_t* keys, int32_t* count, hdy_stream_t stream);
-HDY_API size_t hdy_sort_workspace_bytes(int64_t n_max);
-HDY_API int hdy_sort_keys(uint64_t* keys, uint64_t* tmp, const int32_t* n_dev, int64_t n_max, void* workspace,
-                          size_t workspace_bytes, hdy_stream_t stream);
-/* The same in fewer passes: select_ordered emits the keys in ROW order (block_scratch: 4096 device int32), so a
- * stable sort of the score half alone (sort_keys_bytes with first_byte = 4, n_bytes = 4: four of the eight passes)
- * leaves ties in row order -- the same result as select + sort_keys.  n_bytes must be even (result in `keys`). */
+/* Survivors in the reference's order (`nms(...)[:max_det]`, yolo.py:195): select_ordered -> sort_keys_bytes ->
+ * gather.  select_ordered writes one 64-bit order key (~orderable(score) << 32 | row) per KEPT row, in ROW order, and
+ * their number (block_scratch: 4096 device int32).  sort_keys_bytes is a stable ascending LSD radix sort of the bytes
+ * [first_byte, first_byte + n_bytes) of each key (one pass of 8 bits per byte; n_bytes even; result in `keys`, `tmp`
+ * is scratch of the same size): first_byte = 4, n_bytes = 4 sorts the score half alone and leaves ties in row order,
+ * i.e. score-descending, ties by lower row.  gather emits the first max_det rows. */
 HDY_API int hdy_merge_select_ordered(const uint8_t* state, const float* scores, const int64_t* n_dev, int64_t n_max,
                                      uint64_t* keys, int32_t* count, int32_t* block_scratch, hdy_stream_t stream);
+HDY_API size_t hdy_sort_workspace_bytes(int64_t n_max);
 HDY_API int hdy_sort_keys_bytes(uint64_t* keys, uint64_t* tmp, const int32_t* n_dev, int64_t n_max, int first_byte,
                                 int n_bytes, void* workspace, size_t workspace_bytes, hdy_stream_t stream);
 HDY_API int hdy_merge_gather(const uint64_t* keys, const int32_t* count, int64_t max_det, const float* boxes,
@@ -449,7 +439,7 @@ HDY_API int hdy_rcnn_filter_compact(const float* pred_boxes, const float* scores
                                     float* cand_cls, int32_t* counts, int32_t* status, hdy_stream_t stream);
 
 /* H2 (torchvision rpn.py filter_proposals), step 1: one 64-bit key per anchor so that ONE ascending sort
- * (hdy_sort_keys) leaves every (image, level) segment in place, best objectness logit first, ties by lower anchor.
+ * (hdy_sort_keys_bytes over all eight bytes) leaves every (image, level) segment in place, best objectness logit first, ties by lower anchor.
  *   objectness [N, A] logits, level_sizes_host [nl] anchors per level (sum = A, each <= 262144). */
 HDY_API int hdy_rpn_level_keys(const float* objectness, int N, int A, const int32_t* level_sizes_host, int nl,
                                uint64_t* keys, hdy_stream_t stream);

@@ -1,5 +1,5 @@
 """GPU parity tests of the sharded whole-slide merge: W ranks emulated on one device through the real C-ABI kernels
-(hdy_merge_build / rounds / export_states / import_states / finish) vs torchvision's dense NMS on the slide-wide
+(hdy_seam_* / hdy_merge_rounds / hdy_merge_finish) vs torchvision's dense NMS on the slide-wide
 concatenation (what Ensemble.merge computes, metayolo/models/yolo.py:189-195) and vs the single-device merge."""
 import os
 import sys
