@@ -25,6 +25,8 @@
 //   the first CTAs of the phase-1 launch; in the other forms they get a launch of their own behind phase 2.
 //   The packed + upsampled form needs the windows of hdy_process_mask_geometry; without them the caller falls back to
 //   the per-detection kernel.
+#include <algorithm>
+
 #include "tma_common.cuh"
 #include "mask_common.cuh"
 
@@ -49,8 +51,9 @@ struct RegSmemT {
 __device__ __forceinline__ float proto_f32(float v) { return v; }
 __device__ __forceinline__ float proto_f32(__half v) { return __half2float(v); }  // exact
 
-// workspace: [0] large-detection counter, large list (int32 per slot), the patches, then the per-region detection
-// lists (count + kRegCap uint16 entries per (tile, region); sized for the largest proto plane, see kMaxRegions)
+// workspace: [0] large-detection counter, [1] slot ticket of the packed upsample, large list (int32 per slot), the
+// patches, then the per-region detection lists (count + kRegCap uint16 entries per (tile, region); sized for the
+// largest proto plane, see kMaxRegions)
 constexpr int kRegCap = 254;          // detections listed per region; a region with more falls back to scanning
 constexpr int kMaxRegionsPerTile = 512;  // ceil(mw/24) * ceil(mh/24) <= 512 covers planes up to 528 x 528 (2112 px tiles)
 struct RegionList {
@@ -60,6 +63,7 @@ struct RegionList {
 static_assert(sizeof(RegionList) == 512, "one region list is 512 bytes");
 struct PmWorkspace {
   int32_t* large_count;   // detections left to the per-detection kernel
+  uint32_t* ticket;       // next slot of the packed + upsampled phase 2 (mask_upsample_pack2_kernel)
   int32_t* large_list;
   float* patches;
   RegionList* regions;
@@ -75,6 +79,7 @@ static PmWorkspace pm_workspace(void* base, long long slots) {
   PmWorkspace w;
   unsigned char* p = static_cast<unsigned char*>(base);
   w.large_count = reinterpret_cast<int32_t*>(p);
+  w.ticket = reinterpret_cast<uint32_t*>(p + 4);
   p += 256;
   w.large_list = reinterpret_cast<int32_t*>(p);
   p += align256((size_t)slots * 4);
@@ -651,28 +656,58 @@ __global__ void pm_clear_listed_kernel(const int32_t* __restrict__ geom4, const 
   }
 }
 
-// phase 2 of the packed + upsampled form: one warp per detection, patch from the workspace
-__global__ void __launch_bounds__(kV2Threads) mask_upsample_pack2_kernel(
+// phase 2 of the packed + upsampled form: one warp per detection, patch from the workspace.  Persistent: as many CTAs
+// as fit the GPU at once (6 per SM: 36 KB of shared memory and 256 x 40 registers each), every warp takes `chunk`
+// slots at a time from a ticket until none are left (chunk: about four tickets per warp, at most kV2Chunk -- one
+// atomic per slot would serialise on the ticket, a chunk larger than the work per warp leaves warps without any).
+// With one CTA per 8 slots, a CTA held its shared memory until its slowest warp was done, so the warps of dead slots
+// (beyond counts, not KEPT, listed: 16 % in the slide) and of small masks idled beside the large ones; the ticket
+// also hands the work of CTAs that start late (the SM still holding region CTAs of another stream) to those already
+// running.
+constexpr int kV2Chunk = 16;
+constexpr int kV2CtasPerSm = 6;
+__global__ void __launch_bounds__(kV2Threads, kV2CtasPerSm) mask_upsample_pack2_kernel(
     const float* __restrict__ patches, const int4* __restrict__ krs, const int32_t* __restrict__ geom4,
     const int64_t* __restrict__ offsets, long long n_slots, int mh, int mw, float sxs, float sys,
-    uint32_t* __restrict__ bits, long long capacity_words, int32_t* __restrict__ status) {
+    uint32_t* __restrict__ bits, long long capacity_words, int32_t* __restrict__ status,
+    uint32_t* __restrict__ ticket, int chunk) {
   __shared__ __align__(16) UpWarpSmem S[kV2Warps];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const long long slot = (long long)blockIdx.x * kV2Warps + warp;
-  if (slot >= n_slots) return;
-  const int4 kr = krs[slot];
-  const int pw = kr.z - kr.x, ph = kr.w - kr.y;
-  if (pw <= 0 || ph <= 0) return;  // dead / empty / handed to the per-detection kernel
-  const int4 wdw = reinterpret_cast<const int4*>(geom4)[slot];
-  const long long off = offsets[slot];
-  if (off + (long long)((wdw.z + 31) >> 5) * wdw.w > capacity_words) {
-    if (lane == 0) atomicOr(status, HDY_STATUS_OVERFLOW);
-    return;
-  }
   float* P = S[warp].patch;
-  up_load_patch(P, patches + slot * (kPatchPitch * kPatchPitch), pw, ph, lane);
-  __syncwarp();
-  upsample_pack_v2(P, S[warp].colT, kr, wdw, off, bits, mh, mw, sxs, sys, lane);
+  for (;;) {
+    uint32_t first = 0;
+    if (lane == 0) first = atomicAdd(ticket, (uint32_t)chunk);
+    first = __shfl_sync(0xffffffffu, first, 0);
+    if ((long long)first >= n_slots) return;
+    const long long last = min((long long)first + chunk, n_slots);
+    for (long long slot = first; slot < last; ++slot) {
+      const int4 kr = krs[slot];
+      const int pw = kr.z - kr.x, ph = kr.w - kr.y;
+      if (pw <= 0 || ph <= 0) continue;  // dead / empty / handed to the per-detection kernel
+      const int4 wdw = reinterpret_cast<const int4*>(geom4)[slot];
+      const long long off = offsets[slot];
+      if (off + (long long)((wdw.z + 31) >> 5) * wdw.w > capacity_words) {
+        if (lane == 0) atomicOr(status, HDY_STATUS_OVERFLOW);
+        continue;
+      }
+      __syncwarp();  // the previous slot's upsample is done with P
+      up_load_patch(P, patches + slot * (kPatchPitch * kPatchPitch), pw, ph, lane);
+      __syncwarp();
+      upsample_pack_v2(P, S[warp].colT, kr, wdw, off, bits, mh, mw, sxs, sys, lane);
+    }
+  }
+}
+
+// CTAs of mask_upsample_pack2_kernel that are resident at once on this device (0 on error)
+static int upsample_pack2_grid() {
+  int dev = 0, sms = 0, per_sm = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess ||
+      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
+      cudaFuncSetAttribute((const void*)mask_upsample_pack2_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                           cudaSharedmemCarveoutMaxShared) != cudaSuccess ||
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mask_upsample_pack2_kernel, kV2Threads, 0) != cudaSuccess)
+    return 0;
+  return sms * per_sm;
 }
 
 int launch_process_mask_regions(const void* protos, int proto_dtype, const float* coef, const float* boxes,
@@ -706,7 +741,7 @@ int launch_process_mask_regions(const void* protos, int proto_dtype, const float
                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return 1;
   const PmWorkspace W = pm_workspace(workspace, slots);
-  cudaError_t e = cudaMemsetAsync(W.large_count, 0, 4, stream);
+  cudaError_t e = cudaMemsetAsync(W.large_count, 0, 8, stream);  // large_count and ticket
   if (e == cudaSuccess) e = cudaMemsetAsync(W.regions, 0, (size_t)bs * rxn * ryn * sizeof(RegionList), stream);
   if (e == cudaSuccess)
     e = half ? cudaFuncSetAttribute(proto_patch_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -737,8 +772,15 @@ int launch_process_mask_regions(const void* protos, int proto_dtype, const float
     else
       proto_patch_kernel<float><<<g1, kRegThreads, sizeof(RegSmemT<float>), stream>>>(
           map, coef, W.kr, counts, max_det, rxn, ryn, W.patches, W.regions, LR);
-    mask_upsample_pack2_kernel<<<(unsigned)((slots + kV2Warps - 1) / kV2Warps), kV2Threads, 0, stream>>>(
-        W.patches, W.kr, geom, offsets, slots, mh, mw, sxs, sys, bits, capacity_words, status);
+    const int g2 = upsample_pack2_grid();
+    if (g2 <= 0) {
+      set_error("process_mask(packed): no occupancy for mask_upsample_pack2_kernel");
+      return HDY_ERR_CUDA;
+    }
+    const int chunk = (int)std::min<long long>(kV2Chunk, std::max<long long>(1, slots / (4ll * g2 * kV2Warps)));
+    mask_upsample_pack2_kernel<<<(unsigned)min((long long)g2, (slots + kV2Warps - 1) / kV2Warps), kV2Threads, 0,
+                                 stream>>>(W.patches, W.kr, geom, offsets, slots, mh, mw, sxs, sys, bits, capacity_words,
+                                           status, W.ticket, chunk);
     return check_launch("hdy_process_mask(packed)");
   }
   ListedRide no_ride;
