@@ -20,6 +20,7 @@
 // i0 = (int)src; i1 = min(i0+1, in-1); l1 = src-i0; l0 = 1-l1; v = l0y*(l0x*v00 + l1x*v01) + l1y*(l0x*v10 + l1x*v11).
 #include <stdlib.h>
 #include "mask_common.cuh"
+#include "scan_common.cuh"
 
 namespace hdy {
 
@@ -74,89 +75,22 @@ __device__ __forceinline__ PasteGeom paste_geometry(const float4 b, float scale,
   return g;
 }
 
-// words of the cropped bit plane per mask, then an exclusive scan -> offsets[K+1], in three launches and no scratch:
-//   1. every CTA scans its 1024 masks; the exclusive prefix of a CTA's first mask is 0 by construction, so that slot
-//      (offsets[(b+1)*1024], or offsets[K] for the last CTA) carries the CTA's TOTAL to the next step instead;
-//   2. one CTA turns those totals into running sums: offsets[b*1024] becomes the base of CTA b (its final value),
-//      offsets[K] the grand total;
-//   3. every CTA b >= 1 adds its base to its other 1023 slots.
-constexpr int kScanChunk = 1024;
-
-__device__ __forceinline__ long long block_incl_scan_ll(long long v, long long* warp_sum) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  long long incl = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    long long u = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += u;
-  }
-  if (lane == 31) warp_sum[warp] = incl;
-  __syncthreads();
-  if (warp == 0) {
-    long long s = warp_sum[lane], t = s;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      long long u = __shfl_up_sync(0xffffffffu, t, o);
-      if (lane >= o) t += u;
-    }
-    warp_sum[lane] = t - s;
-  }
-  __syncthreads();
-  const long long r = warp_sum[warp] + incl;
-  __syncthreads();
-  return r;
-}
-
-__global__ void __launch_bounds__(kScanChunk) scan_words_local_kernel(const int32_t* __restrict__ geom4, long long K,
-                                                                      int64_t* __restrict__ offsets) {
-  __shared__ long long warp_sum[32];
-  const long long i = (long long)blockIdx.x * kScanChunk + threadIdx.x;
-  long long v = 0;
-  if (i < K) v = (long long)((geom4[4 * i + 2] + 31) >> 5) * geom4[4 * i + 3];
-  const long long incl = block_incl_scan_ll(v, warp_sum);
-  if (i < K && threadIdx.x != 0) offsets[i] = incl - v;
-  const long long last = min((long long)(blockIdx.x + 1) * kScanChunk, K) - 1;  // last mask of this CTA
-  if (i == last) offsets[last + 1] = incl;                                       // CTA total -> next CTA's first slot
-  if (i == 0) offsets[0] = 0;
-}
-
-__global__ void __launch_bounds__(kScanChunk) scan_words_bases_kernel(long long K, int64_t* __restrict__ offsets) {
-  __shared__ long long warp_sum[32];
-  __shared__ long long carry;
-  const long long nb = (K + kScanChunk - 1) / kScanChunk;  // totals live at slots min((b+1)*1024, K), b = 0..nb-1
-  if (threadIdx.x == 0) carry = 0;
-  __syncthreads();
-  for (long long b0 = 0; b0 < nb; b0 += kScanChunk) {
-    const long long b = b0 + threadIdx.x;
-    const long long slot = min((b + 1) * kScanChunk, K);
-    const long long v = b < nb ? offsets[slot] : 0;
-    const long long incl = block_incl_scan_ll(v, warp_sum) + carry;
-    if (b < nb) offsets[slot] = incl;
-    __syncthreads();
-    if (threadIdx.x == kScanChunk - 1) carry = incl;
-    __syncthreads();
-  }
-}
-
-__global__ void __launch_bounds__(kScanChunk) scan_words_add_kernel(long long K, int64_t* __restrict__ offsets) {
-  const long long first = (long long)(blockIdx.x + 1) * kScanChunk;  // CTA 0 has base 0
-  const long long i = first + threadIdx.x;
-  if (threadIdx.x == 0 || i >= K) return;
-  offsets[i] += offsets[first];
-}
-
-static void launch_scan_words(const int32_t* geom, long long K, int64_t* offsets, cudaStream_t st) {
-  if (K <= 0) {
+// offsets[0..K] of the packed layout: an exclusive scan of the words of every mask's cropped bit plane (words(i)),
+// offsets[K] = the total.  One launch up to 1 024 masks, three beyond (device_exclusive_scan, no scratch).
+template <class Words>
+static void scan_words(Words words, long long K, int64_t* offsets, cudaStream_t st) {
+  if (K <= 0)
     cudaMemsetAsync(offsets, 0, sizeof(int64_t), st);
-    return;
-  }
-  const unsigned nb = (unsigned)((K + kScanChunk - 1) / kScanChunk);
-  scan_words_local_kernel<<<nb, kScanChunk, 0, st>>>(geom, K, offsets);
-  if (nb > 1) {
-    scan_words_bases_kernel<<<1, kScanChunk, 0, st>>>(K, offsets);
-    scan_words_add_kernel<<<nb - 1, kScanChunk, 0, st>>>(K, offsets);
-  }
+  else
+    device_exclusive_scan<int64_t, 1>(words, K, offsets, offsets + K, st);
 }
+
+struct GeomWords {
+  const int32_t* geom4;
+  __device__ int64_t operator()(long long i) const {
+    return (int64_t)((__ldg(geom4 + 4 * i + 2) + 31) >> 5) * __ldg(geom4 + 4 * i + 3);
+  }
+};
 
 __global__ void paste_geometry_kernel(const float4* __restrict__ boxes, const int32_t* __restrict__ channel, int K,
                                       float scale, int H, int W, int32_t* __restrict__ geom4) {
@@ -339,31 +273,29 @@ __global__ void pm_geometry_kernel(const float4* __restrict__ boxes, const int32
   reinterpret_cast<int4*>(geom4)[i] = out;
 }
 
-// pm_geometry_kernel + scan_words_local_kernel in one launch (the step is a chain of small dependent kernels)
-__global__ void __launch_bounds__(kScanChunk) pm_geometry_scan_kernel(
-    const float4* __restrict__ boxes, const int32_t* __restrict__ counts, long long K, int max_det, int mh, int mw,
-    int ih, int iw, int upsample, float rx, float ry, const uint8_t* __restrict__ row_state,
-    const int64_t* __restrict__ tile_offsets, int32_t* __restrict__ geom4, int64_t* __restrict__ offsets) {
-  __shared__ long long warp_sum[32];
-  const long long i = (long long)blockIdx.x * kScanChunk + threadIdx.x;
-  long long v = 0;
-  if (i < K) {
+// words(i) of hdy_process_mask_geometry: the window of slot i, stored to geom4 on the way, so that the geometry and the
+// first pass of the scan are one launch (the step is a chain of small dependent kernels)
+struct PmWindowWords {
+  const float4* boxes;
+  const int32_t* counts;
+  int max_det, mh, mw, ih, iw, upsample;
+  float rx, ry;
+  const uint8_t* row_state;
+  const int64_t* tile_offsets;
+  int32_t* geom4;
+  __device__ int64_t operator()(long long i) const {
     const int tile = (int)(i / max_det), d = (int)(i - (long long)tile * max_det);
     int4 out = make_int4(0, 0, 0, 0);
     // row_state: the slot is row tile_offsets[tile] + d of the slide; only rows the slide-level merge KEPT get a mask
-    if (d < counts[tile] && (!row_state || row_state[tile_offsets[tile] + d] == HDY_STATE_KEPT)) {
-      const PMGeom g = pm_geometry(boxes[i], mh, mw, ih, iw, upsample, rx, ry);
+    if (d < __ldg(counts + tile) &&
+        (!row_state || __ldg(row_state + __ldg(tile_offsets + tile) + d) == HDY_STATE_KEPT)) {
+      const PMGeom g = pm_geometry(__ldg(boxes + i), mh, mw, ih, iw, upsample, rx, ry);
       out = make_int4(g.x0, g.y0, g.w, g.h);
     }
     reinterpret_cast<int4*>(geom4)[i] = out;
-    v = (long long)((out.z + 31) >> 5) * out.w;
+    return (int64_t)((out.z + 31) >> 5) * out.w;
   }
-  const long long incl = block_incl_scan_ll(v, warp_sum);
-  if (i < K && threadIdx.x != 0) offsets[i] = incl - v;
-  const long long last = min((long long)(blockIdx.x + 1) * kScanChunk, K) - 1;
-  if (i == last) offsets[last + 1] = incl;
-  if (i == 0) offsets[0] = 0;
-}
+};
 
 // Slide form of the packed layout: the batch's word offsets move behind the words of the earlier batches (device
 // cursor, ping-pong so that one launch both reads and advances it) and every live slot's window / offset is copied to
@@ -526,7 +458,7 @@ int hdy_paste_geometry(const float* boxes, const int32_t* channel, int K, int M,
     paste_geometry_kernel<<<(unsigned)((K + 127) / 128), 128, 0, st>>>(reinterpret_cast<const float4*>(boxes), channel,
                                                                        K, scale, H, W, geom);
   }
-  launch_scan_words(geom, K, offsets, st);
+  scan_words(GeomWords{geom}, K, offsets, st);
   return check_launch("hdy_paste_geometry");
 }
 
@@ -598,21 +530,13 @@ int hdy_process_mask_geometry(const float* boxes, const int32_t* counts, int bs,
   HDY_REQUIRE(!row_state || tile_offsets, "process_mask_geometry: row_state needs tile_offsets");
   cudaStream_t st = (cudaStream_t)stream;
   const long long K = (long long)bs * max_det;
-  if (K > 0) {
+  if (K > 0)
     HDY_REQUIRE(boxes && counts && geom && ((uintptr_t)boxes & 15) == 0 && ((uintptr_t)geom & 15) == 0,
                 "process_mask_geometry: NULL or misaligned pointer");
-    const float rx = (float)((double)mw / (double)iw), ry = (float)((double)mh / (double)ih);
-    const unsigned nb = (unsigned)((K + kScanChunk - 1) / kScanChunk);
-    pm_geometry_scan_kernel<<<nb, kScanChunk, 0, st>>>(reinterpret_cast<const float4*>(boxes), counts, K, max_det, mh,
-                                                       mw, ih, iw, upsample, rx, ry, row_state, tile_offsets, geom,
-                                                       offsets);
-    if (nb > 1) {
-      scan_words_bases_kernel<<<1, kScanChunk, 0, st>>>(K, offsets);
-      scan_words_add_kernel<<<nb - 1, kScanChunk, 0, st>>>(K, offsets);
-    }
-  } else {
-    launch_scan_words(geom, K, offsets, st);
-  }
+  const float rx = (float)((double)mw / (double)iw), ry = (float)((double)mh / (double)ih);
+  scan_words(PmWindowWords{reinterpret_cast<const float4*>(boxes), counts, max_det, mh, mw, ih, iw, upsample, rx, ry,
+                           row_state, tile_offsets, geom},
+             K, offsets, st);
   return check_launch("hdy_process_mask_geometry");
 }
 

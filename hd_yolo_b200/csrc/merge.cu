@@ -22,8 +22,10 @@
 // that cannot intersect, so it never changes a verdict.
 //
 // Also here: an LSD radix sort (8-bit digits, warp-private stable ranking) used to return survivors in the
-// reference's score-descending order, and the small device-wide exclusive scan both need.
+// reference's score-descending order.  The cell-count and histogram scans and the survivor and seam selections are
+// scan_common.cuh's.
 #include "hdy_common.cuh"
+#include "scan_common.cuh"
 
 namespace hdy {
 
@@ -45,128 +47,21 @@ struct MergeStats {
 };
 
 // ------------------------------------------------------------------------------------------------
-// device-wide exclusive scan of int32 (in place), 3 phases, 4096 items per block
-// ------------------------------------------------------------------------------------------------
-constexpr int kScanThreads = 1024;
-constexpr int kScanItems = 4;
-constexpr int kScanTile = kScanThreads * kScanItems;
-
-__device__ __forceinline__ int block_scan_1024(int v, int* warp_tmp, int& total) {
-  // inclusive scan over the block's `v`; returns this thread's exclusive prefix, total = block sum
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  int incl = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    int u = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += u;
-  }
-  if (lane == 31) warp_tmp[warp] = incl;
-  __syncthreads();
-  if (warp == 0) {
-    int s = warp_tmp[lane], t = s;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      int u = __shfl_up_sync(0xffffffffu, t, o);
-      if (lane >= o) t += u;
-    }
-    warp_tmp[lane] = t - s;
-    if (lane == 31) warp_tmp[32] = t;
-  }
-  __syncthreads();
-  const int excl = warp_tmp[warp] + incl - v;
-  total = warp_tmp[32];
-  __syncthreads();
-  return excl;
-}
-
-__global__ void __launch_bounds__(kScanThreads) scan_reduce_kernel(const int* __restrict__ a, long long n,
-                                                                    int* __restrict__ block_sums) {
-  __shared__ int warp_tmp[33];
-  const long long base = (long long)blockIdx.x * kScanTile + (long long)threadIdx.x * kScanItems;
-  int s = 0;
-#pragma unroll
-  for (int k = 0; k < kScanItems; ++k)
-    if (base + k < n) s += a[base + k];
-  int total;
-  block_scan_1024(s, warp_tmp, total);
-  if (threadIdx.x == 0) block_sums[blockIdx.x] = total;
-}
-
-__global__ void __launch_bounds__(kScanThreads) scan_sums_kernel(int* __restrict__ block_sums, int nblocks,
-                                                                  int* __restrict__ total_out) {
-  __shared__ int warp_tmp[33];
-  __shared__ int carry;
-  if (threadIdx.x == 0) carry = 0;
-  __syncthreads();
-  for (int b0 = 0; b0 < nblocks; b0 += kScanThreads) {
-    const int i = b0 + threadIdx.x;
-    const int v = i < nblocks ? block_sums[i] : 0;
-    int total;
-    const int excl = block_scan_1024(v, warp_tmp, total);
-    if (i < nblocks) block_sums[i] = carry + excl;
-    __syncthreads();
-    if (threadIdx.x == 0) carry += total;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0 && total_out) *total_out = carry;
-}
-
-__global__ void __launch_bounds__(kScanThreads) scan_apply_kernel(int* __restrict__ a, long long n,
-                                                                   const int* __restrict__ block_sums) {
-  __shared__ int warp_tmp[33];
-  const long long base = (long long)blockIdx.x * kScanTile + (long long)threadIdx.x * kScanItems;
-  int v[kScanItems], s = 0;
-#pragma unroll
-  for (int k = 0; k < kScanItems; ++k) {
-    v[k] = (base + k < n) ? a[base + k] : 0;
-    s += v[k];
-  }
-  int total;
-  int run = block_sums[blockIdx.x] + block_scan_1024(s, warp_tmp, total);
-#pragma unroll
-  for (int k = 0; k < kScanItems; ++k) {
-    if (base + k < n) a[base + k] = run;
-    run += v[k];
-  }
-}
-
-static inline size_t scan_scratch_ints(long long n) { return (size_t)((n + kScanTile - 1) / kScanTile) + 1; }
-
-// exclusive scan of a[0..n) in place; *total_out (device, may be NULL) receives the sum
-static int device_exclusive_scan(int* a, long long n, int* scratch, int* total_out, cudaStream_t st) {
-  if (n <= 0) return HDY_OK;
-  const int nblocks = (int)((n + kScanTile - 1) / kScanTile);
-  scan_reduce_kernel<<<nblocks, kScanThreads, 0, st>>>(a, n, scratch);
-  scan_sums_kernel<<<1, kScanThreads, 0, st>>>(scratch, nblocks, total_out);
-  scan_apply_kernel<<<nblocks, kScanThreads, 0, st>>>(a, n, scratch);
-  return check_launch("device_exclusive_scan");
-}
-
-// ------------------------------------------------------------------------------------------------
 // T2: tile-local detections -> slide coordinates, appended to flat arrays
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(1024) append_offsets_kernel(const int32_t* __restrict__ counts, int bs,
-                                                               long long* __restrict__ cursor,
-                                                               long long* __restrict__ tile_offsets) {
-  __shared__ int warp_tmp[33];
-  __shared__ long long carry;
-  if (threadIdx.x == 0) carry = *cursor;
-  __syncthreads();
-  for (int b0 = 0; b0 < bs; b0 += 1024) {
-    const int i = b0 + threadIdx.x;
-    const int v = i < bs ? max(counts[i], 0) : 0;
-    int total;
-    const int excl = block_scan_1024(v, warp_tmp, total);
-    if (i < bs) tile_offsets[i] = carry + excl;
-    __syncthreads();
-    if (threadIdx.x == 0) carry += total;
-    __syncthreads();
+// scan_carry_kernel's view of hdy_merge_append: tile counts (clamped at 0) -> tile_offsets[0..bs], carried on from
+// *cursor, which receives the new end
+struct AppendOffsets {
+  const int32_t* counts;
+  long long* tile_offsets;
+  long long* cursor;
+  int bs;
+  __device__ long long load(long long i) const { return max(__ldg(counts + i), 0); }
+  __device__ void store(long long i, long long x) const {
+    tile_offsets[i] = x;
+    if (i == bs) *cursor = x;
   }
-  if (threadIdx.x == 0) {
-    tile_offsets[bs] = carry;
-    *cursor = carry;
-  }
-}
+};
 
 __global__ void append_tiles_kernel(const float4* __restrict__ boxes, const float* __restrict__ scores,
                                     const int64_t* __restrict__ labels, const uint8_t* __restrict__ fragile,
@@ -308,7 +203,6 @@ __global__ void dirty_tiles_kernel(const float4* __restrict__ far_boxes, const i
 struct MergeWs {
   MergeStats* stats;
   int* cell;       // [G*G + 2] counts -> begin offsets -> end offsets
-  int* scan_tmp;   // scan scratch
   float4* cbox;    // [n_max] boxes in cell order
   uint64_t* ckey;  // [n_max] order keys in cell order
   uint8_t* cstate; // [n_max]
@@ -341,8 +235,6 @@ static MergeWs merge_layout(void* base, long long n_max) {
   o += align256(sizeof(MergeStats));
   w.cell = reinterpret_cast<int*>(p + o);
   o += align256(nb * 4);
-  w.scan_tmp = reinterpret_cast<int*>(p + o);
-  o += align256(scan_scratch_ints((long long)nb) * 4);
   w.cbox = reinterpret_cast<float4*>(p + o);
   o += align256((size_t)n_max * 16);
   w.ckey = reinterpret_cast<uint64_t*>(p + o);
@@ -732,81 +624,21 @@ __global__ void merge_finish_kernel(const uint32_t* __restrict__ pos, const uint
 // survivors -> keys in row order, LSD radix sort, gather
 // ------------------------------------------------------------------------------------------------
 // Keys leave in ROW order, so that a stable sort on the score half alone (4 radix passes instead of 8) already breaks
-// ties by the lower row.  Blocks own contiguous row ranges: count -> scan of the block counts -> write.
-constexpr int kSelThreads = 256;
-constexpr int kSelMaxBlocks = 4096;
-
-__global__ void __launch_bounds__(kSelThreads) select_count_kernel(const uint8_t* __restrict__ state,
-                                                                   const long long* __restrict__ n_dev,
-                                                                   long long n_max, long long chunk,
-                                                                   int* __restrict__ block_counts) {
-  const long long n = n_dev ? min(*n_dev, n_max) : n_max;
-  const long long lo = (long long)blockIdx.x * chunk, hi = min(lo + chunk, n);
-  int c = 0;
-  for (long long i = lo + threadIdx.x; i < hi; i += kSelThreads) c += state[i] == MS_KEPT;
-  __shared__ int part[kSelThreads / 32];
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = c;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    int t = 0;
-    for (int w = 0; w < kSelThreads / 32; ++w) t += part[w];
-    block_counts[blockIdx.x] = t;
+// ties by the lower row.
+struct KeptKeys {
+  struct Shared {};
+  const uint8_t* state;
+  const float* scores;
+  const long long* n_dev;
+  long long n_max;
+  uint64_t* keys;
+  __device__ void init(Shared&) const {}
+  __device__ long long rows() const { return n_dev ? min(*n_dev, n_max) : n_max; }
+  __device__ bool keep(const Shared&, long long i) const { return state[i] == MS_KEPT; }
+  __device__ void emit(const Shared&, long long i, long long slot) const {
+    keys[slot] = make_key(__ldg(scores + i), (uint32_t)i);
   }
-}
-
-__global__ void __launch_bounds__(1024) select_scan_kernel(int* __restrict__ block_counts, int nblocks,
-                                                           int* __restrict__ count_out) {
-  __shared__ int warp_tmp[33];
-  // nblocks <= kSelMaxBlocks = 4 x 1024: four consecutive entries per thread
-  int v[4], s = 0;
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    const int i = threadIdx.x * 4 + j;
-    v[j] = i < nblocks ? block_counts[i] : 0;
-    s += v[j];
-  }
-  int total;
-  int excl = block_scan_1024(s, warp_tmp, total);
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    const int i = threadIdx.x * 4 + j;
-    if (i < nblocks) block_counts[i] = excl;
-    excl += v[j];
-  }
-  if (threadIdx.x == 0) *count_out = total;
-}
-
-__global__ void __launch_bounds__(kSelThreads) select_write_kernel(const uint8_t* __restrict__ state,
-                                                                   const float* __restrict__ scores,
-                                                                   const long long* __restrict__ n_dev,
-                                                                   long long n_max, long long chunk,
-                                                                   const int* __restrict__ block_offsets,
-                                                                   uint64_t* __restrict__ keys) {
-  __shared__ int wcount[kSelThreads / 32];
-  const long long n = n_dev ? min(*n_dev, n_max) : n_max;
-  const long long lo = (long long)blockIdx.x * chunk, hi = min(lo + chunk, n);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  long long running = block_offsets[blockIdx.x];
-  for (long long i0 = lo; i0 < hi; i0 += kSelThreads) {
-    const long long i = i0 + threadIdx.x;
-    const bool k = i < hi && state[i] == MS_KEPT;
-    const unsigned m = __ballot_sync(0xffffffffu, k);
-    if (lane == 0) wcount[warp] = __popc(m);
-    __syncthreads();
-    int before = 0, total = 0;
-#pragma unroll
-    for (int w = 0; w < kSelThreads / 32; ++w) {
-      const int c = wcount[w];
-      if (w < warp) before += c;
-      total += c;
-    }
-    if (k) keys[running + before + __popc(m & ((1u << lane) - 1u))] = make_key(scores[i], (uint32_t)i);
-    running += total;
-    __syncthreads();
-  }
-}
+};
 
 constexpr int kSortThreads = 256;                         // 8 warps
 constexpr int kSortPerWarp = 1024;                        // keys per warp sub-tile
@@ -952,93 +784,53 @@ __global__ void seam_rect_kernel(const float4* __restrict__ boxes, long long n, 
   }
 }
 
-struct SeamRects {
-  float4 r[kSeamMaxWorld];
-  int live[kSeamMaxWorld];
+// Own rows whose box touches (closed intervals) the rectangle of another rank that has rows: a superset of "the boxes
+// intersect", which is all exactness needs (hd_yolo_b200/dist.py).  Payload row k = (box bits, score bits, global
+// index) of own row sel[k]; rows leave in ascending row order.
+struct SeamRows {
+  struct Shared {
+    float4 r[kSeamMaxWorld];
+    int live[kSeamMaxWorld];
+    long long gbase;  // rows owned by lower ranks
+  };
+  const float4* boxes;
+  const float* scores;
+  long long n;
+  const int32_t* summaries;
+  int world, rank, hb, seam_cap;
+  int32_t* sel;
+  int32_t* block;
+  __device__ void init(Shared& S) const {
+    for (int q = threadIdx.x; q < world; q += blockDim.x) {
+      const int32_t* h = summaries + (size_t)q * hb;
+      S.r[q] = make_float4(__int_as_float(h[0]), __int_as_float(h[1]), __int_as_float(h[2]), __int_as_float(h[3]));
+      S.live[q] = (q != rank) && (*reinterpret_cast<const long long*>(h + 6) > 0);
+    }
+    if (threadIdx.x == 0) {
+      long long g = 0;
+      for (int q = 0; q < rank; ++q) g += *reinterpret_cast<const long long*>(summaries + (size_t)q * hb + 6);
+      S.gbase = g;
+    }
+    __syncthreads();
+  }
+  __device__ long long rows() const { return n; }
+  __device__ bool keep(const Shared& S, long long i) const {
+    const float4 b = __ldg(boxes + i);
+    bool s = false;
+    for (int q = 0; q < world; ++q)
+      s |= S.live[q] && (b.z >= S.r[q].x) && (b.x <= S.r[q].z) && (b.w >= S.r[q].y) && (b.y <= S.r[q].w);
+    return s;
+  }
+  __device__ void emit(const Shared& S, long long i, long long slot) const {
+    if (slot >= seam_cap) return;
+    const float4 b = __ldg(boxes + i);
+    sel[slot] = (int32_t)i;
+    int32_t* e = block + kSeamHdr + slot * kSeamRow;
+    e[0] = __float_as_int(b.x), e[1] = __float_as_int(b.y), e[2] = __float_as_int(b.z), e[3] = __float_as_int(b.w);
+    e[4] = __float_as_int(__ldg(scores + i));
+    e[5] = (int32_t)(uint32_t)(S.gbase + i);
+  }
 };
-__device__ __forceinline__ void seam_load_rects(SeamRects& S, const int32_t* summaries, int world, int rank, int hb) {
-  for (int q = threadIdx.x; q < world; q += blockDim.x) {
-    const int32_t* h = summaries + (size_t)q * hb;
-    S.r[q] = make_float4(__int_as_float(h[0]), __int_as_float(h[1]), __int_as_float(h[2]), __int_as_float(h[3]));
-    S.live[q] = (q != rank) && (*reinterpret_cast<const long long*>(h + 6) > 0);
-  }
-  __syncthreads();
-}
-// closed-interval test against every other rank's rectangle: a superset of "the boxes intersect", which is all
-// exactness needs (hd_yolo_b200/dist.py)
-__device__ __forceinline__ bool seam_row(const float4& b, const SeamRects& S, int world) {
-  bool s = false;
-  for (int q = 0; q < world; ++q)
-    s |= S.live[q] && (b.z >= S.r[q].x) && (b.x <= S.r[q].z) && (b.w >= S.r[q].y) && (b.y <= S.r[q].w);
-  return s;
-}
-
-__global__ void __launch_bounds__(kSelThreads) seam_count_kernel(const float4* __restrict__ boxes, long long n,
-                                                                 long long chunk, const int32_t* __restrict__ summaries,
-                                                                 int world, int rank, int hb,
-                                                                 int* __restrict__ block_counts) {
-  __shared__ SeamRects S;
-  __shared__ int part[kSelThreads / 32];
-  seam_load_rects(S, summaries, world, rank, hb);
-  const long long lo = (long long)blockIdx.x * chunk, hi = min(lo + chunk, n);
-  int c = 0;
-  for (long long i = lo + threadIdx.x; i < hi; i += kSelThreads) c += seam_row(boxes[i], S, world);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = c;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    int t = 0;
-    for (int w = 0; w < kSelThreads / 32; ++w) t += part[w];
-    block_counts[blockIdx.x] = t;
-  }
-}
-
-// rows leave in ascending row order: payload row k = (box bits, score bits, global index) of own row sel[k]
-__global__ void __launch_bounds__(kSelThreads) seam_write_kernel(const float4* __restrict__ boxes,
-                                                                 const float* __restrict__ scores, long long n,
-                                                                 long long chunk, const int32_t* __restrict__ summaries,
-                                                                 int world, int rank, int hb,
-                                                                 const int* __restrict__ block_offsets, int seam_cap,
-                                                                 int32_t* __restrict__ sel, int32_t* __restrict__ block) {
-  __shared__ SeamRects S;
-  __shared__ int wcount[kSelThreads / 32];
-  seam_load_rects(S, summaries, world, rank, hb);
-  long long gbase = 0;  // rows owned by lower ranks
-  for (int q = 0; q < rank; ++q) gbase += *reinterpret_cast<const long long*>(summaries + (size_t)q * hb + 6);
-  const long long lo = (long long)blockIdx.x * chunk, hi = min(lo + chunk, n);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  long long running = block_offsets[blockIdx.x];
-  for (long long i0 = lo; i0 < hi; i0 += kSelThreads) {
-    const long long i = i0 + threadIdx.x;
-    float4 b = make_float4(0.f, 0.f, 0.f, 0.f);
-    bool k = false;
-    if (i < hi) {
-      b = boxes[i];
-      k = seam_row(b, S, world);
-    }
-    const unsigned m = __ballot_sync(0xffffffffu, k);
-    if (lane == 0) wcount[warp] = __popc(m);
-    __syncthreads();
-    int before = 0, total = 0;
-#pragma unroll
-    for (int w = 0; w < kSelThreads / 32; ++w) {
-      const int c = wcount[w];
-      if (w < warp) before += c;
-      total += c;
-    }
-    const long long slot = running + before + __popc(m & ((1u << lane) - 1u));
-    if (k && slot < seam_cap) {
-      sel[slot] = (int32_t)i;
-      int32_t* e = block + kSeamHdr + slot * kSeamRow;
-      e[0] = __float_as_int(b.x), e[1] = __float_as_int(b.y), e[2] = __float_as_int(b.z), e[3] = __float_as_int(b.w);
-      e[4] = __float_as_int(scores[i]);
-      e[5] = (int32_t)(uint32_t)(gbase + i);
-    }
-    running += total;
-    __syncthreads();
-  }
-}
 
 __global__ void seam_block_header_kernel(const int* __restrict__ count, int32_t* __restrict__ block) {
   if (threadIdx.x == 0 && blockIdx.x == 0) {
@@ -1176,8 +968,9 @@ int hdy_merge_append(const float* boxes, const float* scores, const int64_t* lab
   HDY_REQUIRE(!out_scores || scores, "hdy_merge_append: out_scores without scores");
   HDY_REQUIRE(!out_labels || labels, "hdy_merge_append: out_labels without labels");
   cudaStream_t st = (cudaStream_t)stream;
-  append_offsets_kernel<<<1, 1024, 0, st>>>(counts, bs, reinterpret_cast<long long*>(cursor),
-                                            reinterpret_cast<long long*>(tile_offsets));
+  long long* cur = reinterpret_cast<long long*>(cursor);
+  scan_carry_kernel<long long><<<1, kScanThreads, 0, st>>>(
+      AppendOffsets{counts, reinterpret_cast<long long*>(tile_offsets), cur, bs}, (long long)bs, cur);
   dim3 grid((unsigned)((max_det + 127) / 128), (unsigned)bs);
   append_tiles_kernel<<<grid, 128, 0, st>>>(reinterpret_cast<const float4*>(boxes), scores, labels, fragile, counts,
                                             reinterpret_cast<const float4*>(rois), max_det, tile_base, scale,
@@ -1268,8 +1061,7 @@ static int merge_build_common(const char* what, MergeIn in, const float* tile_co
   merge_stats_kernel<<<blocks, kMergeThreads, 0, st>>>(in.boxes, in.scores, in.n_dev, n_max, in.conf, w.stats);
   merge_pick_cell_kernel<<<1, 32, 0, st>>>(w.stats);
   merge_classify_kernel<<<blocks, kMergeThreads, 0, st>>>(in, w.stats, w.G, w.cell, state);
-  int rc = device_exclusive_scan(w.cell, (long long)nb - 1, w.scan_tmp, nullptr, st);
-  if (rc) return rc;
+  device_exclusive_scan<int, 4>(ArrayValues<int>{w.cell}, (long long)nb - 1, w.cell, (int*)nullptr, st);
   merge_fill_kernel<<<blocks, kMergeThreads, 0, st>>>(in, w.stats, w.G, w.cell, state, w.cbox, w.ckey, w.cstate,
                                                       w.pos, w.blocked, w.ctile);
   return check_launch(what);
@@ -1313,18 +1105,11 @@ int hdy_seam_select(const float* boxes, const float* scores, int64_t n_local, co
     return HDY_OK;
   }
   HDY_REQUIRE(boxes && scores && ((uintptr_t)boxes & 15) == 0, "hdy_seam_select: NULL or misaligned pointer");
-  long long chunk = (n_local + kSelMaxBlocks - 1) / kSelMaxBlocks;
-  chunk = ((chunk + kSelThreads - 1) / kSelThreads) * kSelThreads;
-  if (chunk < 4 * kSelThreads) chunk = 4 * kSelThreads;
-  const int nblocks = (int)((n_local + chunk - 1) / chunk);
-  const float4* b4 = reinterpret_cast<const float4*>(boxes);
-  const int hb = seam_hb(far_cap);
   // block_scratch: [kSelMaxBlocks] block counts -> offsets, then the total
-  seam_count_kernel<<<nblocks, kSelThreads, 0, st>>>(b4, n_local, chunk, summaries, world, rank, hb, block_scratch);
-  select_scan_kernel<<<1, 1024, 0, st>>>(block_scratch, nblocks, block_scratch + kSelMaxBlocks);
+  const SeamRows f{reinterpret_cast<const float4*>(boxes), scores, n_local, summaries, world, rank, seam_hb(far_cap),
+                   seam_cap, sel, block};
+  launch_compaction(f, n_local, block_scratch, block_scratch + kSelMaxBlocks, st);
   seam_block_header_kernel<<<1, 32, 0, st>>>(block_scratch + kSelMaxBlocks, block);
-  seam_write_kernel<<<nblocks, kSelThreads, 0, st>>>(b4, scores, n_local, chunk, summaries, world, rank, hb,
-                                                     block_scratch, seam_cap, sel, block);
   return check_launch("hdy_seam_select");
 }
 
@@ -1465,7 +1250,7 @@ size_t hdy_sort_workspace_bytes(int64_t n_max) {
   if (n_max <= 0) return 256;
   const long long n_sub = (n_max + kSortPerWarp - 1) / kSortPerWarp;
   const long long hist = 256 * n_sub;
-  return align256((size_t)hist * 4) + align256(scan_scratch_ints(hist) * 4);
+  return align256((size_t)hist * 4);
 }
 
 int hdy_sort_keys_bytes(uint64_t* keys, uint64_t* tmp, const int32_t* n_dev, int64_t n_max, int first_byte,
@@ -1481,14 +1266,12 @@ int hdy_sort_keys_bytes(uint64_t* keys, uint64_t* tmp, const int32_t* n_dev, int
   const int n_sub = (int)((n_max + kSortPerWarp - 1) / kSortPerWarp);
   const long long hist_n = 256ll * n_sub;
   int* hist = static_cast<int*>(workspace);
-  int* scratch = reinterpret_cast<int*>(static_cast<unsigned char*>(workspace) + align256((size_t)hist_n * 4));
   const unsigned blocks = (unsigned)((n_sub + kSortWarps - 1) / kSortWarps);
   uint64_t* src = keys;
   uint64_t* dst = tmp;
   for (int pass = first_byte; pass < first_byte + n_bytes; ++pass) {
     sort_hist_kernel<<<blocks, kSortThreads, 0, st>>>(src, n_dev, (int)n_max, pass * 8, n_sub, hist);
-    int rc = device_exclusive_scan(hist, hist_n, scratch, nullptr, st);
-    if (rc) return rc;
+    device_exclusive_scan<int, 4>(ArrayValues<int>{hist}, hist_n, hist, (int*)nullptr, st);
     sort_scatter_kernel<<<blocks, kSortThreads, 0, st>>>(src, n_dev, (int)n_max, pass * 8, n_sub, hist, dst);
     uint64_t* t = src;
     src = dst;
@@ -1510,15 +1293,8 @@ int hdy_merge_select_ordered(const uint8_t* state, const float* scores, const in
     return HDY_OK;
   }
   HDY_REQUIRE(state && scores && keys, "hdy_merge_select_ordered: NULL pointer");
-  // contiguous row ranges, a multiple of the block size, at most kSelMaxBlocks of them
-  long long chunk = (n_max + kSelMaxBlocks - 1) / kSelMaxBlocks;
-  chunk = ((chunk + kSelThreads - 1) / kSelThreads) * kSelThreads;
-  if (chunk < 4 * kSelThreads) chunk = 4 * kSelThreads;
-  const int nblocks = (int)((n_max + chunk - 1) / chunk);
-  const long long* nd = reinterpret_cast<const long long*>(n_dev);
-  select_count_kernel<<<nblocks, kSelThreads, 0, st>>>(state, nd, n_max, chunk, block_scratch);
-  select_scan_kernel<<<1, 1024, 0, st>>>(block_scratch, nblocks, count);
-  select_write_kernel<<<nblocks, kSelThreads, 0, st>>>(state, scores, nd, n_max, chunk, block_scratch, keys);
+  launch_compaction(KeptKeys{state, scores, reinterpret_cast<const long long*>(n_dev), n_max, keys}, n_max,
+                    block_scratch, count, st);
   return check_launch("hdy_merge_select_ordered");
 }
 

@@ -18,6 +18,7 @@
 // The grid/cell choice only affects speed, never the result: the IoU test itself is exact
 // (hdy_common.cuh: iou_gt) and is evaluated for every pair that can possibly intersect.
 #include "hdy_common.cuh"
+#include "scan_common.cuh"
 
 namespace hdy {
 
@@ -34,45 +35,6 @@ static unsigned long long* g_phase_host = nullptr;
 __device__ __forceinline__ uint32_t next_pow2(uint32_t v) {
   if (v <= 1) return 1;
   return 1u << (32 - __clz(v - 1));
-}
-
-// exclusive scan of a[0..len) in place (ints); returns total.  All threads must call.
-__device__ int block_excl_scan(int* a, int len, int* warp_tmp) {
-  const int t = threadIdx.x, T = kNmsThreads;
-  const int items = (len + T - 1) / T;
-  const int b = min(t * items, len), e = min(b + items, len);
-  int sum = 0;
-  for (int i = b; i < e; ++i) sum += a[i];
-  const int lane = t & 31, warp = t >> 5;
-  int incl = sum;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    int v = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += v;
-  }
-  if (lane == 31) warp_tmp[warp] = incl;
-  __syncthreads();
-  if (warp == 0) {
-    int v = (lane < T / 32) ? warp_tmp[lane] : 0;
-    int s = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      int u = __shfl_up_sync(0xffffffffu, s, o);
-      if (lane >= o) s += u;
-    }
-    if (lane < T / 32) warp_tmp[lane] = s - v;  // exclusive warp offsets
-    if (lane == T / 32 - 1) warp_tmp[T / 32] = s;  // total
-  }
-  __syncthreads();
-  int run = warp_tmp[warp] + incl - sum;
-  for (int i = b; i < e; ++i) {
-    int v = a[i];
-    a[i] = run;
-    run += v;
-  }
-  const int total = warp_tmp[T / 32];
-  __syncthreads();
-  return total;
 }
 
 struct TileOut {
@@ -192,7 +154,7 @@ __device__ void nms_tile_body(const int n_in, const int max_nms, uint64_t* keys,
     if (cls) atomicAdd(&cell[bucket], 1);
   }
   __syncthreads();
-  block_excl_scan(cell, NB, warp_tmp);
+  block_exclusive_scan_inplace<kNmsThreads>(cell, NB, warp_tmp);
   for (int r = t; r < n; r += T) {
     int bucket = 0;
     if (classify(boxes[r], bucket)) items[atomicAdd(&cell[bucket], 1)] = (uint32_t)r;
@@ -325,7 +287,7 @@ __global__ void __launch_bounds__(kNmsThreads, 2) nms_tiles_kernel(
     int32_t* __restrict__ keep_slot, float4* __restrict__ keep_box, float* __restrict__ keep_score,
     float* __restrict__ keep_cls, int32_t* __restrict__ keep_counts, unsigned char* __restrict__ workspace,
     uint8_t* __restrict__ keep_fragile) {
-  __shared__ int warp_tmp[kNmsThreads / 32 + 1];
+  __shared__ int warp_tmp[33];
   __shared__ float red_tmp[kNmsThreads / 32];
   const int tile = blockIdx.x;
   const int n = min(counts[tile], cap);

@@ -22,6 +22,7 @@
 // (fp32, torchvision's operation order), so cell size and bucket choice never change a verdict.
 #include <stddef.h>
 #include "hdy_common.cuh"
+#include "scan_common.cuh"
 
 namespace hdy {
 
@@ -62,46 +63,6 @@ static_assert(sizeof(FastSmemT<kFastCapSmall>::dom) + 3 * kFastCapSmall >= 2 * 3
                       offsetof(FastSmemT<kFastCapSmall>, dom) + sizeof(FastSmemT<kFastCapSmall>::dom) &&
                   offsetof(FastSmemT<kFastCapSmall>, cell) >= offsetof(FastSmemT<kFastCapSmall>, dom) + 2 * 32 * 256 * 2,
               "radix count buffers must fit behind dom");
-
-template <int THREADS>
-__device__ __forceinline__ int block_excl_scan_cells(int* a, int len, int* warp_tmp) {
-  // exclusive scan of a[0..len) in place; returns the total.  All threads call.
-  const int t = threadIdx.x;
-  const int items = (len + THREADS - 1) / THREADS;
-  const int b = min(t * items, len), e = min(b + items, len);
-  int sum = 0;
-  for (int i = b; i < e; ++i) sum += a[i];
-  const int lane = t & 31, warp = t >> 5;
-  int incl = sum;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    int v = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += v;
-  }
-  if (lane == 31) warp_tmp[warp] = incl;
-  __syncthreads();
-  if (warp == 0) {
-    int v = (lane < THREADS / 32) ? warp_tmp[lane] : 0;
-    int s = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      int u = __shfl_up_sync(0xffffffffu, s, o);
-      if (lane >= o) s += u;
-    }
-    warp_tmp[lane] = s - v;
-    if (lane == 31) warp_tmp[32] = s;
-  }
-  __syncthreads();
-  int run = warp_tmp[warp] + incl - sum;
-  for (int i = b; i < e; ++i) {
-    int v = a[i];
-    a[i] = run;
-    run += v;
-  }
-  const int total = warp_tmp[32];
-  __syncthreads();
-  return total;
-}
 
 // Bitonic sort of THREADS keys, one per thread (thread t owns element t).
 template <int THREADS>
@@ -478,7 +439,7 @@ __global__ void __maxnreg__(CAP <= 3072 ? 56 : 64) nms_tiles_smem_kernel(
   }
   __syncthreads();
   // cell[b] = first position of bucket b, cell[NB] = number of binned boxes
-  const int n_active = block_excl_scan_cells<THREADS>(S.cell, kFastNB + 1, S.warp_i);
+  const int n_active = block_exclusive_scan_inplace<THREADS>(S.cell, kFastNB + 1, S.warp_i);
   const int large_begin = S.cell[kFastNB - 1];
 #pragma unroll
   for (int e = 0; e < MAXR; ++e)

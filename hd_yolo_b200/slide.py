@@ -173,8 +173,9 @@ def sort_keys(keys: torch.Tensor, n_dev: Optional[torch.Tensor] = None, first_by
         wbytes = lib.hdy_sort_workspace_bytes(n)
         ws = _ws.get(keys.device, "sort", wbytes)
         tmp = _ws.get(keys.device, "sort_tmp", n * 8)
+        # per pass: histogram, its scan (one launch while the histogram fits one scan tile: n <= 16 384), scatter
         _call("hdy_sort_keys_bytes", ptr(keys), ptr(tmp), ptr(n_dev), n, int(first_byte), int(n_bytes), ptr(ws), wbytes,
-              _stream(), launches=int(n_bytes) * 5)
+              _stream(), launches=int(n_bytes) * (3 if n <= 16384 else 5))
     return keys
 
 
