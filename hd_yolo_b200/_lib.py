@@ -15,7 +15,7 @@ HDY_MAX_ANCHORS = 8
 HDY_MAX_SCORES = 96
 HDY_STATUS_OVERFLOW = 1
 HDY_STATUS_ROUNDS = 2
-HDY_F32, HDY_F16 = 0, 1
+HDY_F32, HDY_F16, HDY_U8 = 0, 1, 2
 HDY_SEAM_HDR_WORDS, HDY_SEAM_FAR_WORDS, HDY_SEAM_ROW_WORDS, HDY_SEAM_META_WORDS, HDY_SEAM_MAX_WORLD = 16, 8, 6, 96, 64
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -118,6 +118,11 @@ SIGNATURES = {
                                             _vp, _vp]),
     "hdy_match_pairs": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _i, _f, _i, _vp, _vp, _vp, _vp, _vp]),
     "hdy_box_iou": (_i, [_vp, _i64, _vp, _i64, _vp, _vp]),
+    "hdy_pack_masks_geometry": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp]),
+    "hdy_pack_masks": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, C.c_int64, _vp, _vp]),
+    "hdy_mask_areas": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
+    "hdy_match_mask_pairs": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _f, _i, _vp, _i, _vp, _vp, _vp,
+                                  _vp]),
 }
 
 _lock = threading.Lock()

@@ -63,6 +63,54 @@ class PackedMasks:
     def nbytes(self) -> int:
         return self.bits.numel() * 4 + self.geom.numel() * 4 + self.offsets.numel() * 8
 
+    @classmethod
+    def from_dense(cls, masks: torch.Tensor) -> "PackedMasks":
+        """The inverse of ``to_dense()``: [K, H, W] or [K, 1, H, W] CUDA masks -> PackedMasks with TIGHT windows (the
+        bounding rectangle of the set pixels; an empty mask gets w = h = 0).  fp32 / fp16 pixels are set iff > 0.5
+        (``paste_masks_in_image(...) > 0.5``), uint8 / bool pixels iff nonzero.  One 8-byte device->host read (the
+        total word count)."""
+        if not isinstance(masks, torch.Tensor) or not masks.is_cuda:
+            raise HdyError("masks must be a CUDA tensor: hd_yolo_b200 has no CPU fallback")
+        codes = {torch.float32: _lib.HDY_F32, torch.float16: _lib.HDY_F16, torch.uint8: _lib.HDY_U8,
+                 torch.bool: _lib.HDY_U8}
+        if masks.dtype not in codes:
+            raise HdyError(f"masks must be float32, float16, uint8 or bool (got {masks.dtype})")
+        if masks.dim() == 4 and masks.shape[1] == 1:
+            masks = masks[:, 0]
+        if masks.dim() != 3:
+            raise HdyError(f"masks must be [K, H, W] or [K, 1, H, W], got {tuple(masks.shape)}")
+        K, H, W = (int(s) for s in masks.shape)
+        if H < 1 or W < 1:
+            raise HdyError(f"empty canvas {H} x {W}")
+        dev = masks.device
+        src = masks.contiguous()
+        if src.dtype == torch.bool:
+            src = src.view(torch.uint8)
+        geom = torch.empty((K, 4), dtype=torch.int32, device=dev)
+        offsets = torch.empty((K + 1,), dtype=torch.int64, device=dev)
+        status = torch.zeros((1,), dtype=torch.int32, device=dev)
+        _call("hdy_pack_masks_geometry", ptr(src), codes[masks.dtype], K, H, W, ptr(geom), ptr(offsets), _stream(),
+              launches=3)
+        words = int(offsets[K].item())
+        bits = torch.empty((max(words, 1),), dtype=torch.int32, device=dev)
+        if K:
+            _call("hdy_pack_masks", ptr(src), codes[masks.dtype], K, H, W, ptr(geom), ptr(offsets), ptr(bits), words,
+                  ptr(status), _stream())
+        return cls(geom, offsets, bits[:words], H, W, status)
+
+    def areas(self) -> torch.Tensor:
+        """[K] int32: set pixels per mask (bits beyond a row's width are ignored, whatever they hold)."""
+        K = len(self)
+        out = torch.empty((K,), dtype=torch.int32, device=self.geom.device)
+        if K:
+            _call("hdy_mask_areas", ptr(_aligned16(self.geom.contiguous())), ptr(self.offsets),
+                  ptr(self._bits_nonempty()), K, ptr(out), _stream())
+        return out
+
+    def _bits_nonempty(self) -> torch.Tensor:
+        """`bits`, or one zero word when no mask has any (an empty tensor has no device address)."""
+        return self.bits if self.bits.numel() else torch.zeros((1,), dtype=torch.int32, device=self.bits.device)
+
 
 def _hw(shape) -> Tuple[int, int]:
     if isinstance(shape, int):

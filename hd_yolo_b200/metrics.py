@@ -1,6 +1,7 @@
 """Prediction <-> ground-truth matching on the device (SURVEY 8f rank 2): host mirror of ``box_iou``
 (metayolo/models/utils_general.py:247-265) and of the matching half of ``APMeter.add``
-(metayolo/models/metrics.py:270-303), over ``hdy_box_iou`` / ``hdy_match_pairs``.
+(metayolo/models/metrics.py:270-303), over ``hdy_box_iou`` / ``hdy_match_pairs``, and by mask IoU over
+``hdy_match_mask_pairs`` (bit-packed masks, ``PackedMasks``).
 
 The reference moves every image's detections to the host and builds a dense k x g IoU matrix there; here the
 matching pairs are produced on the device and only they (a few hundred rows per image) are copied back.
@@ -15,6 +16,7 @@ import numpy as np
 import torch
 
 from ._lib import HdyError, ptr
+from .masks import PackedMasks
 from .ops import _Cand, _aligned16, _call, _need_cuda, _run_nms, _stream
 
 __all__ = ["box_iou", "match_predictions", "APMeter"]
@@ -35,24 +37,34 @@ def box_iou(box1: torch.Tensor, box2: torch.Tensor) -> torch.Tensor:
 
 
 def match_predictions(output: Dict[str, torch.Tensor], target: Dict[str, torch.Tensor], iou_min: float = 0.5,
-                      cap: Optional[int] = None) -> Dict[str, torch.Tensor]:
-    """The device half of APMeter.add (metrics.py:271-284), box IoU only.
+                      cap: Optional[int] = None, iou_type: str = 'boxes') -> Dict[str, torch.Tensor]:
+    """The device half of APMeter.add (metrics.py:271-284), by box IoU or, with iou_type='masks', by mask IoU.
 
     Returns (all on the device): 'order' (rows of `output` by score, descending, ties by lower row), 'scores' /
     'labels' in that order, and the matching pairs 'pred_idx' (rank in `order`), 'true_idx', 'ious' sorted by IoU
-    descending (ties in row-major (pred, true) order).  One D2H read (the pair count)."""
+    descending (ties in row-major (pred, true) order).  One D2H read (the pair count) per pass; a crowded image that
+    overflows `cap` is run again with the size the kernel reported.
+
+    iou_type='masks': output['masks'] and target['masks'] are each a CUDA tensor [n, H, W] / [n, 1, H, W] (packed on
+    the fly by PackedMasks.from_dense: fp32 / fp16 set iff > 0.5, uint8 / bool iff nonzero) or a PackedMasks, with as
+    many rows as the boxes, on one (H, W) canvas.  inter / union are exact pixel counts, iou = float(inter) /
+    float(union); iou_min must be > 0.  Every (prediction, ground truth) pair of windows is tested once (O(k * g), as
+    the box path): sized for an image, not for region- or slide-scale ground truth (1e5+ nuclei per call)."""
+    if iou_type not in ('boxes', 'masks'):
+        raise HdyError(f"iou_type must be 'boxes' or 'masks', got {iou_type!r}")
     boxes, scores, gts = output['boxes'], output['scores'], target['boxes']
     _need_cuda(boxes, "output['boxes']")
     _need_cuda(scores, "output['scores']")
     _need_cuda(gts, "target['boxes']")
     dev = boxes.device
     k, g = int(boxes.shape[0]), int(gts.shape[0])
+    if iou_type == 'masks':
+        _check_mask_inputs(output, target, k, g, iou_min)
     i64 = dict(dtype=torch.int64, device=dev)
     empty = {'pred_idx': torch.empty(0, **i64), 'true_idx': torch.empty(0, **i64),
              'ious': torch.empty(0, dtype=torch.float32, device=dev)}
     if k == 0:
         return {'order': torch.empty(0, **i64), 'scores': scores.reshape(0), 'labels': output['labels'].reshape(0), **empty}
-    boxes = _aligned16(boxes.contiguous())
     # 1. predictions by score: one ascending radix sort of the (~score, row) keys (hdy_sort_keys_bytes), row = low word
     from .slide import sort_keys
     scores = scores.contiguous()
@@ -64,22 +76,19 @@ def match_predictions(output: Dict[str, torch.Tensor], target: Dict[str, torch.T
     res = {'order': order, 'scores': scores[order], 'labels': output['labels'][order]}
     if g == 0:
         return {**res, **empty}
-    gts = _aligned16(gts.contiguous())
-    # 2. pairs with iou >= iou_min
+    # 2. pairs with iou >= iou_min, as order keys (~orderable(iou) << 32 | rank * g + j)
+    if iou_type == 'masks':
+        launch = _mask_pairs(_packed(output['masks']), _packed(target['masks']), order32, k, g, iou_min)
+    else:
+        launch = _box_pairs(_aligned16(boxes.contiguous()), order32, _aligned16(gts.contiguous()), k, g, iou_min)
     cap = int(cap) if cap is not None else max(4 * max(k, g), 1024)
     while True:
-        pk = torch.empty(cap, dtype=torch.int64, device=dev)
-        pb = torch.empty((cap, 4), dtype=torch.float32, device=dev)
-        pc = _Cand.__new__(_Cand)
-        pc.bs, pc.cap, pc.keys, pc.boxes, pc.cls = 1, cap, pk, pb, None
-        pc.counts = torch.zeros(2, dtype=torch.int32, device=dev)
-        kc = torch.tensor([k, g], dtype=torch.int32).to(dev)
-        _call("hdy_match_pairs", ptr(boxes), ptr(order32), ptr(kc[0:1]), 1, k, ptr(gts), ptr(kc[1:2]), g,
-              float(np.float32(iou_min)), cap, ptr(pk), ptr(pb), ptr(pc.counts), pc.status_ptr, _stream())
-        n_match = int(pc.counts[0].item())          # the reference's torch.where synchronises here too
-        if n_match <= cap:
+        pk, needs = launch(cap)
+        needs = needs.tolist()                        # the reference's torch.where synchronises here too
+        n_match = needs[0]
+        if max(needs) <= cap:
             break
-        cap = n_match                                 # a crowded image: retry with the size the kernel reported
+        cap = max(needs)                              # a crowded image: retry with the size the kernel reported
     if n_match == 0:
         return {**res, **empty}
     # 3. IoU-descending order of the pairs: a key sort (pairs of one prediction share a box -- as an "NMS that only
@@ -89,6 +98,75 @@ def match_predictions(output: Dict[str, torch.Tensor], target: Dict[str, torch.T
     pidx = pk & 0xffffffff
     res.update({'pred_idx': pidx // g, 'true_idx': pidx % g, 'ious': _key_scores(pk)})
     return res
+
+
+def _box_pairs(boxes, order32, gts, k, g, iou_min):
+    """launch(cap) -> (pair keys [cap], counts needed: [pairs]) over hdy_match_pairs."""
+    dev = boxes.device
+
+    def launch(cap):
+        pk = torch.empty(cap, dtype=torch.int64, device=dev)
+        pb = torch.empty((cap, 4), dtype=torch.float32, device=dev)
+        pc = _Cand.__new__(_Cand)
+        pc.bs, pc.cap, pc.keys, pc.boxes, pc.cls = 1, cap, pk, pb, None
+        pc.counts = torch.zeros(2, dtype=torch.int32, device=dev)
+        kc = torch.tensor([k, g], dtype=torch.int32).to(dev)
+        _call("hdy_match_pairs", ptr(boxes), ptr(order32), ptr(kc[0:1]), 1, k, ptr(gts), ptr(kc[1:2]), g,
+              float(np.float32(iou_min)), cap, ptr(pk), ptr(pb), ptr(pc.counts), pc.status_ptr, _stream())
+        return pk, pc.counts[:1]
+    return launch
+
+
+def _mask_pairs(pm: PackedMasks, gm: PackedMasks, order32, k, g, iou_min):
+    """launch(cap) -> (pair keys [cap], counts needed: [pairs, candidates]) over hdy_match_mask_pairs; `cap` bounds
+    both lists (every pair is a candidate)."""
+    dev = order32.device
+    ap, ag = pm.areas(), gm.areas()
+    pgeom, ggeom = _aligned16(pm.geom.contiguous()), _aligned16(gm.geom.contiguous())
+    pbits, gbits = pm._bits_nonempty(), gm._bits_nonempty()
+
+    def launch(cap):
+        cand = torch.empty(cap, dtype=torch.int32, device=dev)
+        pk = torch.empty(cap, dtype=torch.int64, device=dev)
+        counts = torch.zeros(3, dtype=torch.int32, device=dev)     # pairs, candidates, status
+        _call("hdy_match_mask_pairs", ptr(pgeom), ptr(pm.offsets), ptr(pbits), ptr(ap), ptr(order32), k, ptr(ggeom),
+              ptr(gm.offsets), ptr(gbits), ptr(ag), g, float(np.float32(iou_min)), cap, ptr(cand), cap, ptr(pk),
+              ptr(counts), ptr(counts[2:]), _stream(), launches=2)
+        return pk, counts[:2]
+    return launch
+
+
+def _mask_canvas(m, n: int, name: str):
+    if isinstance(m, PackedMasks):
+        rows, hw = len(m), (m.H, m.W)
+        if not (m.geom.is_cuda and m.offsets.is_cuda and m.bits.is_cuda):
+            raise HdyError(f"{name} must live on a CUDA device: hd_yolo_b200 has no CPU fallback")
+    elif isinstance(m, torch.Tensor):
+        if m.dim() not in (3, 4) or (m.dim() == 4 and m.shape[1] != 1):
+            raise HdyError(f"{name} must be [n, H, W] or [n, 1, H, W], got {tuple(m.shape)}")
+        rows, hw = int(m.shape[0]), tuple(int(s) for s in m.shape[-2:])
+    else:
+        raise HdyError(f"{name} must be a CUDA tensor or a PackedMasks, got {type(m).__name__}")
+    if rows != n:
+        raise HdyError(f"{name} has {rows} rows for {n} boxes")
+    return hw
+
+
+def _check_mask_inputs(output, target, k: int, g: int, iou_min: float) -> None:
+    if 'masks' not in output or 'masks' not in target:
+        raise HdyError("iou_type='masks' needs 'masks' in both output and target")
+    if not iou_min > 0:
+        raise HdyError(f"mask matching needs iou_min > 0 (pairs of disjoint masks have IoU 0), got {iou_min}")
+    cp, cg = _mask_canvas(output['masks'], k, "output['masks']"), _mask_canvas(target['masks'], g, "target['masks']")
+    if cp != cg:
+        raise HdyError(f"predicted masks lie on a {cp[0]} x {cp[1]} canvas, ground-truth masks on {cg[0]} x {cg[1]}")
+
+
+def _packed(m) -> PackedMasks:
+    if isinstance(m, PackedMasks):
+        m.check()                                     # an overflowed plane lacks bits: its IoUs would be wrong
+        return m
+    return PackedMasks.from_dense(m)
 
 
 def _key_scores(keys: torch.Tensor) -> torch.Tensor:
@@ -118,9 +196,9 @@ class APMeter(object):
         self.m_true = torch.empty(0, dtype=torch.int64)
 
     def add(self, output, target, iou_type='boxes'):
-        if iou_type == 'masks' and ('masks' in output and 'masks' in target):
-            raise HdyError("mask IoU matching is not on the device path; use iou_type='boxes'")
-        m = match_predictions(output, target, float(self.iouv.min()))
+        # the reference's rule: mask IoU when asked for and both sides carry masks, box IoU otherwise
+        use_masks = iou_type == 'masks' and ('masks' in output and 'masks' in target)
+        m = match_predictions(output, target, float(self.iouv.min()), iou_type='masks' if use_masks else 'boxes')
         n_pred, n_true = int(output['boxes'].shape[0]), int(target['boxes'].shape[0])
         self.m_pred = torch.cat([self.m_pred, (m['pred_idx'] + self.n_pred).cpu()])
         self.m_true = torch.cat([self.m_true, (m['true_idx'] + self.n_true).cpu()])

@@ -141,3 +141,43 @@ def slide_tile_protos(n: int, tile: int, seed: int, first_tile: int = 0, nm: int
         g.manual_seed(_tile_seed(seed + 77, first_tile + b))
         out[b] = torch.randn((nm, mh, mh), generator=g, device=dev).to(dtype)
     return out
+
+
+def ellipse_masks(centres: torch.Tensor, radii: torch.Tensor, H: int, W: int, chunk: int = 256) -> torch.Tensor:
+    """Filled axis-aligned ellipses: centres / radii [n, 2] (x, y) in pixels -> [n, H, W] bool on their device."""
+    dev = centres.device
+    n = int(centres.shape[0])
+    out = torch.empty((n, H, W), dtype=torch.bool, device=dev)
+    y = torch.arange(H, dtype=torch.float32, device=dev)[None, :, None] + 0.5
+    x = torch.arange(W, dtype=torch.float32, device=dev)[None, None, :] + 0.5
+    for i in range(0, n, chunk):
+        c, r = centres[i:i + chunk, :, None, None], radii[i:i + chunk, :, None, None]
+        out[i:i + chunk] = ((x - c[:, 0]) / r[:, 0]) ** 2 + ((y - c[:, 1]) / r[:, 1]) ** 2 <= 1.0
+    return out
+
+
+def nuclei_match_case(k: int, g: int, size: int, seed: int, device="cuda"):
+    """Seeded inputs of mask matching on a size x size canvas: g ground-truth nuclei (filled ellipses 12-36 px across),
+    min(k, g) predictions that are jittered copies of them plus k - min(k, g) false positives, in random order; scores
+    quantised to 1/256 (ties).  Returns (output, target) dicts of 'boxes' (the ellipses' boxes), 'scores', 'labels',
+    'masks' ([n, size, size] bool) on `device`."""
+    gen = torch.Generator().manual_seed(seed)
+    cg = torch.rand((g, 2), generator=gen) * size
+    rg = 6.0 + 12.0 * torch.rand((g, 2), generator=gen)
+    m = min(k, g)
+    cp = torch.cat([cg[:m] + torch.randn((m, 2), generator=gen) * 1.5, torch.rand((k - m, 2), generator=gen) * size])
+    rp = torch.cat([rg[:m] * (1.0 + 0.08 * torch.randn((m, 2), generator=gen)),
+                    6.0 + 12.0 * torch.rand((k - m, 2), generator=gen)]).clamp_min(1.0)
+    perm = torch.randperm(k, generator=gen)
+    cp, rp = cp[perm], rp[perm]
+    scores = (torch.rand(k, generator=gen) * 256).round() / 256
+    labels_p, labels_g = torch.randint(-1, 5, (k,), generator=gen), torch.randint(1, 5, (g,), generator=gen)
+
+    def side(c, r, scores_labels):
+        c, r = c.to(device), r.to(device)
+        d = {'boxes': torch.cat([c - r, c + r], 1).clamp(0, size).contiguous(),
+             'masks': ellipse_masks(c, r, size, size)}
+        d.update({key: v.to(device) for key, v in scores_labels.items()})
+        return d
+
+    return side(cp, rp, {'scores': scores, 'labels': labels_p}), side(cg, rg, {'labels': labels_g})

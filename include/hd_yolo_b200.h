@@ -508,6 +508,36 @@ HDY_API int hdy_match_pairs(const float* pred_boxes, const int32_t* pred_order, 
 /* box_iou (metayolo/models/utils_general.py:247-265): out [n, m] fp32, 0/0 = NaN as in the reference. */
 HDY_API int hdy_box_iou(const float* box1, int64_t n, const float* box2, int64_t m, float* out, hdy_stream_t stream);
 
+/* f2 by mask IoU (APMeter.add(..., iou_type='masks'), metrics.py:270-303), over the cropped bit-packed layout above.
+ * A pixel is set iff its value is > 0.5 (HDY_F32, HDY_F16) or nonzero (HDY_U8: uint8 or bool masks).
+ * Dense [K, H, W] masks (H * W < 2^31) -> bit planes with TIGHT windows (bounding rectangle of the set pixels; an empty
+ * mask gets w = h = 0): hdy_pack_masks_geometry fills geom [K,4] (16-byte aligned) and offsets [K+1] (offsets[K] =
+ * total words), hdy_pack_masks writes `bits` (padding bits beyond w are zero; masks that do not fit capacity_words set
+ * HDY_STATUS_OVERFLOW in *status). */
+#define HDY_U8 2
+HDY_API int hdy_pack_masks_geometry(const void* masks, int dtype, int K, int H, int W, int32_t* geom, int64_t* offsets,
+                                    hdy_stream_t stream);
+HDY_API int hdy_pack_masks(const void* masks, int dtype, int K, int H, int W, const int32_t* geom,
+                           const int64_t* offsets, uint32_t* bits, int64_t capacity_words, int32_t* status,
+                           hdy_stream_t stream);
+/* areas [K] i32: set pixels per mask.  The bits beyond w in each row's last word are ignored, whatever they hold. */
+HDY_API int hdy_mask_areas(const int32_t* geom, const int64_t* offsets, const uint32_t* bits, int K, int32_t* areas,
+                           hdy_stream_t stream);
+/* The mask form of hdy_match_pairs for one image.  Both mask sets lie on one canvas (the caller checks); areas from
+ * hdy_mask_areas; pred_order [P] i32 (rank in score order -> row; NULL: rows are already in order).  inter = pixels
+ * set in both, union = area_p + area_g - inter, iou = float(inter) / float(union) (round to nearest, 0/0 = NaN).
+ * Two phases: the pairs whose windows overlap and whose IoU bound float(min(overlap, area_p, area_g)) / float(union)
+ * reaches iou_min go to cand [cand_cap] (u32 rank * G + j; counts[1] = their number), then every candidate's
+ * intersection is counted exactly and the pairs with iou >= iou_min are appended to pair_keys [cap] as in
+ * hdy_match_pairs (counts[0]).  counts [2] is zeroed by the caller; either list overflowing sets HDY_STATUS_OVERFLOW
+ * in *status and its count holds the size needed (call again: cand_cap >= counts[1] and cap >= counts[0]).
+ * iou_min > 0 (pairs of disjoint masks are never listed); P * G < 2^32.  Cost O(P * G) window tests per image. */
+HDY_API int hdy_match_mask_pairs(const int32_t* pred_geom, const int64_t* pred_offsets, const uint32_t* pred_bits,
+                                 const int32_t* pred_areas, const int32_t* pred_order, int P, const int32_t* gt_geom,
+                                 const int64_t* gt_offsets, const uint32_t* gt_bits, const int32_t* gt_areas, int G,
+                                 float iou_min, int cand_cap, uint32_t* cand, int cap, uint64_t* pair_keys,
+                                 int32_t* counts, int32_t* status, hdy_stream_t stream);
+
 /* Utility: zero n int32 words (keeps the host mirror free of extra torch launches). */
 HDY_API int hdy_zero_i32(int32_t* p, size_t n, hdy_stream_t stream);
 
