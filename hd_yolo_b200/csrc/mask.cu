@@ -259,20 +259,6 @@ __global__ void unpack_masks_kernel(const int32_t* __restrict__ geom4, const int
   }
 }
 
-__global__ void pm_geometry_kernel(const float4* __restrict__ boxes, const int32_t* __restrict__ counts, int bs,
-                                   int max_det, int mh, int mw, int ih, int iw, int upsample, float rx, float ry,
-                                   int32_t* __restrict__ geom4) {
-  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= (long long)bs * max_det) return;
-  const int tile = (int)(i / max_det), d = (int)(i - (long long)tile * max_det);
-  int4 out = make_int4(0, 0, 0, 0);
-  if (d < counts[tile]) {
-    const PMGeom g = pm_geometry(boxes[i], mh, mw, ih, iw, upsample, rx, ry);
-    out = make_int4(g.x0, g.y0, g.w, g.h);
-  }
-  reinterpret_cast<int4*>(geom4)[i] = out;
-}
-
 // words(i) of hdy_process_mask_geometry: the window of slot i, stored to geom4 on the way, so that the geometry and the
 // first pass of the scan are one launch (the step is a chain of small dependent kernels)
 struct PmWindowWords {
@@ -329,50 +315,34 @@ __global__ void pm_rows_kernel(int32_t* __restrict__ geom4, int64_t* __restrict_
 
 constexpr int kPmThreads = 128;
 
-// One CTA per detection slot (slot_list == NULL: CTA b handles slot b, all of its proto tiles), or the 2-D grid of the
-// listed form: the CTAs share the listed slots -- the detections too large for the patch path of mask_regions.cu --
-// AND the proto tiles of every slot: blockIdx.y strides the list, blockIdx.x the 32 x 32 proto tiles of a detection.
-// A 1 000-px false positive is 60 tiles; walked by one CTA it took longer than the whole patch path of its batch.
+// One CTA per detection slot, all of its proto tiles: the path of the shapes, workspaces and (packed) missing windows
+// that mask_regions.cu does not take
 template <bool PACKED, bool HALF>
 __global__ void __launch_bounds__(kPmThreads) process_mask_kernel(
     const void* __restrict__ protos, const float* __restrict__ coef, const float4* __restrict__ boxes,
     const int32_t* __restrict__ counts, int max_det, int nm, int mh, int mw, int ih, int iw, int upsample,
     float rx, float ry, float* __restrict__ out_dense, const int32_t* __restrict__ geom4,
     const int64_t* __restrict__ offsets,
-    uint32_t* __restrict__ bits, long long capacity_words, int32_t* __restrict__ status,
-    const int32_t* __restrict__ slot_list, const int32_t* __restrict__ list_count) {
+    uint32_t* __restrict__ bits, long long capacity_words, int32_t* __restrict__ status) {
   __shared__ float stage[kPmStage * kPmStage];
   __shared__ float cf[64];
-  const long long n_items = slot_list ? (long long)*list_count : (long long)gridDim.x;
   process_mask_body<PACKED, HALF>(protos, coef, boxes, counts, max_det, nm, mh, mw, ih, iw, upsample, rx, ry, out_dense,
-                                  geom4, offsets, bits, capacity_words, status, slot_list, n_items,
-                                  slot_list ? blockIdx.y : blockIdx.x, slot_list ? gridDim.y : gridDim.x,
-                                  slot_list ? (int)blockIdx.x : 0, slot_list ? (int)gridDim.x : 1, stage, cf);
+                                  geom4, offsets, bits, capacity_words, status, nullptr, gridDim.x, blockIdx.x,
+                                  gridDim.x, 0, 1, stage, cf);
 }
 
-// used by mask_regions.cu for the detections its two-phase path leaves out
-int launch_process_mask_listed(const void* protos, int proto_dtype, const float* coef, const float* boxes,
-                               const int32_t* counts, int max_det, int nm, int mh, int mw, int ih, int iw, int upsample, float rx, float ry,
-                               float* out_dense, const int64_t* offsets, uint32_t* bits, long long capacity_words,
-                               int32_t* status, const int32_t* slot_list, const int32_t* list_count,
-                               cudaStream_t st) {
-  // x: proto tiles of a detection, y: listed detections.  The list is short (a few background false positives per
-  // batch of 148 tiles) and each item large (up to 64 proto tiles): the call's duration is the longest item's walk, so
-  // one CTA per tile of the largest box (64 x 9 = 576 CTAs; those without a tile leave after reading the geometry)
-  const dim3 grid(64, 9);
-  const float4* b4 = reinterpret_cast<const float4*>(boxes);
-  const bool half = proto_dtype == HDY_F16;
-#define HDY_PM(P, H)                                                                                               \
-  process_mask_kernel<P, H><<<grid, kPmThreads, 0, st>>>(protos, coef, b4, counts, max_det, nm, mh, mw, ih, iw,    \
-                                                         upsample, rx, ry, out_dense, nullptr, offsets, bits,      \
-                                                         capacity_words, status, slot_list, list_count)
-  if (out_dense) {
-    if (half) HDY_PM(false, true); else HDY_PM(false, false);
-  } else {
-    if (half) HDY_PM(true, true); else HDY_PM(true, false);
-  }
-#undef HDY_PM
-  return check_launch("hdy_process_mask(listed)");
+template <bool PACKED>
+static int launch_process_mask_kernel(const void* protos, int proto_dtype, const float* coef, const float* boxes,
+                                      const int32_t* counts, int bs, int max_det, int nm, int mh, int mw, int ih,
+                                      int iw, int upsample, float rx, float ry, float* out_dense,
+                                      const int32_t* geom, const int64_t* offsets, uint32_t* bits,
+                                      long long capacity_words, int32_t* status, cudaStream_t st, const char* what) {
+  const auto kernel = proto_dtype == HDY_F16 ? process_mask_kernel<PACKED, true> : process_mask_kernel<PACKED, false>;
+  kernel<<<(unsigned)((size_t)bs * max_det), kPmThreads, 0, st>>>(protos, coef, reinterpret_cast<const float4*>(boxes),
+                                                                   counts, max_det, nm, mh, mw, ih, iw, upsample, rx,
+                                                                   ry, out_dense, geom, offsets, bits, capacity_words,
+                                                                   status);
+  return check_launch(what);
 }
 
 static int paste_args_ok(const float* src, const float* boxes, int K, int C, int M, int pad, int H, int W) {
@@ -510,16 +480,9 @@ int hdy_process_mask(const void* protos, int proto_dtype, const float* coef, con
   rc = launch_process_mask_regions(protos, proto_dtype, coef, boxes, counts, bs, max_det, nm, mh, mw, ih, iw, upsample,
                                    rx, ry, out, nullptr, nullptr, nullptr, 0, nullptr, workspace, workspace_bytes, st);
   if (rc != 1) return rc;
-  const float4* b4 = reinterpret_cast<const float4*>(boxes);
-  if (proto_dtype == HDY_F16)
-    process_mask_kernel<false, true><<<(unsigned)((size_t)bs * max_det), kPmThreads, 0, st>>>(
-        protos, coef, b4, counts, max_det, nm, mh, mw, ih, iw, upsample, rx, ry, out, nullptr, nullptr, nullptr, 0,
-        nullptr, nullptr, nullptr);
-  else
-    process_mask_kernel<false, false><<<(unsigned)((size_t)bs * max_det), kPmThreads, 0, st>>>(
-        protos, coef, b4, counts, max_det, nm, mh, mw, ih, iw, upsample, rx, ry, out, nullptr, nullptr, nullptr, 0,
-        nullptr, nullptr, nullptr);
-  return check_launch("hdy_process_mask");
+  return launch_process_mask_kernel<false>(protos, proto_dtype, coef, boxes, counts, bs, max_det, nm, mh, mw, ih, iw,
+                                           upsample, rx, ry, out, nullptr, nullptr, nullptr, 0, nullptr, st,
+                                           "hdy_process_mask");
 }
 
 int hdy_process_mask_geometry(const float* boxes, const int32_t* counts, int bs, int max_det, int mh, int mw, int ih,
@@ -578,16 +541,9 @@ int hdy_process_mask_packed(const void* protos, int proto_dtype, const float* co
     set_error("cudaMemsetAsync: %s", cudaGetErrorString(e));
     return HDY_ERR_CUDA;
   }
-  const float4* b4 = reinterpret_cast<const float4*>(boxes);
-  if (proto_dtype == HDY_F16)
-    process_mask_kernel<true, true><<<(unsigned)((size_t)bs * max_det), kPmThreads, 0, st>>>(
-        protos, coef, b4, counts, max_det, nm, mh, mw, ih, iw, upsample, rx, ry, nullptr, geom, offsets, bits,
-        capacity_words, status, nullptr, nullptr);
-  else
-    process_mask_kernel<true, false><<<(unsigned)((size_t)bs * max_det), kPmThreads, 0, st>>>(
-        protos, coef, b4, counts, max_det, nm, mh, mw, ih, iw, upsample, rx, ry, nullptr, geom, offsets, bits,
-        capacity_words, status, nullptr, nullptr);
-  return check_launch("hdy_process_mask_packed");
+  return launch_process_mask_kernel<true>(protos, proto_dtype, coef, boxes, counts, bs, max_det, nm, mh, mw, ih, iw,
+                                          upsample, rx, ry, nullptr, geom, offsets, bits, capacity_words, status, st,
+                                          "hdy_process_mask_packed");
 }
 
 }  // extern "C"

@@ -29,20 +29,40 @@ __device__ __forceinline__ float bilerp(float v00, float v01, float v10, float v
 }
 
 // ------------------------------------------------------------------------------------- (B) process_mask
-// Window of mask i in output pixels.  crop_mask keeps proto pixels with x1d <= col < x2d, y1d <= row < y2d
-// (float compares against arange); with upsample the bilinear taps spread every kept pixel over its
-// neighbours, so the output window is the pre-image of [p0-1, p1) under i0 = floor(src).
-struct PMGeom {
-  float x1d, y1d, x2d, y2d;  // down-scaled box (fp32, as the reference computes it)
-  int px0, py0, px1, py1;    // kept proto pixel range [p0, p1)
-  int x0, y0, w, h;          // output window
-};
-
 __device__ __forceinline__ int ceil_to_int_clamped(float v, int lo, int hi) {
   if (!(v > (float)lo)) return lo;  // also NaN
   if (v >= (float)hi) return hi;
   return (int)ceilf(v);
 }
+
+// The proto pixels crop_mask keeps: x1d <= col < x2d, y1d <= row < y2d (float compares against arange).
+struct KeptRange {
+  float x1d, y1d, x2d, y2d;  // down-scaled box (fp32, as the reference computes it)
+  int px0, py0, px1, py1;    // kept proto pixel range [p0, p1)
+};
+__device__ __forceinline__ KeptRange kept_range(const float4 b, float rx, float ry, int mw, int mh) {
+  KeptRange k;
+  k.x1d = __fmul_rn(b.x, rx);  // downsampled_bboxes[:, 0] *= mw / iw ...
+  k.x2d = __fmul_rn(b.z, rx);
+  k.y1d = __fmul_rn(b.y, ry);
+  k.y2d = __fmul_rn(b.w, ry);
+  // r >= x1 & r < x2 over integers r: [ceil(x1), ceil(x2))
+  k.px0 = ceil_to_int_clamped(k.x1d, 0, mw);
+  k.px1 = ceil_to_int_clamped(k.x2d, 0, mw);
+  k.py0 = ceil_to_int_clamped(k.y1d, 0, mh);
+  k.py1 = ceil_to_int_clamped(k.y2d, 0, mh);
+  // a NaN coordinate fails every crop comparison of the reference: nothing is kept.  For finite coordinates the crop
+  // test x1d <= col < x2d over integer columns IS col in [px0, px1), so the two-phase kernels walk the integer range
+  // and never compare against the floats again.
+  if (!(k.x1d == k.x1d) || !(k.x2d == k.x2d) || !(k.y1d == k.y1d) || !(k.y2d == k.y2d)) k.px1 = k.px0, k.py1 = k.py0;
+  return k;
+}
+
+// Window of mask i in output pixels.  With upsample the bilinear taps spread every kept pixel over its neighbours, so
+// the output window is the pre-image of [p0-1, p1) under i0 = floor(src).
+struct PMGeom : KeptRange {
+  int x0, y0, w, h;  // output window
+};
 
 // Source coordinate of output pixel `dst` exactly as lerp_coord (ATen) computes it.
 __device__ __forceinline__ float pm_src(int dst, float scale) {
@@ -81,18 +101,7 @@ __device__ __forceinline__ void pm_trim(int& o0, int& o1, int p0, int p1, int in
 __device__ __forceinline__ PMGeom pm_geometry(const float4 b, int mh, int mw, int ih, int iw, int upsample,
                                               float rx, float ry) {
   PMGeom g;
-  g.x1d = __fmul_rn(b.x, rx);  // downsampled_bboxes[:, 0] *= mw / iw
-  g.x2d = __fmul_rn(b.z, rx);
-  g.y1d = __fmul_rn(b.y, ry);
-  g.y2d = __fmul_rn(b.w, ry);
-  // r >= x1 & r < x2 over integers r: [ceil(x1), ceil(x2))
-  g.px0 = ceil_to_int_clamped(g.x1d, 0, mw);
-  g.px1 = ceil_to_int_clamped(g.x2d, 0, mw);
-  g.py0 = ceil_to_int_clamped(g.y1d, 0, mh);
-  g.py1 = ceil_to_int_clamped(g.y2d, 0, mh);
-  // a NaN coordinate fails every crop comparison of the reference (r >= x1 ...): the mask is empty
-  const bool nan = !(g.x1d == g.x1d) || !(g.x2d == g.x2d) || !(g.y1d == g.y1d) || !(g.y2d == g.y2d);
-  if (nan) g.px1 = g.px0, g.py1 = g.py0;
+  static_cast<KeptRange&>(g) = kept_range(b, rx, ry, mw, mh);
   if (g.px1 <= g.px0 || g.py1 <= g.py0) {
     g.x0 = g.y0 = g.w = g.h = 0;
     return g;
@@ -259,7 +268,8 @@ __device__ __forceinline__ void process_mask_body(
 
 
 // mask_regions.cu: two-phase process_mask (TMA-staged prototypes -> sigmoid patches -> upsample + pack).  Returns 1
-// when the shapes / workspace do not meet its requirements (the caller then uses the per-detection kernel in mask.cu).
+// when the shapes / workspace / windows do not meet its requirements (the caller then uses the per-detection kernel in
+// mask.cu).
 constexpr int kPatchPitch = 16;  // sigmoid patches of up to 16 x 16 proto pixels go through the workspace
 size_t process_mask_workspace_bytes(long long bs, long long max_det);
 int launch_process_mask_regions(const void* protos, int proto_dtype, const float* coef, const float* boxes,
@@ -267,10 +277,5 @@ int launch_process_mask_regions(const void* protos, int proto_dtype, const float
                                 float ry, float* out_dense, const int32_t* geom, const int64_t* offsets, uint32_t* bits,
                                 long long capacity_words, int32_t* status, void* workspace, size_t workspace_bytes,
                                 cudaStream_t stream);
-// mask.cu: the per-detection kernel over a device-side list of slots
-int launch_process_mask_listed(const void* protos, int proto_dtype, const float* coef, const float* boxes,
-                               const int32_t* counts, int max_det, int nm, int mh, int mw, int ih, int iw, int upsample, float rx, float ry,
-                               float* out_dense, const int64_t* offsets, uint32_t* bits, long long capacity_words,
-                               int32_t* status, const int32_t* slot_list, const int32_t* list_count, cudaStream_t st);
 
 }  // namespace hdy

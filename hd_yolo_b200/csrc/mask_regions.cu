@@ -5,26 +5,30 @@
 // the reference repo has no such function, see DESIGN.md), identical to process_mask_kernel in mask.cu.
 //
 // A tile's prototypes are [32, mh, mw] fp32 (8.4 MB at 1024 px); a nucleus touches a ~10x10 window of all 32 planes
-// and produces a ~36x36 output window.  The two halves of the work want different decompositions:
+// and produces a ~36x36 output window.  The two halves of the work want different decompositions.  Every output form
+// (dense or bit-packed, upsampled or at proto resolution) runs the same launches:
 //
-//   phase 1  proto_patch_kernel, one CTA per (tile, 24x24 proto REGION).  ONE 4-D TMA tile load
-//            (cp.async.bulk.tensor.4d, SASS UTMALDG; out-of-bounds zero-filled by the TMA unit) brings the region's
-//            24x24x32 box into 72 KB of shared memory, so every proto element leaves HBM/L2 exactly once.  While it is
-//            in flight the CTA lists the tile's detections whose box reaches into the region; then one warp per
-//            (detection, region) piece computes the cropped sigmoid(coef . proto) of the piece's pixels (32 LDS + 32
-//            FFMA each) and writes them into the detection's PATCH (<= 16x16 floats) in the workspace.  Three CTAs
-//            per SM, no halo, no atomics.  The tile origin of a TMA load must be 16-byte aligned in the innermost
-//            dimension (measured: tools/micro/tma4d_test.cu faults otherwise), hence 24-pixel regions.
+//   phase 0  proto_bin_fused_kernel, one thread per slot: records the slot's kept proto range and appends the slot to
+//            the list of every 24x24 proto REGION the range touches.  Detections whose kept range exceeds 16x16 proto
+//            pixels (64 px boxes at the usual 4x), or that land in a region whose list is full, are handed over to the
+//            large list instead and their kept range is recorded as empty; the first kRegCap entries of a region's
+//            list are therefore every detection with a piece in it.  (Bit-packed forms: pm_clear_listed_kernel then
+//            clears the words of the listed detections, which the per-detection body ORs into.)
+//   phase 1  proto_patch_kernel, one CTA per (tile, region).  ONE 4-D TMA tile load (cp.async.bulk.tensor.4d, SASS
+//            UTMALDG; out-of-bounds zero-filled by the TMA unit) brings the region's 24x24x32 box into 72 KB of shared
+//            memory, so every proto element leaves HBM/L2 exactly once.  One warp per (detection, region) piece of
+//            the region's list computes the cropped sigmoid(coef . proto) of the piece's pixels (32 LDS + 32 FFMA
+//            each) and writes them into the detection's PATCH (<= 16x16 floats) in the workspace.  Three CTAs per SM,
+//            no halo, no atomics.  The tile origin of a TMA load must be 16-byte aligned in the innermost dimension
+//            (measured: tools/micro/tma4d_test.cu faults otherwise), hence 24-pixel regions.  The listed detections
+//            ride in the first CTAs of the same launch (ListedRide: the per-detection body of mask.cu).
 //   phase 2  one WARP per detection: the patch (with a ring of zeros: the crop) goes to shared memory and is
 //            upsampled with ATen's bilinear (align_corners=False) operation by operation, thresholded and stored.
 //            Every word of every mask is stored exactly once, so the bit planes need no clearing.
 //              * bit-packed + upsampled (the throughput form): mask_upsample_pack2_kernel (upsample_pack_v2 below).
 //              * the other forms (dense output, or packed at proto resolution): mask_upsample_pack_kernel.
-//   Detections whose kept range exceeds 16x16 proto pixels (64 px boxes at the usual 4x), or that fall into an overfull
-//   region, are listed and handled by the per-detection body of mask.cu.  In the packed + upsampled form they ride in
-//   the first CTAs of the phase-1 launch; in the other forms they get a launch of their own behind phase 2.
-//   The packed + upsampled form needs the windows of hdy_process_mask_geometry; without them the caller falls back to
-//   the per-detection kernel.
+//   The bit-packed forms need the windows of hdy_process_mask_geometry; without them the caller falls back to the
+//   per-detection kernel.
 #include <algorithm>
 
 #include "tma_common.cuh"
@@ -37,24 +41,11 @@ constexpr int kRegBoxX = 24, kRegBoxY = 24;
 constexpr int kRegNm = 32;
 constexpr int kRegThreads = 256;
 constexpr int kRegWarps = kRegThreads / 32;
-constexpr int kRegList = 512;  // detections examined per pass
-
-template <typename E>
-struct RegSmemT {
-  E proto[kRegNm][kRegBoxY][kRegBoxX];  // TMA destination (dense, x fastest); fp32, or fp16 widened on use
-  float coef[kRegWarps][kRegNm];
-  uint16_t list[kRegList];
-  int nlist;
-  int pad;
-  uint64_t bar;
-};
-__device__ __forceinline__ float proto_f32(float v) { return v; }
-__device__ __forceinline__ float proto_f32(__half v) { return __half2float(v); }  // exact
 
 // workspace: [0] large-detection counter, [1] slot ticket of the packed upsample, large list (int32 per slot), the
 // patches, then the per-region detection lists (count + kRegCap uint16 entries per (tile, region); sized for the
 // largest proto plane, see kMaxRegions)
-constexpr int kRegCap = 254;          // detections listed per region; a region with more falls back to scanning
+constexpr int kRegCap = 254;          // detections listed per region; the binning hands any more to the large list
 constexpr int kMaxRegionsPerTile = 512;  // ceil(mw/24) * ceil(mh/24) <= 512 covers planes up to 528 x 528 (2112 px tiles)
 struct RegionList {
   int32_t count;
@@ -91,26 +82,15 @@ static PmWorkspace pm_workspace(void* base, long long slots) {
   return w;
 }
 
-struct KeptRange {
-  float x1d, y1d, x2d, y2d;
-  int px0, py0, px1, py1;
+template <typename E>
+struct RegSmemT {
+  E proto[kRegNm][kRegBoxY][kRegBoxX];  // TMA destination (dense, x fastest); fp32, or fp16 widened on use
+  float coef[kRegWarps][kRegNm];
+  uint16_t list[kRegCap];
+  uint64_t bar;
 };
-__device__ __forceinline__ KeptRange kept_range(const float4 b, float rx, float ry, int mw, int mh) {
-  KeptRange k;
-  k.x1d = __fmul_rn(b.x, rx);  // downsampled_bboxes[:, 0] *= mw / iw ...
-  k.x2d = __fmul_rn(b.z, rx);
-  k.y1d = __fmul_rn(b.y, ry);
-  k.y2d = __fmul_rn(b.w, ry);
-  k.px0 = ceil_to_int_clamped(k.x1d, 0, mw);
-  k.px1 = ceil_to_int_clamped(k.x2d, 0, mw);
-  k.py0 = ceil_to_int_clamped(k.y1d, 0, mh);
-  k.py1 = ceil_to_int_clamped(k.y2d, 0, mh);
-  // a NaN coordinate fails every crop comparison of the reference: nothing is kept.  For finite coordinates the crop
-  // test x1d <= col < x2d over integer columns IS col in [px0, px1) (px = ceil, clamped), so the kernels below walk the
-  // integer range and never compare against the floats again.
-  if (!(k.x1d == k.x1d) || !(k.x2d == k.x2d) || !(k.y1d == k.y1d) || !(k.y2d == k.y2d)) k.px1 = k.px0, k.py1 = k.py0;
-  return k;
-}
+__device__ __forceinline__ float proto_f32(float v) { return v; }
+__device__ __forceinline__ float proto_f32(__half v) { return __half2float(v); }  // exact
 
 // floor(v / pw) for 0 <= v < 64 and 1 <= pw <= 16 as (v * ceil(2^16 / pw)) >> 16 (exact while v * pw < 2^16): the
 // piece loops split the 32 lanes into floor(32 / pw) rows of pw pixels, and an integer division costs ~20 instructions
@@ -118,33 +98,59 @@ __constant__ int c_inv16[17] = {0,     65536, 32768, 21846, 16384, 13108, 10923,
                                 7282,  6554,  5958,  5462,  5042,  4682,  4370,  4096};
 
 // ------------------------------------------------------------------------------------------------ phase 0
-// One thread per detection: append it to the list of every region its kept range touches (1-4 for a nucleus), so that
-// a phase-1 CTA does not have to scan the whole tile (121 regions x 2 650 boxes per 1024-px tile otherwise).
-__global__ void __launch_bounds__(256) proto_bin_kernel(const float4* __restrict__ boxes,
-                                                        const int32_t* __restrict__ counts, long long n_slots,
-                                                        int max_det, int mh, int mw, int rxn, int ryn, float rx,
-                                                        float ry, const int32_t* __restrict__ geom4,
-                                                        RegionList* __restrict__ regions, int4* __restrict__ kr) {
+// One thread per detection: record its kept proto range (so nobody recomputes it from the box) and append it to the
+// list of every region the range touches (1-4 for a nucleus), so that a phase-1 CTA does not have to scan the whole
+// tile (121 regions x 2 650 boxes per 1024-px tile otherwise).  A detection the patch path cannot take -- kept range
+// over 16 x 16 proto pixels, or a full region list -- goes to the large list with an empty kept range.
+__global__ void __launch_bounds__(256) proto_bin_fused_kernel(const float4* __restrict__ boxes,
+                                                              const int32_t* __restrict__ counts, long long n_slots,
+                                                              int max_det, int mh, int mw, int rxn, int ryn, float rx,
+                                                              float ry, const int32_t* __restrict__ geom4,
+                                                              RegionList* __restrict__ regions, int4* __restrict__ kr,
+                                                              int32_t* __restrict__ large_count,
+                                                              int32_t* __restrict__ large_list) {
   const long long slot = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (slot >= n_slots) return;
   const int tile = (int)(slot / max_det), d = (int)(slot - (long long)tile * max_det);
-  // a slot beyond counts, or (packed form) without an output window -- empty, or not KEPT by the slide-level merge --
-  // needs no patch: its kept range is recorded as empty
-  const bool live = d < counts[tile] && !(geom4 && (geom4[4 * slot + 2] <= 0 || geom4[4 * slot + 3] <= 0));
+  // beyond counts, or (bit-packed forms) an empty window -- empty, or not KEPT by the slide-level merge: no patch, an
+  // empty kept range
+  const bool live = d < counts[tile] && (!geom4 || (geom4[4 * slot + 2] > 0 && geom4[4 * slot + 3] > 0));
   KeptRange k;
   k.px0 = k.py0 = k.px1 = k.py1 = 0;
   if (live) k = kept_range(boxes[slot], rx, ry, mw, mh);
-  kr[slot] = make_int4(k.px0, k.py0, k.px1, k.py1);
-  if (k.px1 <= k.px0 || k.py1 <= k.py0) return;
-  if (k.px1 - k.px0 > kPatchPitch || k.py1 - k.py0 > kPatchPitch) return;  // per-detection kernel
-  const int rx0 = k.px0 / kRegBoxX, rx1 = (k.px1 - 1) / kRegBoxX;
-  const int ry0 = k.py0 / kRegBoxY, ry1 = (k.py1 - 1) / kRegBoxY;
-  for (int ryy = ry0; ryy <= ry1; ++ryy)
-    for (int rxx = rx0; rxx <= rx1; ++rxx) {
-      RegionList& R = regions[(size_t)tile * (rxn * ryn) + ryy * rxn + rxx];
-      const int pos = atomicAdd(&R.count, 1);
-      if (pos < kRegCap) R.det[pos] = (uint16_t)d;
+  bool leave = false;
+  if (k.px1 > k.px0 && k.py1 > k.py0) {
+    leave = k.px1 - k.px0 > kPatchPitch || k.py1 - k.py0 > kPatchPitch;
+    if (!leave) {
+      const int rx0 = k.px0 / kRegBoxX, rx1 = (k.px1 - 1) / kRegBoxX;
+      const int ry0 = k.py0 / kRegBoxY, ry1 = (k.py1 - 1) / kRegBoxY;
+      for (int ryy = ry0; ryy <= ry1; ++ryy)
+        for (int rxx = rx0; rxx <= rx1; ++rxx) {
+          RegionList& R = regions[(size_t)tile * (rxn * ryn) + ryy * rxn + rxx];
+          const int pos = atomicAdd(&R.count, 1);
+          if (pos < kRegCap)
+            R.det[pos] = (uint16_t)d;
+          else
+            leave = true;  // full region: hand the detection over (its entries in other lists now have an empty range)
+        }
     }
+    if (leave) large_list[atomicAdd(large_count, 1)] = (int32_t)slot;
+  }
+  kr[slot] = leave ? make_int4(0, 0, 0, 0) : make_int4(k.px0, k.py0, k.px1, k.py1);
+}
+
+// the words of the listed detections are cleared (bit-packed forms): the per-detection body ORs its bits in
+__global__ void pm_clear_listed_kernel(const int32_t* __restrict__ geom4, const int64_t* __restrict__ offsets,
+                                       uint32_t* __restrict__ bits, long long capacity_words,
+                                       const int32_t* __restrict__ list, const int32_t* __restrict__ list_count) {
+  const int n = *list_count;
+  for (int item = blockIdx.x; item < n; item += gridDim.x) {
+    const long long slot = list[item];
+    const int4 g = reinterpret_cast<const int4*>(geom4)[slot];
+    const long long words = (long long)((g.z + 31) >> 5) * g.w, off = offsets[slot];
+    if (off + words > capacity_words) continue;  // reported by the kernel that would have filled them
+    for (long long i = threadIdx.x; i < words; i += blockDim.x) bits[off + i] = 0u;
+  }
 }
 
 // ------------------------------------------------------------------------------------------------ phase 1
@@ -179,13 +185,15 @@ __device__ __forceinline__ void contract_piece(const E (*proto)[kRegBoxY][kRegBo
   }
 }
 
-// The detections the patch path leaves out (listed by the binning kernel: windows over 16 x 16 proto pixels, overfull
-// regions) ride in the same launch: the first `ctas` CTAs run the per-detection body of mask.cu on them (64 proto tiles
-// x ctas / 64 list strides), in a corner of the region buffer, while the others stream the regions.  As a kernel of its
-// own behind the upsample that work was a 27-70 us latency chain in a handful of CTAs at the end of every mask call.
+// The detections the patch path leaves out (listed by the binning kernel: windows over 16 x 16 proto pixels, full
+// region lists) ride in the same launch: the first kListedCtas CTAs run the per-detection body of mask.cu on them
+// (kListedTiles proto tiles x 9 list strides; a 1 000-px false positive is 60 tiles), in a corner of the region buffer,
+// while the others stream the regions.  As a kernel of its own behind the upsample that work was a 27-70 us latency
+// chain in a handful of CTAs at the end of every mask call.
 struct ListedRide {
   const void* protos;
   const float4* boxes;
+  float* out_dense;
   const int64_t* offsets;
   uint32_t* bits;
   int32_t* status;
@@ -193,28 +201,28 @@ struct ListedRide {
   const int32_t* list_count;
   long long capacity_words;
   float rx, ry;
-  int nm, mh, mw, ih, iw;
-  int ctas;   // 0: nothing rides (dense / not upsampled forms keep the separate launch)
+  int nm, mh, mw, ih, iw, upsample;
 };
 constexpr int kListedTiles = 64;
+constexpr int kListedCtas = kListedTiles * 9;
 
-template <typename E>
+template <typename E, bool PACKED>
 __global__ void __launch_bounds__(kRegThreads, 3) proto_patch_kernel(
     const __grid_constant__ CUtensorMap tmap, const float* __restrict__ coef, const int4* __restrict__ krs,
     const int32_t* __restrict__ counts, int max_det, int rxn, int ryn, float* __restrict__ patches,
     const RegionList* __restrict__ regions, const ListedRide LR) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  if ((int)blockIdx.x < LR.ctas) {
+  if ((int)blockIdx.x < kListedCtas) {
     float* stage = reinterpret_cast<float*>(smem_raw);
-    process_mask_body<true, sizeof(E) == 2>(LR.protos, coef, LR.boxes, counts, max_det, LR.nm, LR.mh, LR.mw, LR.ih, LR.iw,
-                                            1, LR.rx, LR.ry, nullptr, nullptr, LR.offsets, LR.bits, LR.capacity_words,
-                                            LR.status, LR.list, (long long)*LR.list_count,
-                                            (long long)(blockIdx.x / kListedTiles), (long long)(LR.ctas / kListedTiles),
-                                            (int)(blockIdx.x % kListedTiles), kListedTiles, stage,
-                                            stage + kPmStage * kPmStage);
+    process_mask_body<PACKED, sizeof(E) == 2>(LR.protos, coef, LR.boxes, counts, max_det, LR.nm, LR.mh, LR.mw, LR.ih,
+                                              LR.iw, LR.upsample, LR.rx, LR.ry, LR.out_dense, nullptr, LR.offsets,
+                                              LR.bits, LR.capacity_words, LR.status, LR.list,
+                                              (long long)*LR.list_count, (long long)(blockIdx.x / kListedTiles),
+                                              (long long)(kListedCtas / kListedTiles), (int)(blockIdx.x % kListedTiles),
+                                              kListedTiles, stage, stage + kPmStage * kPmStage);
     return;
   }
-  const int bid = (int)blockIdx.x - LR.ctas;
+  const int bid = (int)blockIdx.x - kListedCtas;
   RegSmemT<E>& S = *reinterpret_cast<RegSmemT<E>*>(smem_raw);
   const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
   const int per_tile = rxn * ryn;
@@ -222,10 +230,9 @@ __global__ void __launch_bounds__(kRegThreads, 3) proto_patch_kernel(
   const int RY = reg / rxn, RX = reg - RY * rxn;
   const int X0 = RX * kRegBoxX, Y0 = RY * kRegBoxY;
   const RegionList& RL = regions[bid];
-  const int listed = RL.count;
-  if (listed <= 0) return;  // nothing reaches into this region: no load at all
-  const bool use_list = listed <= kRegCap;
-  const int n = use_list ? listed : min(counts[tile], max_det);
+  // the count goes on past kRegCap when the list is full; the detections beyond it were handed to the large list
+  const int n = min(RL.count, kRegCap);
+  if (n <= 0) return;  // nothing reaches into this region: no load at all
 
   if (t == 0) {
     mbar_init(&S.bar, 1);
@@ -233,62 +240,34 @@ __global__ void __launch_bounds__(kRegThreads, 3) proto_patch_kernel(
     mbar_arrive_expect_tx(&S.bar, (uint32_t)sizeof(S.proto));
     tma_load_4d(&S.proto[0][0][0], &tmap, X0, Y0, 0, tile, &S.bar);
   }
-  bool loaded = false;
-  for (int base = 0; base < n; base += kRegList) {
-    __syncthreads();
-    if (t == 0) S.nlist = 0;
-    __syncthreads();
-    const int lim = min(base + kRegList, n);
-    if (use_list) {
-      // the binning pass already listed the detections of this region
-      for (int i = base + t; i < lim; i += kRegThreads) S.list[i - base] = RL.det[i];
-      if (t == 0) S.nlist = lim - base;
-    } else {
-      // overfull list (more than kRegCap detections in one region): scan the tile (slots the binning pass skipped --
-      // beyond counts, empty, not KEPT -- carry no kept range of this launch: they are filtered by counts / geometry
-      // in the binning pass only, so the scan re-checks the range itself)
-      for (int d = base + t; d < lim; d += kRegThreads) {
-        const int4 k = krs[(size_t)tile * max_det + d];
-        if (k.z <= k.x || k.w <= k.y) continue;
-        if (k.z - k.x > kPatchPitch || k.w - k.y > kPatchPitch) continue;  // per-detection kernel
-        if (k.z <= X0 || k.x >= X0 + kRegBoxX || k.w <= Y0 || k.y >= Y0 + kRegBoxY) continue;
-        S.list[atomicAdd(&S.nlist, 1)] = (uint16_t)(d - base);
-      }
-    }
-    __syncthreads();
-    const int nl = S.nlist;
-    // software pipeline over this warp's pieces: the kept range and the coefficients of the NEXT piece are requested
-    // before the current one is computed (and those of the first piece before waiting for the TMA load)
-    int e = warp;
-    size_t nslot = 0;
-    int4 nkr = make_int4(0, 0, 0, 0);
-    float ncoef = 0.f;
-    auto fetch = [&](int ee) {
-      nslot = (size_t)tile * max_det + (use_list ? 0 : base) + S.list[ee];
-      nkr = krs[nslot];
-      ncoef = coef[nslot * kRegNm + lane];
-    };
-    if (e < nl) fetch(e);
-    if (!loaded) {
-      while (!mbar_try_wait(&S.bar, 0)) {
-      }
-      loaded = true;
-    }
-    for (; e < nl; e += kRegWarps) {
-      const size_t slot = nslot;
-      const int4 k = nkr;
-      __syncwarp();
-      S.coef[warp][lane] = ncoef;
-      __syncwarp();
-      if (e + kRegWarps < nl) fetch(e + kRegWarps);
-      float* dst = patches + slot * (kPatchPitch * kPatchPitch);
-      contract_piece<E>(S.proto, S.coef[warp], k, X0, Y0, lane,
-                        [&](int px, int py, float v) { dst[py * kPatchPitch + px] = v; });
-    }
+  for (int i = t; i < n; i += kRegThreads) S.list[i] = RL.det[i];
+  __syncthreads();
+  // software pipeline over this warp's pieces: the kept range and the coefficients of the NEXT piece are requested
+  // before the current one is computed (and those of the first piece before waiting for the TMA load)
+  int e = warp;
+  size_t nslot = 0;
+  int4 nkr = make_int4(0, 0, 0, 0);
+  float ncoef = 0.f;
+  auto fetch = [&](int ee) {
+    nslot = (size_t)tile * max_det + S.list[ee];
+    nkr = krs[nslot];
+    ncoef = coef[nslot * kRegNm + lane];
+  };
+  if (e < n) fetch(e);
+  while (!mbar_try_wait(&S.bar, 0)) {
   }
-  if (!loaded) {  // never leave with the bulk copy still in flight
-    while (!mbar_try_wait(&S.bar, 0)) {
-    }
+  for (; e < n; e += kRegWarps) {
+    const size_t slot = nslot;
+    const int4 k = nkr;
+    __syncwarp();
+    S.coef[warp][lane] = ncoef;
+    __syncwarp();
+    if (e + kRegWarps < n) fetch(e + kRegWarps);
+    // a detection listed here and handed over by another region of its range has an empty kept range now
+    if (k.z <= k.x || k.w <= k.y) continue;
+    float* dst = patches + slot * (kPatchPitch * kPatchPitch);
+    contract_piece<E>(S.proto, S.coef[warp], k, X0, Y0, lane,
+                      [&](int px, int py, float v) { dst[py * kPatchPitch + px] = v; });
   }
 }
 
@@ -310,29 +289,26 @@ struct UpSmem {
 
 template <bool PACKED, bool UPSAMPLE>
 __global__ void __launch_bounds__(kUpWarps * 32) mask_upsample_pack_kernel(
-    const float* __restrict__ patches, const float4* __restrict__ boxes, const int32_t* __restrict__ counts,
-    long long n_slots, int max_det, int mh, int mw, int ih, int iw, float rx, float ry, float* __restrict__ out_dense,
+    const float* __restrict__ patches, const int4* __restrict__ krs, const float4* __restrict__ boxes,
+    long long n_slots, int mh, int mw, int ih, int iw, float rx, float ry, float* __restrict__ out_dense,
     const int32_t* __restrict__ geom4, const int64_t* __restrict__ offsets, uint32_t* __restrict__ bits,
-    long long capacity_words,
-    int32_t* __restrict__ status, int32_t* __restrict__ large_count, int32_t* __restrict__ large_list) {
+    long long capacity_words, int32_t* __restrict__ status) {
   static_assert(!(PACKED && UPSAMPLE), "the packed + upsampled form runs mask_upsample_pack2_kernel");
   __shared__ UpSmem S;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const long long slot = (long long)blockIdx.x * kUpWarps + warp;
   if (slot >= n_slots) return;
-  const int tile = (int)(slot / max_det), d = (int)(slot - (long long)tile * max_det);
-  if (d >= counts[tile]) return;
+  const int4 kr = krs[slot];
+  if (kr.z <= kr.x || kr.w <= kr.y) return;  // dead / empty / handed to the per-detection body
+  // the window: computed (and trimmed) once by the geometry kernel for the bit-packed forms, here for the dense ones
   PMGeom g;
-  if (geom4) {
-    // the window was computed (and trimmed) once by the geometry kernel: only the kept proto range is redone here
-    const KeptRange k = kept_range(boxes[slot], rx, ry, mw, mh);
+  if (PACKED) {
     const int4 wdw = reinterpret_cast<const int4*>(geom4)[slot];
-    g.x1d = k.x1d, g.y1d = k.y1d, g.x2d = k.x2d, g.y2d = k.y2d;
-    g.px0 = k.px0, g.py0 = k.py0, g.px1 = k.px1, g.py1 = k.py1;
     g.x0 = wdw.x, g.y0 = wdw.y, g.w = wdw.z, g.h = wdw.w;
   } else {
     g = pm_geometry(boxes[slot], mh, mw, ih, iw, UPSAMPLE ? 1 : 0, rx, ry);
   }
+  g.px0 = kr.x, g.py0 = kr.y, g.px1 = kr.z, g.py1 = kr.w;
   if (g.w <= 0 || g.h <= 0) return;
   const int wpr = (g.w + 31) >> 5;
   const int oh = UPSAMPLE ? ih : mh, ow = UPSAMPLE ? iw : mw;
@@ -345,13 +321,6 @@ __global__ void __launch_bounds__(kUpWarps * 32) mask_upsample_pack_kernel(
     }
   }
   const int pw = g.px1 - g.px0, ph = g.py1 - g.py0;
-  if (pw > kPatchPitch || ph > kPatchPitch) {
-    // too large for the patch path: clear its words (the per-detection kernel ORs into them) and list it
-    if (PACKED)
-      for (long long i = lane; i < (long long)wpr * g.h; i += 32) bits[off + i] = 0u;
-    if (lane == 0) large_list[atomicAdd(large_count, 1)] = (int32_t)slot;
-    return;
-  }
   // ---- patch with its ring of zeros: element (y, x) of the proto plane sits at [(y - py0 + 1)][(x - px0 + 1)]
   float* P = S.patch[warp];
   {
@@ -454,10 +423,7 @@ __global__ void __launch_bounds__(kUpWarps * 32) mask_upsample_pack_kernel(
 }
 
 // ------------------------------------------------------------------------------------------------ packed + upsampled
-// The throughput form (bit planes of the upsampled masks) has kernels of its own:
-//   * the binning kernel records every slot's kept proto range (so nobody recomputes it from the box) and lists the
-//     detections that do not fit the patch path (kept range over 16 x 16 proto pixels, or an overfull region list):
-//     those ride in the region launch (ListedRide), their words cleared beforehand by pm_clear_listed_kernel;
+// The throughput form (bit planes of the upsampled masks) has a phase 2 of its own:
 //   * upsample_pack_v2: one warp per detection.  The sigmoid patch sits in shared memory with a ring of zeros (the
 //     crop).  x pass with lane = output column (two taps per source row), results stored TRANSPOSED; y pass with lane =
 //     output ROW: every lane walks the columns of its row, blends two of the stored values per pixel and sets the bit
@@ -605,57 +571,6 @@ __device__ __forceinline__ void upsample_pack_v2(const float* __restrict__ P, fl
   }
 }
 
-// binning for the packed + upsampled kernels (see above)
-__global__ void __launch_bounds__(256) proto_bin_fused_kernel(const float4* __restrict__ boxes,
-                                                              const int32_t* __restrict__ counts, long long n_slots,
-                                                              int max_det, int mh, int mw, int rxn, int ryn, float rx,
-                                                              float ry, const int32_t* __restrict__ geom4,
-                                                              RegionList* __restrict__ regions, int4* __restrict__ kr,
-                                                              int32_t* __restrict__ large_count,
-                                                              int32_t* __restrict__ large_list) {
-  const long long slot = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (slot >= n_slots) return;
-  const int tile = (int)(slot / max_det), d = (int)(slot - (long long)tile * max_det);
-  // empty window, not KEPT (slide form) or beyond counts: no patch, an empty kept range
-  const bool live = d < counts[tile] && geom4[4 * slot + 2] > 0 && geom4[4 * slot + 3] > 0;
-  KeptRange k;
-  k.px0 = k.py0 = k.px1 = k.py1 = 0;
-  if (live) k = kept_range(boxes[slot], rx, ry, mw, mh);
-  bool leave = false;
-  if (k.px1 > k.px0 && k.py1 > k.py0) {
-    leave = k.px1 - k.px0 > kPatchPitch || k.py1 - k.py0 > kPatchPitch;
-    if (!leave) {
-      const int rx0 = k.px0 / kRegBoxX, rx1 = (k.px1 - 1) / kRegBoxX;
-      const int ry0 = k.py0 / kRegBoxY, ry1 = (k.py1 - 1) / kRegBoxY;
-      for (int ryy = ry0; ryy <= ry1; ++ryy)
-        for (int rxx = rx0; rxx <= rx1; ++rxx) {
-          RegionList& R = regions[(size_t)tile * (rxn * ryn) + ryy * rxn + rxx];
-          const int pos = atomicAdd(&R.count, 1);
-          if (pos < kRegCap)
-            R.det[pos] = (uint16_t)d;
-          else
-            leave = true;  // overfull region: hand the detection over (its other pieces are skipped: empty range)
-        }
-    }
-    if (leave) large_list[atomicAdd(large_count, 1)] = (int32_t)slot;
-  }
-  kr[slot] = leave ? make_int4(0, 0, 0, 0) : make_int4(k.px0, k.py0, k.px1, k.py1);
-}
-
-// the words of the listed detections are cleared: the per-detection kernel ORs its bits in
-__global__ void pm_clear_listed_kernel(const int32_t* __restrict__ geom4, const int64_t* __restrict__ offsets,
-                                       uint32_t* __restrict__ bits, long long capacity_words,
-                                       const int32_t* __restrict__ list, const int32_t* __restrict__ list_count) {
-  const int n = *list_count;
-  for (int item = blockIdx.x; item < n; item += gridDim.x) {
-    const long long slot = list[item];
-    const int4 g = reinterpret_cast<const int4*>(geom4)[slot];
-    const long long words = (long long)((g.z + 31) >> 5) * g.w, off = offsets[slot];
-    if (off + words > capacity_words) continue;  // reported by the kernel that would have filled them
-    for (long long i = threadIdx.x; i < words; i += blockDim.x) bits[off + i] = 0u;
-  }
-}
-
 // phase 2 of the packed + upsampled form: one warp per detection, patch from the workspace.  Persistent: as many CTAs
 // as fit the GPU at once (6 per SM: 36 KB of shared memory and 256 x 40 registers each), every warp takes `chunk`
 // slots at a time from a ticket until none are left (chunk: about four tickets per warp, at most kV2Chunk -- one
@@ -710,6 +625,19 @@ static int upsample_pack2_grid() {
   return sms * per_sm;
 }
 
+template <typename E>
+static cudaError_t launch_patch(bool packed, unsigned grid, const CUtensorMap& map, const float* coef,
+                               const int32_t* counts, int max_det, int rxn, int ryn, const PmWorkspace& W,
+                               const ListedRide& LR, cudaStream_t stream) {
+  const auto kernel = packed ? proto_patch_kernel<E, true> : proto_patch_kernel<E, false>;
+  const cudaError_t e =
+      cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RegSmemT<E>));
+  if (e == cudaSuccess)
+    kernel<<<grid, kRegThreads, sizeof(RegSmemT<E>), stream>>>(map, coef, W.kr, counts, max_det, rxn, ryn, W.patches,
+                                                                W.regions, LR);
+  return e;
+}
+
 int launch_process_mask_regions(const void* protos, int proto_dtype, const float* coef, const float* boxes,
                                 const int32_t* counts,
                                 int bs, int max_det, int nm, int mh, int mw, int ih, int iw, int upsample, float rx,
@@ -722,10 +650,10 @@ int launch_process_mask_regions(const void* protos, int proto_dtype, const float
   const int esz = half ? 2 : 4;
   // TMA: the global address and every stride are multiples of 16 bytes; a tile origin too (24 pixels: 96 / 48 bytes)
   if (nm != kRegNm || (mw * esz & 15) != 0 || ((uintptr_t)protos & 15) != 0 || max_det > 65535) return 1;
-  // the packed + upsampled kernels read the windows hdy_process_mask_geometry wrote; without them the per-detection
-  // kernel recomputes the windows
+  // the bit-packed kernels read the windows and offsets hdy_process_mask_geometry wrote; without the windows the
+  // per-detection kernel recomputes them
   const bool packed = out_dense == nullptr;
-  if (packed && upsample && !geom) return 1;
+  if (packed && !geom) return 1;
   const int rxn = (mw + kRegBoxX - 1) / kRegBoxX, ryn = (mh + kRegBoxY - 1) / kRegBoxY;
   if ((long long)bs * rxn * ryn >= (1ll << 31) || slots >= (1ll << 31) || rxn * ryn > kMaxRegionsPerTile) return 1;
   EncodeTiledFn enc = tensor_map_encoder();
@@ -743,35 +671,30 @@ int launch_process_mask_regions(const void* protos, int proto_dtype, const float
   const PmWorkspace W = pm_workspace(workspace, slots);
   cudaError_t e = cudaMemsetAsync(W.large_count, 0, 8, stream);  // large_count and ticket
   if (e == cudaSuccess) e = cudaMemsetAsync(W.regions, 0, (size_t)bs * rxn * ryn * sizeof(RegionList), stream);
-  if (e == cudaSuccess)
-    e = half ? cudaFuncSetAttribute(proto_patch_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    (int)sizeof(RegSmemT<__half>))
-             : cudaFuncSetAttribute(proto_patch_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    (int)sizeof(RegSmemT<float>));
   if (e != cudaSuccess) {
     set_error("process_mask(regions) setup: %s", cudaGetErrorString(e));
     return HDY_ERR_CUDA;
   }
+  // binning, the listed detections' words cleared (bit-packed forms: their proto tiles OR into them; the dense output
+  // was zeroed by the caller), regions -> patches with the listed detections riding in the same launch, then phase 2
   const float4* b4 = reinterpret_cast<const float4*>(boxes);
-  if (packed && upsample) {
-    // bit-packed + upsampled (the throughput form): binning, the listed detections' words cleared (their tiles OR into
-    // them), regions -> patches with the listed detections riding in the same launch, then upsample_pack_v2
-    const float sxs = (float)mw / (float)iw, sys = (float)mh / (float)ih;  // ATen: scale = in / out (fp32)
-    proto_bin_fused_kernel<<<(unsigned)((slots + 255) / 256), 256, 0, stream>>>(
-        b4, counts, slots, max_det, mh, mw, rxn, ryn, rx, ry, geom, W.regions, W.kr, W.large_count, W.large_list);
+  proto_bin_fused_kernel<<<(unsigned)((slots + 255) / 256), 256, 0, stream>>>(
+      b4, counts, slots, max_det, mh, mw, rxn, ryn, rx, ry, geom, W.regions, W.kr, W.large_count, W.large_list);
+  if (packed)
     pm_clear_listed_kernel<<<148, 256, 0, stream>>>(geom, offsets, bits, capacity_words, W.large_list, W.large_count);
-    ListedRide LR;
-    LR.protos = protos, LR.boxes = b4, LR.offsets = offsets, LR.bits = bits, LR.status = status;
-    LR.list = W.large_list, LR.list_count = W.large_count, LR.capacity_words = capacity_words;
-    LR.rx = rx, LR.ry = ry, LR.nm = nm, LR.mh = mh, LR.mw = mw, LR.ih = ih, LR.iw = iw;
-    LR.ctas = kListedTiles * 9;
-    const unsigned g1 = (unsigned)((long long)bs * rxn * ryn + LR.ctas);
-    if (half)
-      proto_patch_kernel<__half><<<g1, kRegThreads, sizeof(RegSmemT<__half>), stream>>>(
-          map, coef, W.kr, counts, max_det, rxn, ryn, W.patches, W.regions, LR);
-    else
-      proto_patch_kernel<float><<<g1, kRegThreads, sizeof(RegSmemT<float>), stream>>>(
-          map, coef, W.kr, counts, max_det, rxn, ryn, W.patches, W.regions, LR);
+  ListedRide LR;
+  LR.protos = protos, LR.boxes = b4, LR.out_dense = out_dense, LR.offsets = offsets, LR.bits = bits;
+  LR.status = status, LR.list = W.large_list, LR.list_count = W.large_count, LR.capacity_words = capacity_words;
+  LR.rx = rx, LR.ry = ry, LR.nm = nm, LR.mh = mh, LR.mw = mw, LR.ih = ih, LR.iw = iw, LR.upsample = upsample;
+  const unsigned g1 = (unsigned)((long long)bs * rxn * ryn + kListedCtas);
+  e = half ? launch_patch<__half>(packed, g1, map, coef, counts, max_det, rxn, ryn, W, LR, stream)
+           : launch_patch<float>(packed, g1, map, coef, counts, max_det, rxn, ryn, W, LR, stream);
+  if (e != cudaSuccess) {
+    set_error("process_mask(regions) setup: %s", cudaGetErrorString(e));
+    return HDY_ERR_CUDA;
+  }
+  if (packed && upsample) {
+    const float sxs = (float)mw / (float)iw, sys = (float)mh / (float)ih;  // ATen: scale = in / out (fp32)
     const int g2 = upsample_pack2_grid();
     if (g2 <= 0) {
       set_error("process_mask(packed): no occupancy for mask_upsample_pack2_kernel");
@@ -783,34 +706,12 @@ int launch_process_mask_regions(const void* protos, int proto_dtype, const float
                                            status, W.ticket, chunk);
     return check_launch("hdy_process_mask(packed)");
   }
-  ListedRide no_ride;
-  memset(&no_ride, 0, sizeof(no_ride));
-  proto_bin_kernel<<<(unsigned)((slots + 255) / 256), 256, 0, stream>>>(b4, counts, slots, max_det, mh, mw, rxn, ryn, rx,
-                                                                        ry, geom, W.regions, W.kr);
-  if (half)
-    proto_patch_kernel<__half><<<(unsigned)((long long)bs * rxn * ryn), kRegThreads, sizeof(RegSmemT<__half>), stream>>>(
-        map, coef, W.kr, counts, max_det, rxn, ryn, W.patches, W.regions, no_ride);
-  else
-    proto_patch_kernel<float><<<(unsigned)((long long)bs * rxn * ryn), kRegThreads, sizeof(RegSmemT<float>), stream>>>(
-        map, coef, W.kr, counts, max_det, rxn, ryn, W.patches, W.regions, no_ride);
-  const unsigned g2 = (unsigned)((slots + kUpWarps - 1) / kUpWarps);
-#define HDY_UP(P, U)                                                                                              \
-  mask_upsample_pack_kernel<P, U><<<g2, kUpWarps * 32, 0, stream>>>(W.patches, b4, counts, slots, max_det, mh, mw, \
-                                                                    ih, iw, rx, ry, out_dense, geom, offsets, bits, \
-                                                                    capacity_words, status, W.large_count,         \
-                                                                    W.large_list)
-  if (packed)
-    HDY_UP(true, false);
-  else if (upsample)
-    HDY_UP(false, true);
-  else
-    HDY_UP(false, false);
-#undef HDY_UP
-  int rc = check_launch("hdy_process_mask(regions)");
-  if (rc) return rc;
-  return launch_process_mask_listed(protos, proto_dtype, coef, boxes, counts, max_det, nm, mh, mw, ih, iw, upsample, rx, ry,
-                                    out_dense, offsets, bits, capacity_words, status, W.large_list, W.large_count,
-                                    stream);
+  const auto up = packed     ? mask_upsample_pack_kernel<true, false>
+                  : upsample ? mask_upsample_pack_kernel<false, true>
+                             : mask_upsample_pack_kernel<false, false>;
+  up<<<(unsigned)((slots + kUpWarps - 1) / kUpWarps), kUpWarps * 32, 0, stream>>>(
+      W.patches, W.kr, b4, slots, mh, mw, ih, iw, rx, ry, out_dense, geom, offsets, bits, capacity_words, status);
+  return check_launch("hdy_process_mask(regions)");
 }
 
 }  // namespace hdy

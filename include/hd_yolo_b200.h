@@ -234,7 +234,8 @@ HDY_API int hdy_process_mask(const void* protos, int proto_dtype, const float* c
                              const int32_t* counts, int bs, int max_det, int nm, int mh, int mw, int ih, int iw,
                              int upsample, float* out, void* workspace, size_t workspace_bytes, hdy_stream_t stream);
 /* Cropped bit-packed variant; geom [bs*max_det, 4], offsets [bs*max_det + 1] as above (slots >= counts are empty).
- * hdy_process_mask_packed takes the geom array hdy_process_mask_geometry wrote (NULL: windows are recomputed).
+ * hdy_process_mask_packed takes the geom array hdy_process_mask_geometry wrote; the two-phase path needs it (NULL:
+ * the per-detection kernel runs and recomputes the windows).
  * Slide form (row_state / tile_offsets non-NULL): slot d of tile t is row tile_offsets[t] + d of the slide-level
  * arrays (hdy_merge_append); only rows whose verdict row_state[row] is HDY_STATE_KEPT get a window -- Ensemble.merge
  * returns masks[keep] (yolo.py:197-202), so the masks of suppressed duplicates are never computed. */

@@ -196,8 +196,9 @@ def test_process_mask_other_prototype_counts(cuda_device):
 
 
 def test_process_mask_crowded_region_and_empty_regions(cuda_device):
-    """More than 254 detections in one 24x24 proto region (the region's list overflows and the CTA falls back to
-    scanning the tile) while most regions of the plane are touched by nobody (they load nothing)."""
+    """More than 254 detections in one 24x24 proto region (the region's list fills up and the binning hands the rest
+    to the per-detection body, some of them already listed in another region) while most regions of the plane are
+    touched by nobody (they load nothing)."""
     g = torch.Generator().manual_seed(21)
     n, mh, mw, ih, iw = 600, 128, 128, 512, 512
     protos = torch.randn((32, mh, mw), generator=g)
@@ -325,17 +326,19 @@ def test_process_mask_full_size_config2(cuda_device):
     assert int(offs[-1]) <= bits.numel() and int(offs[-1]) > 30 * 2000
 
 
+@pytest.mark.parametrize("form", ["packed_upsampled", "packed", "dense_upsampled", "dense"])
 @pytest.mark.parametrize("mh,mw,ih,iw,md,lo,hi,half", [(160, 160, 640, 640, 900, 12, 36, False),
                                                        (256, 256, 1024, 1024, 2650, 12, 36, False),
                                                        (64, 80, 250, 333, 300, 4, 120, False),
                                                        (128, 128, 512, 512, 700, 10, 70, True)])
-def test_packed_mask_kernel_paths_agree_bit_for_bit(cuda_device, mh, mw, ih, iw, md, lo, hi, half):
-    """The bit-packed, upsampled form runs regions -> patches + upsample_pack_v2, with the detections the patch path
-    leaves out riding in the region launch.  The per-detection kernel, reached by hdy_process_mask_packed without a
-    workspace (a) or without the windows (b, it recomputes them), must give the same bits on the same geometry and
-    offsets -- including boxes too large for the patch path, crowded regions whose lists overflow, empty tiles and
-    non-integer scales."""
+def test_packed_mask_kernel_paths_agree_bit_for_bit(cuda_device, mh, mw, ih, iw, md, lo, hi, half, form):
+    """Every form runs regions -> patches -> upsample / pack, with the detections the patch path leaves out riding in
+    the region launch.  The per-detection kernel must give the same output: for the bit-packed forms reached by
+    hdy_process_mask_packed without a workspace (a) or without the windows (b), on the same geometry and offsets; for
+    the dense forms by hdy_process_mask without a workspace -- including boxes too large for the patch path, crowded
+    regions whose lists overflow, empty tiles and non-integer scales."""
     from hd_yolo_b200 import _lib, ops
+    upsample = form.endswith("upsampled")
     g = torch.Generator().manual_seed(mh + md)
     bs = 3
     protos = torch.randn((bs, 32, mh, mw), generator=g)
@@ -348,24 +351,37 @@ def test_packed_mask_kernel_paths_agree_bit_for_bit(cuda_device, mh, mw, ih, iw,
     boxes[0, 3] = torch.tensor([5.0, 7.0, iw - 20.0, ih * 0.6])                       # huge: per-detection kernel
     counts = torch.tensor([md, md - 7, 0], dtype=torch.int32)
     protos, coef, boxes, counts = (t.to(cuda_device) for t in (protos, coef, boxes, counts))
-    pk = hm.process_mask_packed(protos, coef, boxes, counts, (ih, iw), upsample=True)
-    pk.check()
-    words = int(pk.offsets[-1])
     lib = _lib.load()
     ws_bytes = lib.hdy_process_mask_workspace_bytes(bs, md)
     ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=cuda_device)
     dtype = _lib.HDY_F16 if half else _lib.HDY_F32
+    if form.startswith("dense"):
+        oh, ow = (ih, iw) if upsample else (mh, mw)
+        outs = []
+        for workspace, nbytes in ((ws, ws_bytes), (None, 0)):
+            out = torch.full((bs, md, oh, ow), -1.0, dtype=torch.float32, device=cuda_device)
+            _lib.check(lib.hdy_process_mask(_lib.ptr(protos), dtype, _lib.ptr(coef), _lib.ptr(boxes), _lib.ptr(counts),
+                                            bs, md, 32, mh, mw, ih, iw, int(upsample), _lib.ptr(out),
+                                            _lib.ptr(workspace), nbytes, ops._stream()))
+            outs.append(out)
+        a, b = outs
+        assert torch.equal(a, b), f"dense outputs differ in {int((a != b).sum())} pixels"
+        assert float(a[0].sum()) > (50 if upsample else 3) * md
+        return
+    pk = hm.process_mask_packed(protos, coef, boxes, counts, (ih, iw), upsample=upsample)
+    pk.check()
+    words = int(pk.offsets[-1])
     for what, geom, workspace, nbytes in (("no workspace", pk.geom, None, 0), ("no geom", None, ws, ws_bytes)):
         bits = torch.full((max(words, 1),), -1, dtype=torch.int32, device=cuda_device)
         status = torch.zeros((1,), dtype=torch.int32, device=cuda_device)
         _lib.check(lib.hdy_process_mask_packed(_lib.ptr(protos), dtype, _lib.ptr(coef), _lib.ptr(boxes),
                                                _lib.ptr(counts), _lib.ptr(geom), _lib.ptr(pk.offsets), bs, md, 32, mh,
-                                               mw, ih, iw, 1, _lib.ptr(bits), words, _lib.ptr(status),
+                                               mw, ih, iw, int(upsample), _lib.ptr(bits), words, _lib.ptr(status),
                                                _lib.ptr(workspace), nbytes, ops._stream()))
         assert int(status.item()) == 0, f"{what}: status {int(status.item())}"
         d = bits[:words]
         assert torch.equal(pk.bits, d), f"{what}: bits differ ({int((pk.bits != d).sum())} of {words} words)"
-    assert words > 20 * (md - 7)
+    assert words > (20 if upsample else 2) * (md - 7)
 
 
 def test_mask_agreement_is_tight_inside_the_windows(cuda_device):
