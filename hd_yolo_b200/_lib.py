@@ -123,6 +123,15 @@ SIGNATURES = {
     "hdy_mask_areas": (_i, [_vp, _vp, _vp, _i, _vp, _vp]),
     "hdy_match_mask_pairs": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _f, _i, _vp, _i, _vp, _vp, _vp,
                                   _vp]),
+    "hdy_match_bin_stats": (_i, [_vp, _vp, _i, _vp, _vp]),
+    "hdy_match_bin_entries": (_i, [_vp, _vp, _i, _f, _f, _f, _i, _i, _vp, _vp, _vp]),
+    "hdy_match_bin_cells": (_i, [_vp, _i64, _i64, _vp, _vp]),
+    "hdy_match_boxes_binned": (_i, [_vp, _vp, _i, _vp, _i, _f, _f, _f, _i, _i, _vp, _vp, _f, _vp, _vp, _vp, _vp, _vp]),
+    "hdy_match_mask_candidates_binned": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _i, _f, _f, _f, _i, _i, _vp, _vp, _f, _vp,
+                                              _vp, _vp, _vp]),
+    "hdy_match_mask_exact_list": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _f, _vp, _vp, _vp,
+                                       _vp, _vp, _vp, _vp]),
+    "hdy_match_order_keys": (_i, [_vp, _i64, _vp, _vp]),
 }
 
 _lock = threading.Lock()

@@ -12,16 +12,9 @@
 //   * box_iou_kernel: the dense matrix itself, for callers that want it (box_iou is also used on its own).
 // IoU arithmetic is the reference's: inter = clamp(min(a2,b2) - max(a1,b1), 0).prod(); iou = inter / (area1 + area2 -
 // inter), fp32, one rounding per operation; 0/0 = NaN fails `>=` exactly as in the reference.
-#include "hdy_common.cuh"
+#include "match_common.cuh"
 
 namespace hdy {
-
-__device__ __forceinline__ float ref_box_iou(const float4& a, float area_a, const float4& b, float area_b) {
-  const float w = fmaxf(__fsub_rn(fminf(a.z, b.z), fmaxf(a.x, b.x)), 0.0f);
-  const float h = fmaxf(__fsub_rn(fminf(a.w, b.w), fmaxf(a.y, b.y)), 0.0f);
-  const float inter = __fmul_rn(w, h);
-  return __fdiv_rn(inter, __fsub_rn(__fadd_rn(area_a, area_b), inter));
-}
 
 constexpr int kMatchThreads = 256;
 

@@ -14,6 +14,7 @@
 //     with iou >= iou_min as order keys ~orderable(iou) << 32 | (rank * g + j), the box path's keys (match.cu).
 // A pixel is set iff its value is > 0.5 (fp32 / fp16) or nonzero (uint8 / bool).  iou = float(inter) / float(union),
 // both conversions and the division rounded to nearest: what `inter.float() / union.float()` gives in torch.
+#include "match_common.cuh"
 #include "scan_common.cuh"
 
 namespace hdy {
@@ -193,21 +194,11 @@ __global__ void __launch_bounds__(kAreaThreads) areas_kernel(const int32_t* __re
 }
 
 // ---------------------------------------------------------------------------------------------- matching
-// iou = float(inter) / float(union), each step rounded to nearest (torch: inter.float() / union.float())
-__device__ __forceinline__ float mask_iou(int inter, int area_a, int area_b) {
-  const long long uni = (long long)area_a + area_b - inter;
-  return __fdiv_rn(__int2float_rn(inter), __ll2float_rn(uni));
-}
-
 constexpr int kCandThreads = 256;
 
 // One thread per prediction (rank r in score order), the ground-truth windows and areas staged through shared memory
-// in chunks (as match_pairs_kernel does with boxes).  A pair is a candidate when its windows overlap and
-//   mask_iou(min(overlap area, area_p, area_g), area_p, area_g) >= iou_min.
-// The intersection can be at most that bound, the IoU inter / (area_p + area_g - inter) increases with inter, and the
-// round-to-nearest conversions and division are monotone, so the fp32 IoU of every pair is <= the fp32 bound: no pair
-// whose exact IoU reaches iou_min is ever dropped here.  Pairs that do not overlap have inter = 0, iou 0 or NaN, and
-// never match since iou_min > 0.
+// in chunks (as match_pairs_kernel does with boxes).  A pair is a candidate when its windows overlap and its IoU upper
+// bound reaches iou_min (window_pair_may_match, match_common.cuh): no pair whose exact IoU reaches iou_min is dropped.
 __global__ void __launch_bounds__(kCandThreads) candidates_kernel(
     const int32_t* __restrict__ pred_geom, const int32_t* __restrict__ pred_areas,
     const int32_t* __restrict__ pred_order, int P, const int32_t* __restrict__ gt_geom,
@@ -235,13 +226,7 @@ __global__ void __launch_bounds__(kCandThreads) candidates_kernel(
     if (!live) continue;
     const int lim = min(kCandThreads, G - j0);
     for (int j = 0; j < lim; ++j) {
-      const int4 b = gw[j];
-      const int ow = min(a.x + a.z, b.x + b.z) - max(a.x, b.x);
-      const int oh = min(a.y + a.w, b.y + b.w) - max(a.y, b.y);
-      if (ow <= 0 || oh <= 0) continue;
-      const int area_b = ga[j];
-      const int inter_max = (int)min((long long)ow * oh, (long long)min(area_a, area_b));
-      if (mask_iou(inter_max, area_a, area_b) >= iou_min) {
+      if (window_pair_may_match(a, area_a, gw[j], ga[j], iou_min)) {
         const int pos = atomicAdd(&counts[1], 1);
         if (pos < cand_cap)
           cand[pos] = (uint32_t)r * (uint32_t)G + (uint32_t)(j0 + j);
@@ -252,22 +237,11 @@ __global__ void __launch_bounds__(kCandThreads) candidates_kernel(
   }
 }
 
-// 32 bits of a row of a bit plane starting at bit `dx` (>= 0) of the row; the word after the one holding `dx` is only
-// read when the shift needs it and it belongs to the row.
-__device__ __forceinline__ uint32_t row_bits(const uint32_t* __restrict__ row, int wpr, int dx) {
-  const int k = dx >> 5, s = dx & 31;
-  const uint32_t lo = __ldg(row + k);
-  const uint32_t hi = (s && k + 1 < wpr) ? __ldg(row + k + 1) : 0u;
-  return __funnelshift_r(lo, hi, s);
-}
-
 constexpr int kExactThreads = 256;
 constexpr int kExactMaxBlocks = 4096;
 
-// One warp per candidate (grid-stride over the candidates found, up to cand_cap).  The lanes split the overlap
-// rectangle into (row, 32-pixel chunk) items; both planes are aligned to the chunk's first pixel with a funnel shift,
-// the chunk's pixels beyond the overlap are masked off (so padding bits never count), and popc(a & b) is summed over
-// the warp.  Pairs with iou >= iou_min are appended as make_key(iou, rank * G + j).
+// One warp per candidate (grid-stride over the candidates found, up to cand_cap) counts the intersection
+// (warp_window_intersection, match_common.cuh).  Pairs with iou >= iou_min are appended as make_key(iou, rank * G + j).
 __global__ void __launch_bounds__(kExactThreads) exact_kernel(
     const int32_t* __restrict__ pred_geom, const int64_t* __restrict__ pred_offsets,
     const uint32_t* __restrict__ pred_bits, const int32_t* __restrict__ pred_areas,
@@ -284,24 +258,7 @@ __global__ void __launch_bounds__(kExactThreads) exact_kernel(
     const int row = pred_order ? pred_order[r] : r;
     const int4 a = reinterpret_cast<const int4*>(pred_geom)[row];
     const int4 b = reinterpret_cast<const int4*>(gt_geom)[j];
-    const int ox0 = max(a.x, b.x), ox1 = min(a.x + a.z, b.x + b.z);
-    const int oy0 = max(a.y, b.y), oy1 = min(a.y + a.w, b.y + b.w);
-    const int wa = (a.z + 31) >> 5, wb = (b.z + 31) >> 5;
-    const uint32_t* pa = pred_bits + pred_offsets[row] + (long long)(oy0 - a.y) * wa;
-    const uint32_t* pb = gt_bits + gt_offsets[j] + (long long)(oy0 - b.y) * wb;
-    const int nch = (ox1 - ox0 + 31) >> 5;
-    const int items = (oy1 - oy0) * nch;
-    int inter = 0;
-    for (int t = lane; t < items; t += 32) {
-      const int y = t / nch, ch = t - y * nch;
-      const int x = ox0 + (ch << 5);
-      const int nv = min(32, ox1 - x);
-      const uint32_t m = nv == 32 ? 0xffffffffu : (1u << nv) - 1u;
-      const uint32_t va = row_bits(pa + (long long)y * wa, wa, x - a.x);
-      const uint32_t vb = row_bits(pb + (long long)y * wb, wb, x - b.x);
-      inter += __popc(va & vb & m);
-    }
-    inter = __reduce_add_sync(0xffffffffu, inter);
+    const int inter = warp_window_intersection(a, pred_bits + pred_offsets[row], b, gt_bits + gt_offsets[j], lane);
     if (lane == 0) {
       const float iou = mask_iou(inter, pred_areas[row], gt_areas[j]);
       if (iou >= iou_min) {

@@ -107,6 +107,46 @@ class PackedMasks:
                   ptr(self._bits_nonempty()), K, ptr(out), _stream())
         return out
 
+    def select(self, rows) -> "PackedMasks":
+        """The masks of `rows` (index tensor or sequence), in that order, sharing `bits`: geom[rows] and offsets[rows]
+        address them, offsets[-1] stays the total word count.  Turns a slide result into matcher input:
+        ``res['masks'].select(res['index'] - res['base'])``."""
+        rows = torch.as_tensor(rows, dtype=torch.int64, device=self.geom.device)
+        if rows.dim() != 1:
+            raise HdyError(f"rows must be one-dimensional, got {tuple(rows.shape)}")
+        return PackedMasks(self.geom[rows].contiguous(), torch.cat([self.offsets[rows], self.offsets[-1:]]), self.bits,
+                           self.H, self.W, self.status)
+
+    @classmethod
+    def cat(cls, parts, origins, canvas) -> "PackedMasks":
+        """Masks of several canvases placed on one: part i's canvas (its H x W) goes to (x, y) = origins[i] of the
+        (H, W) `canvas` and must lie inside it -- e.g. the ground truth of several annotated regions of a slide on the
+        slide canvas.  Rows in part order; windows move by the origin (empty windows stay empty), offsets by the words
+        of the parts before; `bits` is the parts' planes one after another.  The status word is the OR of the parts'."""
+        parts, origins = list(parts), [tuple(int(v) for v in o) for o in origins]
+        if not parts or len(parts) != len(origins):
+            raise HdyError(f"cat takes one origin per part ({len(parts)} parts, {len(origins)} origins)")
+        H, W = _hw(canvas)
+        for p, (x, y) in zip(parts, origins):
+            if x < 0 or y < 0 or x + p.W > W or y + p.H > H:
+                raise HdyError(f"a {p.H} x {p.W} canvas at (x, y) = ({x}, {y}) does not fit the {H} x {W} canvas")
+        geoms, offs, bits, base = [], [], [], 0
+        for p, (x, y) in zip(parts, origins):
+            g = p.geom.clone()
+            live = (g[:, 2] > 0) & (g[:, 3] > 0)
+            g[:, 0] += torch.where(live, x, 0).to(g.dtype)
+            g[:, 1] += torch.where(live, y, 0).to(g.dtype)
+            geoms.append(g)
+            offs.append(p.offsets[:-1] + base)
+            bits.append(p.bits)
+            base += int(p.bits.numel())
+        dev = parts[0].geom.device
+        status = parts[0].status.clone()
+        for p in parts[1:]:
+            status |= p.status
+        offsets = torch.cat(offs + [torch.tensor([base], dtype=torch.int64, device=dev)])
+        return cls(torch.cat(geoms).contiguous(), offsets, torch.cat(bits), H, W, status)
+
     def _bits_nonempty(self) -> torch.Tensor:
         """`bits`, or one zero word when no mask has any (an empty tensor has no device address)."""
         return self.bits if self.bits.numel() else torch.zeros((1,), dtype=torch.int32, device=self.bits.device)

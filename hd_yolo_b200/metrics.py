@@ -1,7 +1,8 @@
 """Prediction <-> ground-truth matching on the device (SURVEY 8f rank 2): host mirror of ``box_iou``
 (metayolo/models/utils_general.py:247-265) and of the matching half of ``APMeter.add``
 (metayolo/models/metrics.py:270-303), over ``hdy_box_iou`` / ``hdy_match_pairs``, and by mask IoU over
-``hdy_match_mask_pairs`` (bit-packed masks, ``PackedMasks``).
+``hdy_match_mask_pairs`` (bit-packed masks, ``PackedMasks``); at region and slide scale over the binned matchers of
+csrc/match_binned.cu (``binned=True``).
 
 The reference moves every image's detections to the host and builds a dense k x g IoU matrix there; here the
 matching pairs are produced on the device and only they (a few hundred rows per image) are copied back.
@@ -10,6 +11,7 @@ plotting code runs on it unchanged.
 """
 from __future__ import annotations
 
+import math
 from typing import Dict, Optional
 
 import numpy as np
@@ -37,7 +39,7 @@ def box_iou(box1: torch.Tensor, box2: torch.Tensor) -> torch.Tensor:
 
 
 def match_predictions(output: Dict[str, torch.Tensor], target: Dict[str, torch.Tensor], iou_min: float = 0.5,
-                      cap: Optional[int] = None, iou_type: str = 'boxes') -> Dict[str, torch.Tensor]:
+                      cap: Optional[int] = None, iou_type: str = 'boxes', binned: bool = False) -> Dict[str, torch.Tensor]:
     """The device half of APMeter.add (metrics.py:271-284), by box IoU or, with iou_type='masks', by mask IoU.
 
     Returns (all on the device): 'order' (rows of `output` by score, descending, ties by lower row), 'scores' /
@@ -49,9 +51,20 @@ def match_predictions(output: Dict[str, torch.Tensor], target: Dict[str, torch.T
     the fly by PackedMasks.from_dense: fp32 / fp16 set iff > 0.5, uint8 / bool iff nonzero) or a PackedMasks, with as
     many rows as the boxes, on one (H, W) canvas.  inter / union are exact pixel counts, iou = float(inter) /
     float(union); iou_min must be > 0.  Every (prediction, ground truth) pair of windows is tested once (O(k * g), as
-    the box path): sized for an image, not for region- or slide-scale ground truth (1e5+ nuclei per call)."""
+    the box path): sized for an image, not for region- or slide-scale ground truth (1e5+ nuclei per call).
+
+    binned=True: the same result, bit for bit, for region- and slide-scale inputs (k, g < 2^31, fewer than 2^31
+    matching pairs, k * g unrestricted).  The ground truth is put into a uniform grid over its extent and a prediction
+    is tested only against the ground truth listed in the cells its box (or mask window) covers; `cap` is not used.
+    Needs iou_min > 0 for boxes too (the grid only finds pairs that overlap).  Small D2H reads: three for boxes (grid
+    statistics, entry count, pair count), four for masks (+ the matched count), plus what the mask inputs take as
+    everywhere (PackedMasks.check's status read per PackedMasks side, from_dense's word count per dense side).  One
+    rank's rows only: a ground-truth nucleus on a seam
+    between ranks can match predictions of both, so gather a multi-rank slide result to one rank before matching."""
     if iou_type not in ('boxes', 'masks'):
         raise HdyError(f"iou_type must be 'boxes' or 'masks', got {iou_type!r}")
+    if binned and not np.float32(iou_min) > 0:
+        raise HdyError(f"binned matching needs iou_min > 0 (the grid only finds pairs that overlap), got {iou_min}")
     boxes, scores, gts = output['boxes'], output['scores'], target['boxes']
     _need_cuda(boxes, "output['boxes']")
     _need_cuda(scores, "output['scores']")
@@ -76,6 +89,10 @@ def match_predictions(output: Dict[str, torch.Tensor], target: Dict[str, torch.T
     res = {'order': order, 'scores': scores[order], 'labels': output['labels'][order]}
     if g == 0:
         return {**res, **empty}
+    if binned:
+        if max(k, g) >= 2 ** 31:
+            raise HdyError(f"binned matching takes fewer than 2^31 predictions and ground truth (got {k}, {g})")
+        return {**res, **_binned_match(output, target, iou_type, order32, k, g, iou_min, empty)}
     # 2. pairs with iou >= iou_min, as order keys (~orderable(iou) << 32 | rank * g + j)
     if iou_type == 'masks':
         launch = _mask_pairs(_packed(output['masks']), _packed(target['masks']), order32, k, g, iou_min)
@@ -134,6 +151,100 @@ def _mask_pairs(pm: PackedMasks, gm: PackedMasks, order32, k, g, iou_min):
               ptr(counts), ptr(counts[2:]), _stream(), launches=2)
         return pk, counts[:2]
     return launch
+
+
+def _f32_of_orderable(o: int) -> float:
+    o &= 0xffffffff
+    u = (o & 0x7fffffff) if o & 0x80000000 else (~o & 0xffffffff)
+    return float(np.array(u, dtype=np.uint32).view(np.float32))
+
+
+def _pick_grid(stats):
+    """(ox, oy, inv_cell, nx, ny) from hdy_match_bin_stats: cells about one mean ground-truth side across (a nucleus
+    covers a few cells), at most 2 * n + 1024 of them (n valid ground truth), larger cells where the extent needs it.
+    Any grid gives the same pairs (the cell function clamps: a short last row or column of cells only holds more);
+    this one keeps the lists short.  The extent of finite fp32 coordinates is below 2^129, so the cell is below
+    2^129 / sqrt(1024) and 1 / cell stays a normal fp32."""
+    n = stats[4]
+    x0, y0, x1, y1 = (_f32_of_orderable(v) for v in stats[:4])
+    w, h = max(x1 - x0, 0.0), max(y1 - y0, 0.0)
+    max_cells = min(2 * n + 1024, 1 << 26)
+    cell = max(stats[5] / 16.0 / n, 1.0, math.sqrt(w * h / max_cells))
+    inv = float(np.float32(1.0 / cell))
+    nx = min(int(w * inv) + 1, max_cells)
+    ny = min(int(h * inv) + 1, max(max_cells // nx, 1))
+    return float(np.float32(x0)), float(np.float32(y0)), inv, nx, ny
+
+
+def _binned_match(output, target, iou_type, order32, k, g, iou_min, empty):
+    """'pred_idx', 'true_idx', 'ious' of match_predictions(binned=True) over csrc/match_binned.cu."""
+    dev = order32.device
+    i64 = dict(dtype=torch.int64, device=dev)
+    i32 = dict(dtype=torch.int32, device=dev)
+    thr = float(np.float32(iou_min))
+    if iou_type == 'masks':
+        pm, gm = _packed(output['masks']), _packed(target['masks'])
+        pred = _aligned16(pm.geom.contiguous())
+        gb, gg = None, _aligned16(gm.geom.contiguous())
+    else:
+        pred = _aligned16(output['boxes'].contiguous())
+        gb, gg = _aligned16(target['boxes'].contiguous()), None
+    # 1. the grid (one read: its statistics), the ground truth's cell entries (one read: their number), sorted by cell
+    stats = torch.empty(6, **i64)
+    _call("hdy_match_bin_stats", ptr(gb), ptr(gg), g, ptr(stats), _stream(), launches=2)
+    stats = stats.tolist()
+    if stats[4] == 0:
+        return empty                                  # no ground truth can overlap anything
+    grid = _pick_grid(stats)
+    n_cells = grid[3] * grid[4]
+    ent_off = torch.empty(g + 1, **i64)
+    _call("hdy_match_bin_entries", ptr(gb), ptr(gg), g, *grid, ptr(ent_off), None, _stream(), launches=3)
+    n_ent = int(ent_off[g].item())
+    cell_keys = torch.empty(n_ent, **i64)
+    _call("hdy_match_bin_entries", ptr(gb), ptr(gg), g, *grid, ptr(ent_off), ptr(cell_keys), _stream())
+    from .slide import sort_keys
+    sort_keys(cell_keys, first_byte=4, n_bytes=2 if n_cells <= 1 << 16 else 4)
+    cell_start = torch.empty(n_cells + 1, **i64)
+    _call("hdy_match_bin_cells", ptr(cell_keys), n_ent, n_cells, ptr(cell_start), _stream())
+    # 2. the pairs (boxes) or candidates (masks) of every prediction rank, in (rank, j) order (one read: their number)
+    off = torch.empty(k + 1, **i64)
+    if iou_type == 'masks':
+        ap, ag = pm.areas(), gm.areas()
+        fn, head = "hdy_match_mask_candidates_binned", (ptr(pred), ptr(ap), ptr(order32), k, ptr(gg), ptr(ag), g)
+    else:
+        fn, head = "hdy_match_boxes_binned", (ptr(pred), ptr(order32), k, ptr(gb), g)
+    tail = (ptr(cell_start), ptr(cell_keys), thr, ptr(off))
+    _call(fn, *head, *grid, *tail, *((None,) * (2 if iou_type == 'masks' else 3)), _stream(), launches=4)
+    n = int(off[k].item())
+    if n >= 2 ** 31:
+        raise HdyError(f"{n} {'candidate pairs' if iou_type == 'masks' else 'matching pairs'}: binned matching "
+                       "takes fewer than 2^31")
+    if n == 0:
+        return empty
+    rank, j = torch.empty(n, **i32), torch.empty(n, **i32)
+    iou = torch.empty(n, dtype=torch.float32, device=dev)
+    if iou_type == 'masks':
+        _call(fn, *head, *grid, *tail, ptr(rank), ptr(j), _stream())
+        # 3. exact intersections of the candidates, the matching ones compacted in order (one read: their number)
+        cand_iou = torch.empty(n, dtype=torch.float32, device=dev)
+        pr, pj = torch.empty(n, **i32), torch.empty(n, **i32)
+        count = torch.zeros(1, **i32)
+        blk = torch.empty(4096, **i32)
+        _call("hdy_match_mask_exact_list", ptr(pred), ptr(pm.offsets), ptr(pm._bits_nonempty()), ptr(ap),
+              ptr(order32), ptr(gg), ptr(gm.offsets), ptr(gm._bits_nonempty()), ptr(ag), ptr(rank), ptr(j), n, thr,
+              ptr(cand_iou), ptr(pr), ptr(pj), ptr(iou), ptr(count), ptr(blk), _stream(), launches=4)
+        rank, j = pr, pj
+        n = int(count.item())
+        if n == 0:
+            return empty
+    else:
+        _call(fn, *head, *grid, *tail, ptr(rank), ptr(j), ptr(iou), _stream())
+    # 4. IoU-descending order, ties in (rank, j) order: a stable sort of the IoU half of (~orderable(iou), position)
+    keys = torch.empty(n, **i64)
+    _call("hdy_match_order_keys", ptr(iou), n, ptr(keys), _stream())
+    sort_keys(keys, first_byte=4, n_bytes=4)
+    pos = keys & 0xffffffff
+    return {'pred_idx': rank[pos].to(torch.int64), 'true_idx': j[pos].to(torch.int64), 'ious': _key_scores(keys)}
 
 
 def _mask_canvas(m, n: int, name: str):
@@ -195,10 +306,12 @@ class APMeter(object):
         self.m_pred = torch.empty(0, dtype=torch.int64)
         self.m_true = torch.empty(0, dtype=torch.int64)
 
-    def add(self, output, target, iou_type='boxes'):
+    def add(self, output, target, iou_type='boxes', binned=False):
+        """binned=True: match_predictions(..., binned=True), for region- or slide-scale inputs (same fields)."""
         # the reference's rule: mask IoU when asked for and both sides carry masks, box IoU otherwise
         use_masks = iou_type == 'masks' and ('masks' in output and 'masks' in target)
-        m = match_predictions(output, target, float(self.iouv.min()), iou_type='masks' if use_masks else 'boxes')
+        m = match_predictions(output, target, float(self.iouv.min()), iou_type='masks' if use_masks else 'boxes',
+                              binned=binned)
         n_pred, n_true = int(output['boxes'].shape[0]), int(target['boxes'].shape[0])
         self.m_pred = torch.cat([self.m_pred, (m['pred_idx'] + self.n_pred).cpu()])
         self.m_true = torch.cat([self.m_true, (m['true_idx'] + self.n_true).cpu()])

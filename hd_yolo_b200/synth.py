@@ -51,6 +51,23 @@ def _tile_seed(seed: int, tile_index: int) -> int:
     return (int(seed) * 1000003 + int(tile_index) * 7919 + 12345) & 0x7fffffffffff
 
 
+def _field_uniform(h: torch.Tensor, k: int) -> torch.Tensor:
+    """Uniform k in [0, 1) of the global nuclei field at grid hash h: a pure function of (h, k)."""
+    v = (h * (2 * k + 1) + 0x9E3779B9 * (k + 1)) & 0x7fffffff
+    v = (v * 1103515245 + 12345) & 0x7fffffff
+    return (v >> 7).to(torch.float32) / float(1 << 24)
+
+
+def _field_nuclei(I: torch.Tensor, J: torch.Tensor, pitch: float, size_range):
+    """Centre, box side and score of the field's nucleus at grid index (I, J) (int64 tensors)."""
+    h = (I * 73856093) ^ (J * 19349663)
+    cx = (I.float() + 0.15 + 0.7 * _field_uniform(h, 0)) * pitch
+    cy = (J.float() + 0.15 + 0.7 * _field_uniform(h, 1)) * pitch
+    side = size_range[0] + (size_range[1] - size_range[0]) * _field_uniform(h, 2)
+    score = 0.3 + 0.65 * _field_uniform(h, 3)
+    return cx, cy, side, score
+
+
 def slide_tile_logits(rois: torch.Tensor, tile: int, nc: int, seed: int, pitch: float = 18.7, extra: int = 0,
                       conf: float = 0.25, size_range=(12.0, 30.0), strides=STRIDES_3, anchors=ANCHORS_3,
                       device="cuda", background_mu: float = -6.0, first_tile: int = 0, dtype=torch.float32):
@@ -91,17 +108,7 @@ def slide_tile_logits(rois: torch.Tensor, tile: int, nc: int, seed: int, pitch: 
         ii = torch.arange(i0, i0 + ncell, device=dev, dtype=torch.int64)
         jj = torch.arange(j0, j0 + ncell, device=dev, dtype=torch.int64)
         J, I = torch.meshgrid(jj, ii, indexing='ij')
-        # hash (I, J) -> four uniforms in [0,1): pure function of the grid index
-        h = (I * 73856093) ^ (J * 19349663)
-
-        def u(k):
-            v = (h * (2 * k + 1) + 0x9E3779B9 * (k + 1)) & 0x7fffffff
-            v = (v * 1103515245 + 12345) & 0x7fffffff
-            return (v >> 7).to(torch.float32) / float(1 << 24)
-        cx = (I.float() + 0.15 + 0.7 * u(0)) * pitch
-        cy = (J.float() + 0.15 + 0.7 * u(1)) * pitch
-        side = size_range[0] + (size_range[1] - size_range[0]) * u(2)
-        score = 0.3 + 0.65 * u(3)
+        cx, cy, side, score = _field_nuclei(I, J, pitch, size_range)
         inside = (cx >= x0) & (cx < x1) & (cy >= y0) & (cy < y1)
         cx, cy, side, score = cx[inside] - x0, cy[inside] - y0, side[inside], score[inside]
         jitter = torch.rand((ncell * ncell,), generator=g, device=dev)[:score.numel()]   # fixed draw count per tile
@@ -181,3 +188,77 @@ def nuclei_match_case(k: int, g: int, size: int, seed: int, device="cuda"):
         return d
 
     return side(cp, rp, {'scores': scores, 'labels': labels_p}), side(cg, rg, {'labels': labels_g})
+
+
+def slide_nuclei(region, canvas=None, pitch: float = 18.7, size_range=(12.0, 30.0), nc: int = 4, seed: int = 0,
+                 jitter: float = 0.0, device="cuda", rows_per_band: int = 256, masks_per_chunk: int = 1 << 20):
+    """The nuclei of slide_tile_logits' global field (same `pitch` / `size_range`) whose centres lie in the slide region
+    (x0, y0, x1, y1), as ground truth: 'boxes' [n, 4] (clipped to the canvas), 'labels' [n] int64 in 1..nc, 'scores'
+    (the field's), and 'masks', filled ellipses (x radius side / 2, y radius 0.7-1.0 of it) built straight into a
+    PackedMasks -- each one in a small patch of its own, never a canvas as large as the slide.  Coordinates are slide
+    pixels on the (H, W) `canvas` (default: (y1, x1)).  Rows in grid order (row-major over the field's grid).
+    jitter > 0: every nucleus moves by up to `jitter` px and its radii by up to jitter / 10 relative, seeded by (seed,
+    grid index) -- a second, prediction-like set over the same field."""
+    from .masks import PackedMasks
+    dev = torch.device(device)
+    x0, y0, x1, y1 = (float(v) for v in region)
+    H, W = (int(y1), int(x1)) if canvas is None else (int(canvas[0]), int(canvas[1]))
+    i0, i1 = int(math.floor(x0 / pitch)) - 1, int(math.ceil(x1 / pitch)) + 1
+    j0, j1 = int(math.floor(y0 / pitch)) - 1, int(math.ceil(y1 / pitch)) + 1
+    rmax = 0.5 * size_range[1] * (1.0 + jitter / 10.0)
+    S = int(math.ceil(2.0 * rmax)) + 2                   # patch side: holds every ellipse
+    boxes, labels, scores, cs, rs = [], [], [], [], []
+    ii = torch.arange(i0, i1 + 1, device=dev, dtype=torch.int64)
+    for jb in range(j0, j1 + 1, rows_per_band):
+        jj = torch.arange(jb, min(jb + rows_per_band, j1 + 1), device=dev, dtype=torch.int64)
+        J, I = torch.meshgrid(jj, ii, indexing='ij')
+        I, J = I.reshape(-1), J.reshape(-1)
+        cx, cy, side, score = _field_nuclei(I, J, pitch, size_range)
+        keep = (cx >= x0) & (cx < x1) & (cy >= y0) & (cy < y1)
+        I, J, cx, cy, side, score = I[keep], J[keep], cx[keep], cy[keep], side[keep], score[keep]
+        h = (I * 73856093) ^ (J * 19349663)
+        rx = 0.5 * side
+        ry = rx * (0.7 + 0.3 * _field_uniform(h, 5))
+        if jitter > 0:
+            hs = h ^ (int(seed) * 83492791 + 1)
+            cx = cx + jitter * (2.0 * _field_uniform(hs, 6) - 1.0)
+            cy = cy + jitter * (2.0 * _field_uniform(hs, 7) - 1.0)
+            rx = rx * (1.0 + jitter / 10.0 * (2.0 * _field_uniform(hs, 8) - 1.0))
+            ry = ry * (1.0 + jitter / 10.0 * (2.0 * _field_uniform(hs, 9) - 1.0))
+        labels.append(1 + torch.clamp((_field_uniform(h, 4) * nc).long(), max=nc - 1))
+        scores.append(score)
+        boxes.append(torch.stack([cx - rx, cy - ry, cx + rx, cy + ry], 1))
+        cs.append(torch.stack([cx, cy], 1))
+        rs.append(torch.stack([rx, ry], 1))
+    boxes, c, r = torch.cat(boxes), torch.cat(cs), torch.cat(rs)
+    boxes[:, 0::2] = boxes[:, 0::2].clamp(0, W)
+    boxes[:, 1::2] = boxes[:, 1::2].clamp(0, H)
+    # masks: patch S x S at (floor(cx - rx), floor(cy - ry)); pixel centres tested as ellipse_masks does
+    n = int(c.shape[0])
+    geoms, offs, bits, base = [], [], [], 0
+    k = torch.arange(S, device=dev, dtype=torch.float32)
+    for a in range(0, n, masks_per_chunk):
+        cc, rr = c[a:a + masks_per_chunk], r[a:a + masks_per_chunk]
+        org = torch.floor(cc - rr)
+        px = org[:, 0, None] + k[None, :]                 # [m, S] pixel x
+        py = org[:, 1, None] + k[None, :]
+        fx = ((px + 0.5 - cc[:, 0, None]) / rr[:, 0, None]) ** 2
+        fy = ((py + 0.5 - cc[:, 1, None]) / rr[:, 1, None]) ** 2
+        inside = (fy[:, :, None] + fx[:, None, :] <= 1.0)
+        inside &= ((py >= 0) & (py < H))[:, :, None] & ((px >= 0) & (px < W))[:, None, :]
+        pm = PackedMasks.from_dense(inside)
+        g = pm.geom.clone()
+        live = (g[:, 2] > 0) & (g[:, 3] > 0)
+        g[:, 0] += torch.where(live, org[:, 0].to(torch.int32), 0)
+        g[:, 1] += torch.where(live, org[:, 1].to(torch.int32), 0)
+        geoms.append(g)
+        offs.append(pm.offsets[:-1] + base)
+        bits.append(pm.bits)
+        base += int(pm.bits.numel())
+    if n == 0:
+        geoms, offs = [torch.zeros((0, 4), dtype=torch.int32, device=dev)], [torch.zeros(0, dtype=torch.int64, device=dev)]
+    masks = PackedMasks(torch.cat(geoms).contiguous(),
+                        torch.cat(offs + [torch.tensor([base], dtype=torch.int64, device=dev)]),
+                        torch.cat(bits) if bits else torch.zeros(0, dtype=torch.int32, device=dev), H, W,
+                        torch.zeros(1, dtype=torch.int32, device=dev))
+    return {'boxes': boxes.contiguous(), 'labels': torch.cat(labels), 'scores': torch.cat(scores), 'masks': masks}

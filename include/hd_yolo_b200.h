@@ -539,6 +539,58 @@ HDY_API int hdy_match_mask_pairs(const int32_t* pred_geom, const int64_t* pred_o
                                  float iou_min, int cand_cap, uint32_t* cand, int cap, uint64_t* pair_keys,
                                  int32_t* counts, int32_t* status, hdy_stream_t stream);
 
+/* f2 at region and slide scale (match_predictions(..., binned=True)): the pairs of hdy_match_pairs /
+ * hdy_match_mask_pairs, bit for bit, without their P * G < 2^32 limit or their O(P * G) work: P, G < 2^31 and fewer
+ * than 2^31 pairs (candidates, for masks).  iou_min > 0.  The ground truth is binned into a uniform grid; a pair is
+ * tested only in the cell holding (max(x0_p, x0_g), max(y0_p, y0_g)), so each pair is seen exactly once.  Rectangles:
+ * boxes [n, 4] xyxy fp32 (rows with a non-finite coordinate or without positive width and height match nothing and are
+ * never binned) or mask windows geom [n, 4] {x0, y0, w, h} (empty windows likewise).  All arrays 16-byte aligned where
+ * they hold rectangles.  Grid: cell (cx, cy) of a point is clamp(floor((x - ox) * inv_cell), 0, nx - 1) (same in y),
+ * evaluated in fp32; any grid gives the same pairs, the grid only sets the cost.
+ *
+ * bin_stats: stats [6] u64 = orderable_u32 of min x0, min y0, max x1, max y1 of the valid ground truth (x1, y1: the last
+ * pixel of a window), their number, and the sum of their sides max(w, h) in 1/16 px -- what the caller picks the grid
+ * from.  Pass exactly one of gt_boxes / gt_geom.
+ * bin_entries, count pass (cell_keys NULL): ent_off [G+1] = exclusive scan of the cells each ground truth covers
+ * (ent_off[G] = E entries).  Emit pass: cell_keys [E] = cell << 32 | j, in ascending j.  The caller then sorts
+ * cell_keys by the cell (hdy_sort_keys_bytes, first_byte 4: stable, so every cell lists ascending j) and
+ * bin_cells writes cell_start [n_cells + 1] (n_cells = nx * ny): the first entry of every cell.
+ * boxes_binned, count pass (pair_rank / pair_j / pair_iou NULL): pair_off [P+1] = exclusive scan of the pairs with
+ * box_iou >= iou_min of every prediction rank (pred_order [P] i32: rank -> row; NULL: identity).  Emit pass: the pairs
+ * of rank r go to [pair_off[r], pair_off[r+1]) of pair_rank / pair_j / pair_iou, sorted by j: the whole list is in
+ * row-major (rank, j) order.
+ * mask_candidates_binned: the same two passes over windows; a pair is a candidate when its windows overlap and its
+ * IoU bound (hdy_match_mask_pairs) reaches iou_min.  areas from hdy_mask_areas.
+ * mask_exact_list: counts every candidate's intersection exactly (cand_iou [n_cand] scratch) and compacts the pairs
+ * with iou >= iou_min, in candidate order, into pair_rank / pair_j / pair_iou; *pair_count (device) = their number
+ * (block_scratch: 4096 int32).
+ * order_keys: keys [n] = ~orderable(ious[i]) << 32 | i; sorting their high half (hdy_sort_keys_bytes, first_byte 4,
+ * n_bytes 4) orders a (rank, j)-ordered list by IoU, descending, with ties in (rank, j) order. */
+HDY_API int hdy_match_bin_stats(const float* gt_boxes, const int32_t* gt_geom, int G, uint64_t* stats,
+                                hdy_stream_t stream);
+HDY_API int hdy_match_bin_entries(const float* gt_boxes, const int32_t* gt_geom, int G, float ox, float oy,
+                                  float inv_cell, int nx, int ny, int64_t* ent_off, uint64_t* cell_keys,
+                                  hdy_stream_t stream);
+HDY_API int hdy_match_bin_cells(const uint64_t* cell_keys, int64_t E, int64_t n_cells, int64_t* cell_start,
+                                hdy_stream_t stream);
+HDY_API int hdy_match_boxes_binned(const float* pred_boxes, const int32_t* pred_order, int P, const float* gt_boxes,
+                                   int G, float ox, float oy, float inv_cell, int nx, int ny, const int64_t* cell_start,
+                                   const uint64_t* cell_keys, float iou_min, int64_t* pair_off, int32_t* pair_rank,
+                                   int32_t* pair_j, float* pair_iou, hdy_stream_t stream);
+HDY_API int hdy_match_mask_candidates_binned(const int32_t* pred_geom, const int32_t* pred_areas,
+                                             const int32_t* pred_order, int P, const int32_t* gt_geom,
+                                             const int32_t* gt_areas, int G, float ox, float oy, float inv_cell,
+                                             int nx, int ny, const int64_t* cell_start, const uint64_t* cell_keys,
+                                             float iou_min, int64_t* cand_off, int32_t* cand_rank, int32_t* cand_j,
+                                             hdy_stream_t stream);
+HDY_API int hdy_match_mask_exact_list(const int32_t* pred_geom, const int64_t* pred_offsets, const uint32_t* pred_bits,
+                                      const int32_t* pred_areas, const int32_t* pred_order, const int32_t* gt_geom,
+                                      const int64_t* gt_offsets, const uint32_t* gt_bits, const int32_t* gt_areas,
+                                      const int32_t* cand_rank, const int32_t* cand_j, int64_t n_cand, float iou_min,
+                                      float* cand_iou, int32_t* pair_rank, int32_t* pair_j, float* pair_iou,
+                                      int32_t* pair_count, int32_t* block_scratch, hdy_stream_t stream);
+HDY_API int hdy_match_order_keys(const float* ious, int64_t n, uint64_t* keys, hdy_stream_t stream);
+
 /* Utility: zero n int32 words (keeps the host mirror free of extra torch launches). */
 HDY_API int hdy_zero_i32(int32_t* p, size_t n, hdy_stream_t stream);
 
