@@ -23,6 +23,7 @@ from .ops import (  # noqa: F401
 
 from . import masks  # noqa: F401,E402
 from .masks import (  # noqa: F401,E402
+    MaskContours,
     PackedMasks,
     mask_select,
     paste_masks_in_image,
@@ -49,7 +50,7 @@ from .slide import (  # noqa: F401,E402
 )
 
 from . import dist, hnet, io, metrics, pipeline, roi  # noqa: F401,E402
-from .io import load_detections, save_detections  # noqa: F401,E402
+from .io import load_detections, save_detections, save_geojson  # noqa: F401,E402
 from .metrics import APMeter, box_iou, match_predictions  # noqa: F401,E402
 from .roi import batch_rois, compute_outputs, multiscale_roi_align, roi_align  # noqa: F401,E402
 from .pipeline import SlidePostprocessor  # noqa: F401,E402

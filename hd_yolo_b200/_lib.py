@@ -77,6 +77,8 @@ SIGNATURES = {
     "hdy_paste_geometry": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "hdy_paste_masks_packed": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, C.c_int64, _vp, _vp]),
     "hdy_unpack_masks": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp]),
+    "hdy_mask_contour_sizes": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp]),
+    "hdy_mask_contours": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "hdy_process_mask_workspace_bytes": (_sz, [_i, _i]),
     "hdy_process_mask": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _sz, _vp]),
     "hdy_process_mask_geometry": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),

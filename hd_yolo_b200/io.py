@@ -6,6 +6,9 @@ One little-endian file: a JSON header line (magic, version, array table with dty
 package works in (``boxes`` fp32 [k,4], ``scores`` fp32 [k], ``labels`` int64 stored as int16, optional ``index``);
 masks are the cropped bit planes of ``PackedMasks`` (geom / offsets / bits), ~100-300 bytes per nucleus.  Host-side
 only (CUDA tensors are read back once); loading memory-maps the file and returns CPU tensors.
+
+``save_geojson`` writes the boundary polygons of PackedMasks.contours() as one RFC 7946 FeatureCollection, the format
+slide viewers, annotation tools and morphometry code read.
 """
 from __future__ import annotations
 
@@ -17,9 +20,9 @@ import numpy as np
 import torch
 
 from ._lib import HdyError
-from .masks import PackedMasks
+from .masks import MaskContours, PackedMasks
 
-__all__ = ["save_detections", "load_detections"]
+__all__ = ["save_detections", "load_detections", "save_geojson"]
 
 MAGIC = "hd_yolo_b200.detections"
 VERSION = 1
@@ -101,3 +104,61 @@ def load_detections(path: str, mmap: bool = True) -> Tuple[Dict[str, torch.Tenso
         masks = PackedMasks(out.pop("mask_geom"), out.pop("mask_offsets"), out.pop("mask_bits"), int(H), int(W),
                             torch.zeros((1,), dtype=torch.int32))
     return out, masks, header.get("meta", {})
+
+
+def save_geojson(path: str, result: Dict[str, torch.Tensor], contours: MaskContours, chunk_rows: int = 65536) -> int:
+    """Writes one RFC 7946 FeatureCollection with a Feature per row of `contours` that has a ring: a Polygon for one
+    exterior ring, a MultiPolygon for several, each exterior followed by its holes, every ring closed by repeating its
+    first vertex.  Coordinates are canvas pixel corners (x, y).  Properties: 'index' (``result['index']`` if present,
+    else the row), 'score' and 'label' (``result['scores']`` / ``result['labels']`` if present).  `contours` may be on
+    the CPU or a CUDA device; it is read back `chunk_rows` rows at a time and the text is streamed to `path` + '.tmp',
+    then renamed.  Returns the number of Features written."""
+    K = len(contours)
+    cols = {}
+    for key, name in (("index", "index"), ("scores", "score"), ("labels", "label")):
+        t = result.get(key)
+        if isinstance(t, torch.Tensor):
+            if t.shape[0] != K:
+                raise HdyError(f"result['{key}'] has {t.shape[0]} rows, contours {K}")
+            cols[name] = t
+    if chunk_rows < 1:
+        raise HdyError("chunk_rows must be >= 1")
+    n = 0
+    tmp = path + ".tmp"
+    with open(tmp, "w") as f:
+        f.write('{"type": "FeatureCollection", "features": [')
+        for a in range(0, K, chunk_rows):
+            b = min(a + chunk_rows, K)
+            mr = contours.mask_rings[a:b + 1].cpu().tolist()
+            r0, r1 = mr[0], mr[-1]
+            rv = contours.ring_verts[r0:r1 + 1].cpu().numpy()
+            xy = contours.xy[int(rv[0]):int(rv[-1])].cpu().numpy().tolist()
+            parent = contours.parent[r0:r1].cpu().numpy().tolist()
+            props = {name: t[a:b].cpu().tolist() for name, t in cols.items()}
+            v0 = int(rv[0])
+            for i in range(a, b):
+                lo, hi = mr[i - a], mr[i - a + 1]
+                if lo == hi:
+                    continue
+                polys, at = [], {}
+                for r in range(lo, hi):
+                    ring = xy[int(rv[r - r0]) - v0:int(rv[r - r0 + 1]) - v0]
+                    ring.append(ring[0])
+                    p = parent[r - r0]
+                    if p < 0:
+                        at[r] = len(polys)
+                        polys.append([ring])
+                    else:
+                        polys[at[p]].append(ring)
+                geometry = ({"type": "Polygon", "coordinates": polys[0]} if len(polys) == 1 else
+                            {"type": "MultiPolygon", "coordinates": polys})
+                pr = {"index": props["index"][i - a] if "index" in props else i}
+                for name in ("score", "label"):
+                    if name in props:
+                        pr[name] = props[name][i - a]
+                f.write((",\n" if n else "\n") +
+                        json.dumps({"type": "Feature", "geometry": geometry, "properties": pr}, separators=(",", ":")))
+                n += 1
+        f.write("\n]}\n")
+    os.replace(tmp, path)
+    return n

@@ -25,8 +25,26 @@ from .ops import _Scratch, _aligned16, _call, _need_cuda, _need_head_tensor, _st
 
 _pm_scratch = _Scratch()
 
-__all__ = ["PackedMasks", "mask_select", "paste_masks_in_image", "paste_masks_packed", "process_mask",
+__all__ = ["MaskContours", "PackedMasks", "mask_select", "paste_masks_in_image", "paste_masks_packed", "process_mask",
            "process_mask_batch", "process_mask_packed", "SlideMaskBuilder"]
+
+
+@dataclass
+class MaskContours:
+    """Boundary polygons of K masks (PackedMasks.contours(); contract in include/hd_yolo_b200.h and DESIGN §3.10).
+
+    The rings of mask i are mask_rings[i] .. mask_rings[i+1]-1; ring r's vertices are xy[ring_verts[r]:ring_verts[r+1]]
+    (x, y) pixel corners on the canvas, y down, starting at the least one in (y, x) order, not closed.  Exterior rings
+    have positive shoelace area (counter-clockwise read with y up); parent[r] = -1 for them, else the index of the
+    exterior ring of the hole's component."""
+
+    mask_rings: torch.Tensor   # [K+1] int64
+    ring_verts: torch.Tensor   # [R+1] int64
+    xy: torch.Tensor           # [V, 2] int32
+    parent: torch.Tensor       # [R] int32
+
+    def __len__(self):
+        return self.mask_rings.shape[0] - 1
 
 
 @dataclass
@@ -106,6 +124,28 @@ class PackedMasks:
             _call("hdy_mask_areas", ptr(_aligned16(self.geom.contiguous())), ptr(self.offsets),
                   ptr(self._bits_nonempty()), K, ptr(out), _stream())
         return out
+
+    def contours(self) -> MaskContours:
+        """The boundary polygons of every mask, traced on the device (csrc/contours.cu).  One 16-byte device->host read
+        (the ring and vertex totals).  Rows: ``masks.select(rows).contours()``."""
+        if not self.geom.is_cuda:
+            raise HdyError("contours() needs the planes on a CUDA device: hd_yolo_b200 has no CPU fallback")
+        self.check()
+        K, dev = len(self), self.geom.device
+        geom, bits = _aligned16(self.geom.contiguous()), self._bits_nonempty()
+        mask_rings = torch.empty((K + 1,), dtype=torch.int64, device=dev)
+        vert_off = torch.empty((K + 1,), dtype=torch.int64, device=dev)
+        _call("hdy_mask_contour_sizes", ptr(geom), ptr(self.offsets), ptr(bits), K, ptr(mask_rings), ptr(vert_off),
+              _stream(), launches=4)
+        R, V = torch.stack([mask_rings[K], vert_off[K]]).tolist()
+        if R >= 2 ** 31:
+            raise HdyError(f"{R} rings: parent indices are int32, trace fewer rows at a time")
+        ring_verts = torch.empty((R + 1,), dtype=torch.int64, device=dev)
+        parent = torch.empty((max(R, 1),), dtype=torch.int32, device=dev)
+        xy = torch.empty((max(V, 1), 2), dtype=torch.int32, device=dev)
+        _call("hdy_mask_contours", ptr(geom), ptr(self.offsets), ptr(bits), K, ptr(mask_rings), ptr(vert_off),
+              ptr(ring_verts), ptr(parent), ptr(xy), _stream(), launches=2)
+        return MaskContours(mask_rings, ring_verts, xy[:V], parent[:R])
 
     def select(self, rows) -> "PackedMasks":
         """The masks of `rows` (index tensor or sequence), in that order, sharing `bits`: geom[rows] and offsets[rows]

@@ -220,6 +220,31 @@ HDY_API int hdy_paste_masks_packed(const float* src, const int32_t* channel, con
 HDY_API int hdy_unpack_masks(const int32_t* geom, const int64_t* offsets, const uint32_t* bits, int K, int H,
                              int W, uint8_t* out, hdy_stream_t stream);
 
+/* Boundary polygons of cropped bit planes (PackedMasks.contours, csrc/contours.cu).  Coordinates are canvas pixel
+ * corners: pixel (x, y) is the unit square [x, x+1] x [y, y+1], x to the right, y down.  Pixels outside a mask's
+ * window are unset; padding bits beyond w are ignored, whatever they hold (as in hdy_mask_areas).
+ *   edges     a boundary edge is a unit edge between a set and an unset pixel, directed so that the set pixel lies on
+ *             its right as drawn on screen (y down): a top edge runs toward +x;
+ *   saddles   at a corner whose 2 x 2 pixels are set only on one diagonal a ring turns right, hugging the pixel it
+ *             walks along: set pixels are 4-connected, background pixels 8-connected;
+ *   vertices  only the corners where the direction changes, the closing vertex not repeated;
+ *   order     each ring starts at its least vertex in (y, x) order (unique within the ring); a mask's rings are
+ *             ordered by that start, and no two share one;
+ *   sign      the shoelace sum 1/2 sum(x_i y_i+1 - x_i+1 y_i) is positive for exterior rings and negative for holes
+ *             (counter-clockwise exteriors read with y up, RFC 7946);
+ *   parent    every ring hugs one 4-connected component, which has exactly one exterior ring; parent[r] = -1 for an
+ *             exterior ring, else the global index of its component's exterior ring.
+ * hdy_mask_contour_sizes: ring_off [K+1], vert_off [K+1] = exclusive scans of each mask's ring and vertex counts, the
+ * totals R and V at [K].  hdy_mask_contours then fills ring_verts [R+1] (first vertex of each ring, ring_verts[R] = V),
+ * parent [R] (R < 2^31) and xy [V, 2] i32 (8-byte aligned); ring r of mask i is one of ring_off[i] .. ring_off[i+1]-1.
+ * A mask is addressed through geom[i] (16-byte aligned) and offsets[i] only.  Any window size works: windows up to
+ * 64 x 64 are traced one thread per mask, larger ones one CTA per mask. */
+HDY_API int hdy_mask_contour_sizes(const int32_t* geom, const int64_t* offsets, const uint32_t* bits, int K,
+                                   int64_t* ring_off, int64_t* vert_off, hdy_stream_t stream);
+HDY_API int hdy_mask_contours(const int32_t* geom, const int64_t* offsets, const uint32_t* bits, int K,
+                              const int64_t* ring_off, const int64_t* vert_off, int64_t* ring_verts, int32_t* parent,
+                              int32_t* xy, hdy_stream_t stream);
+
 /* North-star process_mask (ultralytics/yolov5 v7 utils/segment/general.py::process_mask + crop_mask; the
  * reference itself has no such function): mask = sigmoid(coef . protos), zero outside the box scaled by
  * (mw/iw, mh/ih), optional bilinear upsample (align_corners=False) to (ih, iw), > 0.5.  Batched over tiles:
