@@ -24,6 +24,7 @@ from .ops import (  # noqa: F401
 from . import masks  # noqa: F401,E402
 from .masks import (  # noqa: F401,E402
     MaskContours,
+    MaskMeasurements,
     PackedMasks,
     mask_select,
     paste_masks_in_image,

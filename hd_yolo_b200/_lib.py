@@ -79,6 +79,7 @@ SIGNATURES = {
     "hdy_unpack_masks": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _vp]),
     "hdy_mask_contour_sizes": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "hdy_mask_contours": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "hdy_mask_measure": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "hdy_process_mask_workspace_bytes": (_sz, [_i, _i]),
     "hdy_process_mask": (_i, [_vp, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _sz, _vp]),
     "hdy_process_mask_geometry": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),

@@ -8,19 +8,21 @@ masks are the cropped bit planes of ``PackedMasks`` (geom / offsets / bits), ~10
 only (CUDA tensors are read back once); loading memory-maps the file and returns CPU tensors.
 
 ``save_geojson`` writes the boundary polygons of PackedMasks.contours() as one RFC 7946 FeatureCollection, the format
-slide viewers, annotation tools and morphometry code read.
+slide viewers, annotation tools and morphometry code read; with ``measurements`` (PackedMasks.measure()) each Feature
+also carries its row of the morphometry table.
 """
 from __future__ import annotations
 
 import json
+import math
 import os
-from typing import Dict, Optional, Tuple
+from typing import Dict, Optional, Tuple, Union
 
 import numpy as np
 import torch
 
 from ._lib import HdyError
-from .masks import MaskContours, PackedMasks
+from .masks import MaskContours, MaskMeasurements, PackedMasks
 
 __all__ = ["save_detections", "load_detections", "save_geojson"]
 
@@ -106,13 +108,21 @@ def load_detections(path: str, mmap: bool = True) -> Tuple[Dict[str, torch.Tenso
     return out, masks, header.get("meta", {})
 
 
-def save_geojson(path: str, result: Dict[str, torch.Tensor], contours: MaskContours, chunk_rows: int = 65536) -> int:
+def _json_number(v):
+    """JSON has no NaN or infinity: such a value is written as null."""
+    return v if not isinstance(v, float) or math.isfinite(v) else None
+
+
+def save_geojson(path: str, result: Dict[str, torch.Tensor], contours: MaskContours, chunk_rows: int = 65536,
+                 measurements: Union[MaskMeasurements, Dict[str, torch.Tensor], None] = None) -> int:
     """Writes one RFC 7946 FeatureCollection with a Feature per row of `contours` that has a ring: a Polygon for one
     exterior ring, a MultiPolygon for several, each exterior followed by its holes, every ring closed by repeating its
     first vertex.  Coordinates are canvas pixel corners (x, y).  Properties: 'index' (``result['index']`` if present,
     else the row), 'score' and 'label' (``result['scores']`` / ``result['labels']`` if present).  `contours` may be on
     the CPU or a CUDA device; it is read back `chunk_rows` rows at a time and the text is streamed to `path` + '.tmp',
-    then renamed.  Returns the number of Features written."""
+    then renamed.  `measurements` (a MaskMeasurements, whose ``columns()`` are written, or a dict of [K] tensors) adds
+    ``properties.measurements = {name: value}`` to each Feature, the key QuPath reads; non-finite values are written as
+    null.  Returns the number of Features written."""
     K = len(contours)
     cols = {}
     for key, name in (("index", "index"), ("scores", "score"), ("labels", "label")):
@@ -121,6 +131,11 @@ def save_geojson(path: str, result: Dict[str, torch.Tensor], contours: MaskConto
             if t.shape[0] != K:
                 raise HdyError(f"result['{key}'] has {t.shape[0]} rows, contours {K}")
             cols[name] = t
+    if isinstance(measurements, MaskMeasurements):
+        measurements = measurements.columns()
+    for key, t in (measurements or {}).items():
+        if not isinstance(t, torch.Tensor) or t.dim() != 1 or t.shape[0] != K:
+            raise HdyError(f"measurements['{key}'] must be a [{K}] tensor")
     if chunk_rows < 1:
         raise HdyError("chunk_rows must be >= 1")
     n = 0
@@ -135,6 +150,7 @@ def save_geojson(path: str, result: Dict[str, torch.Tensor], contours: MaskConto
             xy = contours.xy[int(rv[0]):int(rv[-1])].cpu().numpy().tolist()
             parent = contours.parent[r0:r1].cpu().numpy().tolist()
             props = {name: t[a:b].cpu().tolist() for name, t in cols.items()}
+            meas = {name: t[a:b].cpu().tolist() for name, t in measurements.items()} if measurements else None
             v0 = int(rv[0])
             for i in range(a, b):
                 lo, hi = mr[i - a], mr[i - a + 1]
@@ -156,6 +172,8 @@ def save_geojson(path: str, result: Dict[str, torch.Tensor], contours: MaskConto
                 for name in ("score", "label"):
                     if name in props:
                         pr[name] = props[name][i - a]
+                if meas is not None:
+                    pr["measurements"] = {name: _json_number(v[i - a]) for name, v in meas.items()}
                 f.write((",\n" if n else "\n") +
                         json.dumps({"type": "Feature", "geometry": geometry, "properties": pr}, separators=(",", ":")))
                 n += 1

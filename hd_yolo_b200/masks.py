@@ -14,8 +14,9 @@ No CPU fallback: CPU tensors raise HdyError.
 """
 from __future__ import annotations
 
+import math
 from dataclasses import dataclass
-from typing import Optional, Tuple
+from typing import Dict, Optional, Tuple
 
 import torch
 
@@ -25,7 +26,7 @@ from .ops import _Scratch, _aligned16, _call, _need_cuda, _need_head_tensor, _st
 
 _pm_scratch = _Scratch()
 
-__all__ = ["MaskContours", "PackedMasks", "mask_select", "paste_masks_in_image", "paste_masks_packed", "process_mask",
+__all__ = ["MaskContours", "MaskMeasurements", "PackedMasks", "mask_select", "paste_masks_in_image", "paste_masks_packed", "process_mask",
            "process_mask_batch", "process_mask_packed", "SlideMaskBuilder"]
 
 
@@ -45,6 +46,147 @@ class MaskContours:
 
     def __len__(self):
         return self.mask_rings.shape[0] - 1
+
+
+@dataclass
+class MaskMeasurements:
+    """Morphometry of K masks (PackedMasks.measure(); contract in include/hd_yolo_b200.h and DESIGN §3.10b).
+
+    Pixel (x, y) is the unit square [x, x+1] x [y, y+1] of the canvas, y down; dx = x - gx and dy = y - gy are pixel
+    indices relative to the window (gx, gy, w, h) = geom[i].  The fields are exact, computed on the device:
+
+    * area [K] i32; bbox [K, 4] i32 (x0, y0, x1, y1), the tight box of the set pixels, x1 / y1 exclusive;
+    * moments [K, 5] i64: sum dx, sum dy, sum dx^2, sum dy^2, sum dx*dy over the set pixels;
+    * quads [K, 4] i32: over the (w+1)(h+1) corners of the window, the 2 x 2 pixel patterns around each corner with n1
+      (one set), n2 (two sharing an edge), n3 (three) and nD (two on a diagonal) set pixels;
+    * convex_area2 [K] i64, hull_verts [K] i32, feret_max2 [K] i64: twice the area, the vertex count and the largest
+      squared vertex distance of the convex hull of the set pixels' squares;
+    * convex_perimeter, feret_min [K] f64: the hull's edge lengths summed in order from its least vertex in (y, x)
+      order, and its least caliper width.
+
+    The derived columns are fp64 expressions of those, computed with torch on access (A = area):
+
+    * centroid = (gx + sum dx / A + 0.5, gy + sum dy / A + 0.5), the centroid of the pixel squares;
+    * perimeter = n1 + n2 + n3 + 2 nD, the length of the contours() rings, holes included;
+    * perimeter_smooth = n2 + (n1 + n3 + 2 nD) sqrt(1/2), the marching-squares contour through the pixel-edge midpoints;
+    * euler = (n1 - n3 + 2 nD) / 4: 4-connected components minus holes;
+    * convex_area = convex_area2 / 2; solidity = A / convex_area; extent = A / bbox area;
+    * equivalent_diameter = sqrt(4 A / pi); circularity = 4 pi A / perimeter_smooth^2, not clamped: a digital disc
+      gives 0.83 at radius 6 and 0.87 at radius 20, not 1;
+    * mx = sum dx / A, c20 = sum dx^2 / A - mx^2, c02 likewise, c11 = sum dx dy / A - mx my: the central second moments
+      of the pixel centres; l1, l2 = (c20 + c02) / 2 +- sqrt(((c20 - c02) / 2)^2 + c11^2), l2 clamped at 0;
+      major_axis, minor_axis = 4 sqrt(l1), 4 sqrt(l2) (skimage's axis_major_length); eccentricity = sqrt(1 - l2 / l1),
+      0 when l1 = 0; orientation = atan2(2 c11, c20 - c02) / 2, the major axis' angle from +x toward +y, in
+      (-pi/2, pi/2];
+    * feret_max = sqrt(feret_max2).
+
+    Rows with area 0 give NaN for the centroid and every ratio."""
+
+    geom: torch.Tensor              # [K, 4] int32: the windows the moments are relative to
+    area: torch.Tensor              # [K] int32
+    bbox: torch.Tensor              # [K, 4] int32
+    moments: torch.Tensor           # [K, 5] int64
+    quads: torch.Tensor             # [K, 4] int32
+    convex_area2: torch.Tensor      # [K] int64
+    hull_verts: torch.Tensor        # [K] int32
+    feret_max2: torch.Tensor        # [K] int64
+    convex_perimeter: torch.Tensor  # [K] float64
+    feret_min: torch.Tensor         # [K] float64
+
+    def __len__(self):
+        return self.area.shape[0]
+
+    def _q(self):
+        q = self.quads.long()
+        return q[:, 0], q[:, 1], q[:, 2], q[:, 3]
+
+    @property
+    def centroid(self) -> torch.Tensor:
+        """[K, 2] float64 (x, y) in canvas pixels: the coordinates of the contours() polygons."""
+        A, m, g = self.area.double(), self.moments.double(), self.geom.double()
+        return torch.stack([g[:, 0] + m[:, 0] / A + 0.5, g[:, 1] + m[:, 1] / A + 0.5], 1)
+
+    @property
+    def perimeter(self) -> torch.Tensor:
+        n1, n2, n3, nd = self._q()
+        return (n1 + n2 + n3 + 2 * nd).double()
+
+    @property
+    def perimeter_smooth(self) -> torch.Tensor:
+        n1, n2, n3, nd = self._q()
+        return n2.double() + (n1 + n3 + 2 * nd).double() * math.sqrt(0.5)
+
+    @property
+    def euler(self) -> torch.Tensor:
+        n1, _, n3, nd = self._q()
+        return (n1 - n3 + 2 * nd) // 4
+
+    @property
+    def convex_area(self) -> torch.Tensor:
+        return self.convex_area2.double() / 2
+
+    @property
+    def solidity(self) -> torch.Tensor:
+        return self.area.double() / self.convex_area
+
+    @property
+    def extent(self) -> torch.Tensor:
+        b = self.bbox.long()
+        return self.area.double() / ((b[:, 2] - b[:, 0]) * (b[:, 3] - b[:, 1])).double()
+
+    @property
+    def equivalent_diameter(self) -> torch.Tensor:
+        return torch.sqrt(4 * self.area.double() / math.pi)
+
+    @property
+    def circularity(self) -> torch.Tensor:
+        ps = self.perimeter_smooth
+        return 4 * math.pi * self.area.double() / (ps * ps)
+
+    def _central(self):
+        A, m = self.area.double(), self.moments.double()
+        mx, my = m[:, 0] / A, m[:, 1] / A
+        return m[:, 2] / A - mx * mx, m[:, 3] / A - my * my, m[:, 4] / A - mx * my
+
+    def _eigen(self):
+        c20, c02, c11 = self._central()
+        d = (c20 - c02) / 2
+        half, root = (c20 + c02) / 2, torch.sqrt(d * d + c11 * c11)
+        return half + root, torch.clamp(half - root, min=0.0)
+
+    @property
+    def major_axis(self) -> torch.Tensor:
+        return 4 * torch.sqrt(self._eigen()[0])
+
+    @property
+    def minor_axis(self) -> torch.Tensor:
+        return 4 * torch.sqrt(self._eigen()[1])
+
+    @property
+    def eccentricity(self) -> torch.Tensor:
+        l1, l2 = self._eigen()
+        return torch.where(l1 == 0, torch.zeros_like(l1), torch.sqrt(1 - l2 / l1))
+
+    @property
+    def orientation(self) -> torch.Tensor:
+        c20, c02, c11 = self._central()
+        return torch.atan2(2 * c11, c20 - c02) / 2
+
+    @property
+    def feret_max(self) -> torch.Tensor:
+        return torch.sqrt(self.feret_max2.double())
+
+    def columns(self) -> Dict[str, torch.Tensor]:
+        """The user-facing columns, one [K] tensor each, in table order.  ``save_detections(path, {**result,
+        **m.columns()}, masks)`` stores them beside the detections; ``save_geojson(..., measurements=m)`` writes them
+        into each Feature's properties."""
+        c = self.centroid
+        return {"centroid_x": c[:, 0], "centroid_y": c[:, 1], "area": self.area, "perimeter": self.perimeter,
+                "perimeter_smooth": self.perimeter_smooth, "euler": self.euler, "convex_area": self.convex_area,
+                "convex_perimeter": self.convex_perimeter, "solidity": self.solidity, "extent": self.extent,
+                "equivalent_diameter": self.equivalent_diameter, "circularity": self.circularity,
+                "major_axis": self.major_axis, "minor_axis": self.minor_axis, "eccentricity": self.eccentricity,
+                "orientation": self.orientation, "feret_max": self.feret_max, "feret_min": self.feret_min}
 
 
 @dataclass
@@ -146,6 +288,36 @@ class PackedMasks:
         _call("hdy_mask_contours", ptr(geom), ptr(self.offsets), ptr(bits), K, ptr(mask_rings), ptr(vert_off),
               ptr(ring_verts), ptr(parent), ptr(xy), _stream(), launches=2)
         return MaskContours(mask_rings, ring_verts, xy[:V], parent[:R])
+
+    def measure(self) -> MaskMeasurements:
+        """Area, box, moments, corner patterns, convex hull and calipers of every mask, on the device
+        (csrc/measure.cu), with the derived columns as properties of the result.  Window sides up to 32 768; a larger
+        window raises.  One 4-byte device->host read (the least area, and the overflow flag of the planes).  Rows:
+        ``masks.select(rows).measure()``."""
+        if not self.geom.is_cuda:
+            raise HdyError("measure() needs the planes on a CUDA device: hd_yolo_b200 has no CPU fallback")
+        K, dev = len(self), self.geom.device
+        geom, bits = _aligned16(self.geom.contiguous()), self._bits_nonempty()
+        area = torch.empty((K,), dtype=torch.int32, device=dev)
+        bbox = torch.empty((K, 4), dtype=torch.int32, device=dev)
+        moments = torch.empty((K, 5), dtype=torch.int64, device=dev)
+        quads = torch.empty((K, 4), dtype=torch.int32, device=dev)
+        hull = torch.empty((K, 3), dtype=torch.int64, device=dev)
+        hull_len = torch.empty((K, 2), dtype=torch.float64, device=dev)
+        flag = (self.status[:1] & _lib.HDY_STATUS_OVERFLOW) * -2
+        if K:
+            _call("hdy_mask_measure", ptr(geom), ptr(self.offsets), ptr(bits), K, ptr(area), ptr(bbox), ptr(moments),
+                  ptr(quads), ptr(hull), ptr(hull_len), _stream(), launches=2)
+            flag = torch.minimum(flag, area.amin().view(1))
+        low = int(flag.item())
+        if low == -2:
+            raise HdyError("bit-plane capacity overflow: pass a larger capacity_words")
+        if low < 0:
+            row = int(torch.nonzero(area < 0)[0, 0])
+            w, h = self.geom[row, 2:].tolist()
+            raise HdyError(f"mask {row} has a {w} x {h} window: measure() takes window sides up to 32768")
+        return MaskMeasurements(self.geom, area, bbox, moments, quads, hull[:, 0], hull[:, 2].to(torch.int32),
+                                hull[:, 1], hull_len[:, 0], hull_len[:, 1])
 
     def select(self, rows) -> "PackedMasks":
         """The masks of `rows` (index tensor or sequence), in that order, sharing `bits`: geom[rows] and offsets[rows]

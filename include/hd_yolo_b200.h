@@ -245,6 +245,28 @@ HDY_API int hdy_mask_contours(const int32_t* geom, const int64_t* offsets, const
                               const int64_t* ring_off, const int64_t* vert_off, int64_t* ring_verts, int32_t* parent,
                               int32_t* xy, hdy_stream_t stream);
 
+/* Morphometry of cropped bit planes (PackedMasks.measure, csrc/measure.cu; DESIGN §3.10b).  Pixels, windows and padding
+ * bits as for the contours above; (gx, gy, w, h) = geom[i], dx = x - gx and dy = y - gy window-relative pixel indices.
+ * Exact fields of mask i (all integers but the two f64 values, whose operation order is fixed):
+ *   area [K] i32          set pixels (= hdy_mask_areas)
+ *   bbox [K,4] i32        tight box of the set pixels (x0, y0, x1, y1), canvas corners, x1 / y1 exclusive
+ *   moments [K,5] i64     sum dx, sum dy, sum dx^2, sum dy^2, sum dx*dy over the set pixels
+ *   quads [K,4] i32       over the (w+1)(h+1) corners of the window, the 2 x 2 pixel patterns around the corner
+ *                         (outside the window = unset): n1 (one set), n2 (two sharing an edge), n3 (three set), nD (two
+ *                         on a diagonal)
+ *   hull [K,3] i64        convex_area2 (twice the area of the convex hull of the set pixels' unit squares), feret_max2
+ *                         (largest squared distance between two hull vertices), hull_verts (vertices: pixel corners,
+ *                         collinear points dropped)
+ *   hull_len [K,2] f64    convex_perimeter = sum of sqrt((double)(dx^2 + dy^2)) over the hull's edges in order, starting
+ *                         at the least hull vertex in (y, x) order and going in the exterior rings' rotational sense;
+ *                         feret_min = min over hull edges e = b - a of (double)max_v |cross(e, v - a)| / sqrt((double)e.e)
+ * Empty masks (w or h <= 0, or no set pixel) give 0 in every field.  Window sides up to 32 768 keep every sum exact; a
+ * larger window gets area -1 and 0 in every other field.  geom is 16-byte aligned; K = 0 is a no-op.  Windows up to
+ * 64 x 64 are measured one warp per mask, larger ones one CTA per mask. */
+HDY_API int hdy_mask_measure(const int32_t* geom, const int64_t* offsets, const uint32_t* bits, int K, int32_t* area,
+                             int32_t* bbox, int64_t* moments, int32_t* quads, int64_t* hull, double* hull_len,
+                             hdy_stream_t stream);
+
 /* North-star process_mask (ultralytics/yolov5 v7 utils/segment/general.py::process_mask + crop_mask; the
  * reference itself has no such function): mask = sigmoid(coef . protos), zero outside the box scaled by
  * (mw/iw, mh/ih), optional bilinear upsample (align_corners=False) to (ih, iw), > 0.5.  Batched over tiles:
